@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--reads n --read-len L --read-groups R] [--layout auto|segmented|read-order]
-                    [--scaling weak|strong --total-reads T] [--stream-batch B]
+                    [--scaling weak|strong --total-reads T] [--stream-batch B] [--dump-outputs DIR]
 
 Metric (BASELINE.json): bases/sec recalibrated (table build + apply).  Workload:
   N = 1   BASELINE config 2: synthetic 10 M x 150 bp interleaved pairs, 1 read group, Q2-Q41, 1 % mismatches
@@ -29,6 +29,11 @@ and compares tables and output checksums with the N-rank result, outside the tim
 `--impl reference` times the CPU restatement of the reference's algorithm (oracle/, all host threads) on a
 bounded sample of the same workload; the Python reference itself is pure Python, cannot travel to the GPU box
 and runs at ~0.26 Mbases/s/core (tools/reference_speed.py).
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (see dump_outputs): the inputs
+are a pure function of the arguments, so two builds of the project can be compared output for output.
+
+The benchmark runs from the tree as it was built and writes nothing there (no bytecode, no compiling).
 """
 import argparse
 import ctypes as C
@@ -39,6 +44,7 @@ import subprocess
 import sys
 import time
 
+sys.dont_write_bytecode = True   # the tree may be read-only: leave no __pycache__ behind in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "kbbq-py_b200"))
 
@@ -195,9 +201,8 @@ class ClockSampler:
 def cpu_port_throughput(n_reads, L, R, seed, target_s, threads=0):
     """Oracle (CPU port of the reference algorithm) on a bounded sample -> (bases/s, sample description)."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import oracle
+    import oracle   # loads the libkbbq_oracle.so the build made; nothing is compiled here
     from kbbq import synth
-    oracle.build()
     # every hardware thread this process may run on; torchrun exports OMP_NUM_THREADS=1 to its workers, which
     # omp_get_max_threads() would obey, so the count is passed explicitly (omp_set_num_threads in the oracle)
     threads = threads or len(os.sched_getaffinity(0)) or oracle.max_threads()
@@ -455,6 +460,35 @@ def checksum(t, L):
         ramp = (torch.arange(lo, lo + x.shape[0], device=t.device, dtype=torch.int64) % 65521) + 1
         s3 += int((rows * ramp).sum())
     return [s1, s2, s3]
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, hp):
+    """--dump-outputs: what a caller of the hot path holds after the last timed step, one DIR/<name>.npy per array.
+    The tables and the model under the reference's names (meanq ... dinuc_total, rgdq ... dindq) as float64, exact
+    for these int64 counts; the recalibrated qualities of a sample of reads drawn with the workload's seed as
+    float32 [rows, L] (`out_qual`), with their read numbers in the batch (`out_qual_reads`).  DUMP_BYTES at most."""
+    import numpy as np
+    import torch
+    rec, N, L = hp.rec, hp.wl.N, hp.wl.L
+    fields = {"meanq": rec.meanq, "rg_errs": rec.rg_errs, "rg_total": rec.rg_total, "q_errs": rec.q_errs,
+              "q_total": rec.q_total, "pos_errs": rec.pos_errs, "pos_total": rec.pos_total,
+              "dinuc_errs": rec.din_errs, "dinuc_total": rec.din_total,
+              "rgdq": rec.rgdq, "qdq": rec.qdq, "posdq": rec.posdq, "dindq": rec.dindq}
+    arrays = {name: t.cpu().numpy().astype(np.float64) for name, t in fields.items()}
+    room = DUMP_BYTES - (1 << 16) - sum(a.nbytes for a in arrays.values())   # 64 KB for the .npy headers
+    rows = min(N, 1 << 16, room // (4 * L + 8))
+    if rows <= 0:
+        raise SystemExit("bench.py: the tables alone exceed the %d bytes of --dump-outputs" % DUMP_BYTES)
+    idx = np.sort(np.random.default_rng(hp.wl.seed).choice(N, rows, replace=False))
+    out = hp.output_in_read_order()
+    arrays["out_qual"] = out[torch.from_numpy(idx).to(out.device)].cpu().numpy().astype(np.float32)
+    arrays["out_qual_reads"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def link_rates(dev, barrier, world, nbytes=1 << 30):
@@ -729,6 +763,8 @@ def run_b200(args):
     if batch <= 0 and N * L * (8 if R > 1 else 4) > 120e9:
         batch = 32_000_000 if R == 1 else 25_000_000
     if batch > 0:
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs needs the batch resident in HBM, not streamed in batches")
         sampler = ClockSampler(local) if rank == 0 else None
         r = run_streamed_config(wl, batch, dev, world, rank, barrier)
         clocks = sampler.stop() if sampler else None
@@ -759,6 +795,8 @@ def run_b200(args):
     config["layout"] = ("segmented: rows sorted by (read group, mate), spans padded to 16 rows -- the layout the host-buffer "
                         "entry points keep in HBM (segmentation: see `layouts` and `e2e`)") if layout == "segmented" else \
         "read order: rows as the host has them" + (", rg[] per read (work-list gather)" if R > 1 else "")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, hp)   # rank 0's shard starts at read 0 of the stream
 
     parity_n = None
     if world > 1 and not args.no_verify:
@@ -921,7 +959,14 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` / `layouts` blocks")
     ap.add_argument("--no-fastq", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="N > 1: skip the parity check against rank 0 alone")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the tables, the model and the qualities of a seeded sample of "
+                         "reads that the last step computed to DIR/<name>.npy (float32 / float64, 64 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -41,3 +41,31 @@ def test_b200_arm_line():
     assert d["e2e"]["h2d_bytes_per_step"] > 0 and d["e2e"]["d2h_bytes_per_step"] == 400000 * 150
     assert d["cpu_baseline"]["kind"] == "port" and "workload" in d["config"] and "model" not in d["config"]
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("R", [1, 8])
+def test_dump_outputs_match_oracle(tmp_path, oracle_mod, R):
+    """--dump-outputs: float32 / float64 arrays, 64 MB at most, and what the oracle computes on the same reads (rows in
+    read order with one read group, the segmented layout with several)."""
+    import numpy as np
+    from conftest import DELTA_KEYS, TABLE_KEYS
+    from kbbq import synth
+    N, L = 100_000, 150
+    d = _run(["--reads", str(N), "--read-groups", str(R), "--steps", "2", "--warmup", "1", "--no-configs", "--no-e2e",
+              "--no-fastq", "--no-cpu", "--dump-outputs", str(tmp_path)])
+    assert d["steps"] == 2
+    names = os.listdir(tmp_path)
+    got = {f[:-len(".npy")]: np.load(tmp_path / f) for f in names}
+    assert set(got) == set(TABLE_KEYS + DELTA_KEYS + ("out_qual", "out_qual_reads"))
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert sum(os.path.getsize(tmp_path / f) for f in names) <= 64_000_000
+    seq, qual, corr, rg, second = synth.synth_reads(d["config"]["seed"], 0, N, L, R)
+    tables = oracle_mod.covariate_arrays(seq, qual, corr, rg, second, L, R)
+    deltas = oracle_mod.get_delta_qs(*tables)
+    for name, want in zip(TABLE_KEYS + DELTA_KEYS, tables + deltas):
+        assert np.array_equal(got[name], want), name
+    rows = got["out_qual_reads"].astype(np.int64)
+    assert rows.size == 1 << 16 and np.all(np.diff(rows) > 0)
+    want = oracle_mod.apply(seq[rows], qual[rows], rg[rows], second[rows], L, R, tables[0], *deltas)
+    assert np.array_equal(got["out_qual"], want)
