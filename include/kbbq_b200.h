@@ -121,6 +121,10 @@ int kbbq_posterior_q_real(const double *prior_q_dev, const int64_t *numerrs_dev,
  * into canonical reads (position = cycle, reverse strand complemented, skipped and N bases at quality
  * 0) and goes through the shared-memory kernels of kbbq_build / kbbq_apply; with workspace == NULL the
  * direct one-thread-per-base kernels run (global atomics: correct, two orders of magnitude slower).
+ * Both paths compute the same tables, qualities and status: a base outside ACGTN in a usable dinucleotide of a
+ * forward read raises KBBQ_FLAG_BAD_BASE (the reference's TypeError); elsewhere such a base is tallied and
+ * recalibrated as N is in the dinucleotide covariate, and as the base it is in the cycle covariate.
+ * aln_start / aln_end past L are cut at L, and aln_end < aln_start is an empty window.  minscore: 0..42.
  */
 int kbbq_bam_workspace_bytes(int64_t N, int L, int R, size_t *bytes);
 int kbbq_build_bam(const uint8_t *seq_dev, const uint8_t *qual_dev, const uint8_t *err_dev,
@@ -166,8 +170,16 @@ int kbbq_get_delta_qs(const int64_t *meanq_dev, const int64_t *rg_errs_dev,
  * with dinuc -1 gathering the last dinuc column and read-2 cycles indexing from the end.  The
  * delta tables have the reference's shapes: qdq [R][nq], posdq [R][nq][2L], dindq [R][nq][ndin1]
  * (nq <= 43; a quality >= nq raises KBBQ_FLAG_QUAL_RANGE).  out_qual is u8[N*L] (no clamp: the
- * low 8 bits of the sum, as the reference keeps whatever the sum is).
+ * low 8 bits of the sum, as the reference keeps whatever the sum is).  A base outside ACGTN anywhere in the
+ * batch raises KBBQ_FLAG_BAD_BASE, the rule of kbbq_build, on every path (the shared-memory, generic and
+ * segmented kernels write the same bytes and the same status for any input with qualities below 128).
+ * minscore: 0..42 (0 has no shared-memory plan: path 1 and the segmented entry points refuse it).
+ * path: 0 = shared-memory kernel when a plan fits, else generic; 1 = shared-memory kernel or KBBQ_E_ARG; 2 = generic.
+ * path | KBBQ_APPLY_BASES_CHECKED skips the base check: for a caller that has passed these very bytes to kbbq_build
+ * and reads the same status word (the build has flagged any base outside ACGTN), or that knows they hold ACGTN only.
+ * The check costs the shared-memory kernel about 6 % (DESIGN.md).
  */
+#define KBBQ_APPLY_BASES_CHECKED 0x10
 int kbbq_apply(const uint8_t *seq_dev, const uint8_t *qual_dev, const uint16_t *rg_dev,
                const uint8_t *second_dev, int64_t N, int L, int R, int minscore,
                const int64_t *meanq_dev, const int64_t *rgdq_dev, const int64_t *qdq_dev,
@@ -219,6 +231,13 @@ int kbbq_apply_segmented(const uint8_t *seq_dev, const uint8_t *qual_dev, const 
                          const int64_t *qdq_dev, const int64_t *posdq_dev, const int64_t *dindq_dev, int nq,
                          int ndin1, uint8_t *out_qual_dev, void *workspace_dev, size_t workspace_bytes,
                          int *status_dev, void *stream);
+/* kbbq_apply_segmented with flags = 0 or KBBQ_APPLY_BASES_CHECKED (as kbbq_apply's path flag, for a batch that went
+ * through kbbq_build_segmented unchanged) */
+int kbbq_apply_segmented_flags(const uint8_t *seq_dev, const uint8_t *qual_dev, const uint32_t *seg_dev,
+                               int64_t rows_bound, int L, int R, int minscore, const int64_t *meanq_dev,
+                               const int64_t *rgdq_dev, const int64_t *qdq_dev, const int64_t *posdq_dev,
+                               const int64_t *dindq_dev, int nq, int ndin1, uint8_t *out_qual_dev, void *workspace_dev,
+                               size_t workspace_bytes, int *status_dev, int flags, void *stream);
 
 /*
  * Whole path on HOST buffers: H2D, build, marginals, deltas, apply, D2H -- what
@@ -364,7 +383,10 @@ int kbbq_synth_reads(uint64_t seed, int64_t first_read, int64_t n, int L, int R,
  * out[10] = {reads per group, lanes per group, thread-groups, consumer threads, producer warps,
  * groups per thread-group and stage, ring depth, dinuc replicas, dynamic shared memory, table bytes}.
  * KBBQ_E_ARG when the shape falls back to the generic kernels.  Diagnostics / tests.
+ * arrays | KBBQ_PLAN_SEGMENTED: the plan of kbbq_build_segmented / kbbq_apply_segmented instead (the span geometry
+ * of a segmented batch, which may differ from that of the same reads in read order).
  */
+#define KBBQ_PLAN_SEGMENTED 0x100
 int kbbq_plan_info(int L, int R, int minscore, int arrays, int max_smem, int *out);
 
 /*

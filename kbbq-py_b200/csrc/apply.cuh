@@ -44,8 +44,9 @@ static_assert((offsetof(ApplyArgs, t) + offsetof(TableCfg, ohe)) % 16 == 0,
 // bytes of shared memory the apply tables take
 __host__ __device__ inline int apply_table_bytes(const TableCfg &t) { return t.table_bytes; }
 
-// Consumer side of the apply kernel; UNI as in build_consume (build.cuh).
-template <int KPS, bool UNI>
+// Consumer side of the apply kernel; UNI as in build_consume (build.cuh).  VALIDATE: flag a base outside ACGTN as the
+// build does (off when the caller vouches for the bases: KBBQ_APPLY_BASES_CHECKED, kbbq_b200.cu).
+template <int KPS, bool UNI, bool VALIDATE>
 __device__ __forceinline__ void apply_consume(const ApplyArgs &a, unsigned char *smem_raw, uint32_t lo, uint32_t hi,
                                               uint32_t uni_flo, uint32_t uni_fhi) {
     const Geom &g = a.g;
@@ -81,8 +82,9 @@ __device__ __forceinline__ void apply_consume(const ApplyArgs &a, unsigned char 
     const uint32_t revoff = t.revoff, addq = t.addq, gbytes = g.gbytes;
     const uint32_t addnq = (uint32_t)(128 - a.nq) * ONE4;  // q + this has bit 7 set iff q >= nq (q < 128)
     const uint32_t one = pin(1u);                          // see add_fma (build.cuh)
+    const uint32_t lut_lo = pin(0x43014101u), lut_hi = pin(0x474E0154u);  // base validation LUT (build.cuh)
     uint32_t stage = 0, phase = 0;
-    uint32_t qgood = 0xFFFFFFFFu;
+    uint32_t qgood = 0xFFFFFFFFu, bbad = 0;
 
     int cur_rg = -1, cur_sub = -1;
     int hs0 = 0, hs1 = 1;   // half of the cycle axis each table slot holds (build.cuh)
@@ -157,6 +159,13 @@ __device__ __forceinline__ void apply_consume(const ApplyArgs &a, unsigned char 
                 const uint32_t nm8 = prmt((sw | pw) * 16u, 0xFFFFFFFFu, seln);
                 const uint32_t qd = qrow4 & ~nm8;
                 const uint32_t x01 = prmt(d4, qd, 0x5140u), x23 = prmt(d4, qd, 0x7362u);  // see build.cuh
+                if (VALIDATE) {
+                    // base validation as in the build: rebuild each byte from its 3-bit code, any difference = a base
+                    // outside ACGTN (foreign bytes are masked off by rowmask at the end)
+                    const uint32_t code3 = sw & 0x07070707u;
+                    const uint32_t vsel = __dp2a_hi(t.val16[1], code3, __dp2a_lo(t.val16[0], code3, 0u));
+                    bbad |= prmt(lut_lo, lut_hi, vsel) ^ sw;
+                }
 
                 uint32_t v[4];
 #pragma unroll
@@ -233,10 +242,11 @@ __device__ __forceinline__ void apply_consume(const ApplyArgs &a, unsigned char 
         }
     }
     if (~qgood & rowmask & H4) atomicOr(a.status, KBBQ_FLAG_QUAL_RANGE);
+    if (VALIDATE && (bbad & rowmask)) atomicOr(a.status, KBBQ_FLAG_BAD_BASE);
 }
 
 
-template <int KPS>
+template <int KPS, bool VALIDATE>
 __global__ void __launch_bounds__(MAX_THREADS, 1) apply_smem_kernel(const __grid_constant__ ApplyArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const Geom &g = a.g;
@@ -269,8 +279,8 @@ __global__ void __launch_bounds__(MAX_THREADS, 1) apply_smem_kernel(const __grid
         return;
     }
 
-    if (uniform) apply_consume<KPS, true>(a, smem_raw, lo, hi, a.uni[1], a.uni[2]);
-    else apply_consume<KPS, false>(a, smem_raw, lo, hi, 0u, 0u);
+    if (uniform) apply_consume<KPS, true, VALIDATE>(a, smem_raw, lo, hi, a.uni[1], a.uni[2]);
+    else apply_consume<KPS, false, VALIDATE>(a, smem_raw, lo, hi, 0u, 0u);
 }
 
 // Generic path (any L): one thread per base, folded tables gathered from global memory (L1/L2).
@@ -283,6 +293,7 @@ struct ApplyGenericArgs {
     int L, R, minscore, nq;
     const short *fold_cyc, *fold_din;
     int *status;
+    bool validate;   // see apply_consume
 };
 
 __global__ void apply_generic_kernel(ApplyGenericArgs a) {
@@ -292,6 +303,8 @@ __global__ void apply_generic_kernel(ApplyGenericArgs a) {
         const long long r = i / a.L;
         const int c = (int)(i - r * a.L);
         const unsigned int q = a.qual[i];
+        const uint8_t s = a.seq[i];
+        if (a.validate && base_code_ref(s) == 5) atomicOr(a.status, KBBQ_FLAG_BAD_BASE);   // the build's rule: any byte outside ACGTN
         if ((int)q < a.minscore) { a.out[i] = (uint8_t)q; continue; }
         if ((int)q >= a.nq) { atomicOr(a.status, KBBQ_FLAG_QUAL_RANGE); a.out[i] = (uint8_t)q; continue; }
         const unsigned int g = a.rg ? a.rg[r] : 0;
@@ -300,8 +313,9 @@ __global__ void apply_generic_kernel(ApplyGenericArgs a) {
         const size_t gq = (size_t)g * NQ + q;
         int v = a.fold_cyc[gq * (2 * a.L) + c2];
         if (c > 0) {
-            const uint8_t s = a.seq[i], ps = a.seq[i - 1];
-            if (s != 'N' && ps != 'N') v += a.fold_din[gq * DIN_SLOTS + ((((ps >> 1) & 3) << 2) | ((s >> 1) & 3))];
+            // as the shared-memory kernel: a byte with bit 3 set (of ACGTN only N) has no dinucleotide term
+            const uint8_t ps = a.seq[i - 1];
+            if (!((s | ps) & 8u)) v += a.fold_din[gq * DIN_SLOTS + ((((ps >> 1) & 3) << 2) | ((s >> 1) & 3))];
         }
         a.out[i] = (uint8_t)v;
     }

@@ -49,6 +49,14 @@ __device__ __forceinline__ int bam_dinuc(const uint8_t *row, int i, int lo, int 
     return 4 * prev + cur;
 }
 
+// An aligned window reaching past the read is cut at its end, and an inverted one is empty (the canonical form
+// does the same): query_alignment_start / _end never exceed the read length, so this only keeps bad input in bounds.
+__device__ __forceinline__ void bam_clamp_window(int L, int *lo, int *hi) {
+    if (*lo > L) *lo = L;
+    if (*hi > L) *hi = L;
+    if (*hi < *lo) *hi = *lo;
+}
+
 struct BuildBamArgs {
     const uint8_t *seq, *qual, *err, *skip;
     const uint16_t *rg;
@@ -74,7 +82,8 @@ __global__ void build_bam_kernel(BuildBamArgs a) {
         const unsigned int g = a.rg ? a.rg[r] : 0;
         if (g >= (unsigned int)a.R) { atomicOr(a.status, KBBQ_FLAG_RG_RANGE); continue; }
         const int fl = a.flags ? a.flags[r] : 0;
-        const int lo = a.aln_start ? a.aln_start[r] : 0, hi = a.aln_end ? a.aln_end[r] : a.L;
+        int lo = a.aln_start ? a.aln_start[r] : 0, hi = a.aln_end ? a.aln_end[r] : a.L;
+        bam_clamp_window(a.L, &lo, &hi);
         const bool reverse = fl & BAM_FLAG_REVERSE;
         int cyc = 0, din = 0;                                     // clipped bases keep 0 (:24,:43)
         if (i >= lo && i < hi) {
@@ -154,7 +163,7 @@ struct BamCanonArgs {
     const uint8_t *flags;
     const uint16_t *aln_start, *aln_end;
     long long N;
-    int L, R, minscore;
+    int L, R, minscore, nq;   // nq: qualities the apply's delta tables hold (the build: 43)
     bool build;               // false: apply (whole read, qualities untouched, no corrected array)
     uint8_t *cseq, *cqual, *ccorr, *csecond;
     unsigned long long *pos_errs, *pos_total, *din_errs, *din_total;
@@ -198,6 +207,13 @@ __device__ __forceinline__ uint32_t complement4(uint32_t w) {
     const uint32_t bad = nonzero_mask(self ^ w);              // a byte that is not the base its code stands for
     return (comp & ~bad) | (0x4E4E4E4Eu & bad);
 }
+// 0xFF in every byte of w that is not one of A, C, G, T, N
+__device__ __forceinline__ uint32_t nonacgtn_mask(uint32_t w) {
+    const uint32_t code3 = (w >> 1) & 0x07070707u;
+    const uint32_t y = code3 | (code3 >> 4);
+    const uint32_t sel = __byte_perm(y, 0u, 0x4420u) & 0x7777u;
+    return nonzero_mask(__byte_perm(0x47544341u /* A C T G */, 0x4E000000u /* . . . N */, sel) ^ w);
+}
 
 // One thread per aligned output word (`wmax` word slots per read, r0 = first read of this launch), so
 // that nothing waits for anything: a warp-per-read loop was bound by its chain of round trips.
@@ -215,9 +231,7 @@ __global__ void __launch_bounds__(BAM_WARPS * 32) bam_canon_kernel(BamCanonArgs 
     if (a.build) {
         lo = a.aln_start ? a.aln_start[r] : 0;
         hi = a.aln_end ? a.aln_end[r] : a.L;
-        if (lo > a.L) lo = a.L;
-        if (hi > a.L) hi = a.L;
-        if (hi < lo) hi = lo;
+        bam_clamp_window(a.L, &lo, &hi);
     }
     const int alen = hi - lo;
     const long long row = r * a.L;
@@ -227,7 +241,10 @@ __global__ void __launch_bounds__(BAM_WARPS * 32) bam_canon_kernel(BamCanonArgs 
     if (k == 0) a.csecond[r] = (uint8_t)(fl & BAM_FLAG_READ2);
     if (k >= ((ao + a.L + 3) >> 2)) return;
     const int p0 = 4 * k - ao;
-    if (p0 >= 0 && p0 + 3 < alen) {  // four positions inside the window: word path
+    // four positions inside the window: word path -- unless a forward-strand base of the word, or the one before it,
+    // lies outside ACGTN: the byte-wise path writes those as N and applies the reference's rule to them
+    if (p0 >= 0 && p0 + 3 < alen &&
+        (reverse || (!nonacgtn_mask(load4_any(seq + row + lo + p0)) && (p0 == 0 || bam_code(seq[row + lo + p0 - 1]) != 5)))) {
         const long long s = row + (reverse ? hi - 4 - p0 : lo + p0);
         uint32_t ws = load4_any(seq + s), wq = load4_any(qual + s), we = 0u, wk = 0u;
         if (a.build) {
@@ -265,7 +282,16 @@ __global__ void __launch_bounds__(BAM_WARPS * 32) bam_canon_kernel(BamCanonArgs 
         const bool sk = a.build && skipp && skipp[i] != 0;
         uint8_t b = 'N', q = 0, c = 'N';
         if (inside) {
-            b = reverse ? bam_complement(s) : s;
+            // a forward-strand base outside ACGTN: N in the canonical read, which leaves out its dinucleotides as the
+            // reference does where it does not raise; where it raises (bam_dinuc), the flag is set here
+            b = reverse ? bam_complement(s) : bam_code(s) == 5 ? (uint8_t)'N' : s;
+            if (!reverse && p > 0 && (a.build ? !sk : true)) {
+                const int cc = bam_code(s), pc = bam_code(seq[i - 1]);
+                const unsigned int g = a.rg ? a.rg[r] : 0;
+                if ((int)qq >= a.minscore && (int)qq < a.nq && g < (unsigned int)a.R && cc != 4 && pc != 4 &&
+                    (cc == 5 || pc == 5))
+                    atomicOr(a.status, KBBQ_FLAG_BAD_BASE);
+            }
             q = (a.build && (sk || s == 'N')) ? (uint8_t)0 : (uint8_t)qq;
             c = e ? (uint8_t)(b ^ 1) : b;
         } else if (a.build && !sk && (int)qq >= a.minscore && s != 'N') {

@@ -195,7 +195,8 @@ bool want_segmode(int L, int R, int minscore, int64_t C) {
 
 // pack < 0: the transport follows from the host threads this session has (pack_mode)
 int session_create(int device, int L, int R, int minscore, int64_t C, int64_t M, int host_threads, int pack, kbbq_session **out) {
-    if (device < 0 || L < 1 || R < 1 || R > 65535 || C < 1 || M < 0 || !out) return KBBQ_E_ARG;
+    if (device < 0 || L < 1 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ || C < 1 || M < 0 || !out)
+        return KBBQ_E_ARG;
     KBBQ_CUDA(cudaSetDevice(device));
     std::unique_ptr<kbbq_session> S(new kbbq_session);
     S->device = device; S->L = L; S->R = R; S->minscore = minscore;

@@ -150,23 +150,23 @@ static int launch_build_smem(const BuildArgs &a, int grid, size_t smem, cudaStre
 }
 
 template <int KPS>
-static int launch_apply_kps(const ApplyArgs &a, int grid, size_t smem, cudaStream_t st) {
-    auto kern = apply_smem_kernel<KPS>;
+static int launch_apply_kps(const ApplyArgs &a, bool validate, int grid, size_t smem, cudaStream_t st) {
+    auto kern = validate ? apply_smem_kernel<KPS, true> : apply_smem_kernel<KPS, false>;
     KBBQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, a.g.threads + 32 * a.g.nprod, smem, st>>>(a);  // + the producer warp(s)
     KBBQ_LAUNCHED();
     return KBBQ_OK;
 }
-static int launch_apply_smem(const ApplyArgs &a, int grid, size_t smem, cudaStream_t st) {
+static int launch_apply_smem(const ApplyArgs &a, bool validate, int grid, size_t smem, cudaStream_t st) {
     switch (a.sl.kps) {
-    case 8: return launch_apply_kps<8>(a, grid, smem, st);
-    case 7: return launch_apply_kps<7>(a, grid, smem, st);
-    case 6: return launch_apply_kps<6>(a, grid, smem, st);
-    case 5: return launch_apply_kps<5>(a, grid, smem, st);
-    case 4: return launch_apply_kps<4>(a, grid, smem, st);
-    case 3: return launch_apply_kps<3>(a, grid, smem, st);
-    case 2: return launch_apply_kps<2>(a, grid, smem, st);
-    default: return launch_apply_kps<1>(a, grid, smem, st);
+    case 8: return launch_apply_kps<8>(a, validate, grid, smem, st);
+    case 7: return launch_apply_kps<7>(a, validate, grid, smem, st);
+    case 6: return launch_apply_kps<6>(a, validate, grid, smem, st);
+    case 5: return launch_apply_kps<5>(a, validate, grid, smem, st);
+    case 4: return launch_apply_kps<4>(a, validate, grid, smem, st);
+    case 3: return launch_apply_kps<3>(a, validate, grid, smem, st);
+    case 2: return launch_apply_kps<2>(a, validate, grid, smem, st);
+    default: return launch_apply_kps<1>(a, validate, grid, smem, st);
     }
 }
 
@@ -204,11 +204,13 @@ int64_t kbbq_din_table_elems(int R) { return (int64_t)R * NQ * 16; }
 int64_t kbbq_launch_count(void) { return g_launches.load(); }
 
 int kbbq_plan_info(int L, int R, int minscore, int arrays, int max_smem, int *out) {
+    const bool segmode = (arrays & KBBQ_PLAN_SEGMENTED) != 0;
+    arrays &= ~KBBQ_PLAN_SEGMENTED;
     if (!out || L < 1 || R < 1 || (arrays != 2 && arrays != 3)) return KBBQ_E_ARG;
     Geom g;
     TableCfg tc;
     StageLayout sl;
-    if (!plan_kernel(L, R, minscore, arrays, max_smem > 0 ? max_smem : 232448, &g, &tc, &sl))
+    if (!plan_kernel(L, R, minscore, arrays, max_smem > 0 ? max_smem : 232448, &g, &tc, &sl, segmode))
         return KBBQ_E_ARG;  // the generic kernels would be used
     const int v[10] = {g.G, g.lanes, g.ng, g.threads, g.nprod, sl.kps, sl.stages, tc.drep, sl.total, tc.table_bytes};
     for (int i = 0; i < 10; ++i) out[i] = v[i];
@@ -392,7 +394,7 @@ int kbbq_build_bam(const uint8_t *seq, const uint8_t *qual, const uint8_t *err, 
                    const uint8_t *flags, const uint16_t *aln_start, const uint16_t *aln_end, int64_t N, int L, int R,
                    int minscore, int64_t *pos_errs, int64_t *pos_total, int64_t *din_errs, int64_t *din_total,
                    void *workspace, size_t workspace_bytes, int *status, void *stream) {
-    if (N < 0 || L < 1 || L > 32767 || R < 1 || R > 65535 || minscore < 0 || minscore > NQ) return KBBQ_E_ARG;
+    if (N < 0 || L < 1 || L > 32767 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ) return KBBQ_E_ARG;
     if (!pos_errs || !pos_total || !din_errs || !din_total || !status) return KBBQ_E_ARG;
     if (N == 0) return KBBQ_OK;
     if (!seq || !qual || !err) return KBBQ_E_ARG;
@@ -404,7 +406,7 @@ int kbbq_build_bam(const uint8_t *seq, const uint8_t *qual, const uint8_t *err, 
     if (workspace && minscore >= 1) {  // canonical form + the shared-memory build kernel
         BamWorkspace w = carve_bam_workspace(workspace, N, L, R);
         if (workspace_bytes < w.bytes) return KBBQ_E_WORKSPACE;
-        BamCanonArgs c = {seq, qual, err, skip, rg, flags, aln_start, aln_end, N, L, R, minscore, true,
+        BamCanonArgs c = {seq, qual, err, skip, rg, flags, aln_start, aln_end, N, L, R, minscore, NQ, true,
                           w.cseq, w.cqual, w.cthird, w.csecond,
                           (unsigned long long *)pos_errs, (unsigned long long *)pos_total,
                           (unsigned long long *)din_errs, (unsigned long long *)din_total, status};
@@ -425,7 +427,9 @@ int kbbq_apply_bam(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, 
                    int R, int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
                    const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual, void *workspace,
                    size_t workspace_bytes, int *status, void *stream) {
-    if (N < 0 || L < 1 || L > 32767 || R < 1 || R > 65535 || nq < 1 || nq > 256 || ndin1 != 17) return KBBQ_E_ARG;
+    if (N < 0 || L < 1 || L > 32767 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ || nq < 1 || nq > 256 ||
+        ndin1 != 17)
+        return KBBQ_E_ARG;
     if (!meanq || !rgdq || !qdq || !posdq || !dindq || !status) return KBBQ_E_ARG;
     if (N == 0) return KBBQ_OK;
     if (!seq || !qual || !out_qual) return KBBQ_E_ARG;
@@ -437,11 +441,12 @@ int kbbq_apply_bam(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, 
     if (workspace && minscore >= 1 && nq <= NQ) {  // canonical form + the shared-memory apply kernel + flip back
         BamWorkspace w = carve_bam_workspace(workspace, N, L, R);
         if (workspace_bytes < w.bytes) return KBBQ_E_WORKSPACE;
-        BamCanonArgs c = {seq, qual, nullptr, nullptr, rg, flags, nullptr, nullptr, N, L, R, minscore, false,
+        BamCanonArgs c = {seq, qual, nullptr, nullptr, rg, flags, nullptr, nullptr, N, L, R, minscore, nq, false,
                           w.cseq, w.cqual, nullptr, w.csecond, nullptr, nullptr, nullptr, nullptr, status};
         { const int rc_ = launch_bam_canon(c, st); if (rc_) return rc_; }
+        // the canonical reads hold A, C, G, T, N only: bam_canon_kernel has already applied the reference's rule
         int rc = kbbq_apply(w.cseq, w.cqual, rg, w.csecond, N, L, R, minscore, meanq, rgdq, qdq, posdq, dindq, nq, ndin1,
-                            w.cthird, w.inner, w.inner_bytes, status, 0, stream);
+                            w.cthird, w.inner, w.inner_bytes, status, KBBQ_APPLY_BASES_CHECKED, stream);
         if (rc) return rc;
         {
             const unsigned int wmax = (unsigned int)((3 + L + 3) >> 2);
@@ -532,6 +537,8 @@ static int apply_impl(const uint8_t *seq, const uint8_t *qual, const uint16_t *r
                       void *workspace, size_t workspace_bytes, int *status, int path, void *stream,
                       const unsigned int *seg_rows) {
     const bool segmode = seg_rows != nullptr;
+    const bool validate = !(path & KBBQ_APPLY_BASES_CHECKED);
+    path &= ~KBBQ_APPLY_BASES_CHECKED;
     if (N < 0 || L < 1 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ) return KBBQ_E_ARG;
     if (nq < 1 || nq > NQ || ndin1 < 16 || ndin1 > 64) return KBBQ_E_ARG;
     if (!meanq || !rgdq || !qdq || !posdq || !dindq || !status) return KBBQ_E_ARG;
@@ -558,7 +565,7 @@ static int apply_impl(const uint8_t *seq, const uint8_t *qual, const uint16_t *r
                          (uint64_t)((N + g.G - 1) / g.G) < 0xFFFFFFFFull;
     if (!smem_ok) {
         if (path == 1 || segmode) return KBBQ_E_ARG;
-        ApplyGenericArgs a = {seq, qual, rg, second, out_qual, N, L, R, minscore, nq, w.fold_cyc, w.fold_din, status};
+        ApplyGenericArgs a = {seq, qual, rg, second, out_qual, N, L, R, minscore, nq, w.fold_cyc, w.fold_din, status, validate};
         apply_generic_kernel<<<sms * 8, 256, 0, st>>>(a);
         KBBQ_LAUNCHED();
         return KBBQ_OK;
@@ -567,7 +574,7 @@ static int apply_impl(const uint8_t *seq, const uint8_t *qual, const uint16_t *r
     if (tail) {
         const int64_t n0 = N - tail;
         ApplyGenericArgs ga = {seq + n0 * L, qual + n0 * L, rg ? rg + n0 : nullptr, second ? second + n0 : nullptr,
-                               out_qual + n0 * L, tail, L, R, minscore, nq, w.fold_cyc, w.fold_din, status};
+                               out_qual + n0 * L, tail, L, R, minscore, nq, w.fold_cyc, w.fold_din, status, validate};
         apply_generic_kernel<<<1, 256, 0, st>>>(ga);
         KBBQ_LAUNCHED();
         N = n0;
@@ -584,7 +591,7 @@ static int apply_impl(const uint8_t *seq, const uint8_t *qual, const uint16_t *r
     a.seq = seq; a.qual = qual; a.out = out_qual; a.total_bytes = N * L; a.g = g; a.t = tc; a.R = R; a.nq = nq;
     a.sl = sl;
     a.entries = w.entries; a.seg = w.seg; a.uni = w.uni; a.fold_cyc = w.fold_cyc; a.fold_din = w.fold_din; a.status = status;
-    return launch_apply_smem(a, sms, a.sl.total, st);
+    return launch_apply_smem(a, validate, sms, a.sl.total, st);
 }
 
 int kbbq_apply(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second, int64_t N,
@@ -595,13 +602,21 @@ int kbbq_apply(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, cons
                       workspace, workspace_bytes, status, path, stream, nullptr);
 }
 
+int kbbq_apply_segmented_flags(const uint8_t *seq, const uint8_t *qual, const uint32_t *seg, int64_t rows_bound, int L,
+                               int R, int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
+                               const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual,
+                               void *workspace, size_t workspace_bytes, int *status, int flags, void *stream) {
+    if (!seg || rows_bound % SEG_ALIGN || (flags & ~KBBQ_APPLY_BASES_CHECKED)) return KBBQ_E_ARG;
+    return apply_impl(seq, qual, nullptr, nullptr, rows_bound, L, R, minscore, meanq, rgdq, qdq, posdq, dindq, nq, ndin1,
+                      out_qual, workspace, workspace_bytes, status, 1 | flags, stream, seg);
+}
+
 int kbbq_apply_segmented(const uint8_t *seq, const uint8_t *qual, const uint32_t *seg, int64_t rows_bound, int L, int R,
                          int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
                          const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual,
                          void *workspace, size_t workspace_bytes, int *status, void *stream) {
-    if (!seg || rows_bound % SEG_ALIGN) return KBBQ_E_ARG;
-    return apply_impl(seq, qual, nullptr, nullptr, rows_bound, L, R, minscore, meanq, rgdq, qdq, posdq, dindq, nq, ndin1,
-                      out_qual, workspace, workspace_bytes, status, 1, stream, seg);
+    return kbbq_apply_segmented_flags(seq, qual, seg, rows_bound, L, R, minscore, meanq, rgdq, qdq, posdq, dindq, nq, ndin1,
+                                      out_qual, workspace, workspace_bytes, status, 0, stream);
 }
 
 // ---- segmented batch layout (segment.cuh) ----

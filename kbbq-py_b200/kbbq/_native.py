@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(HERE, "libkbbq_b200.so")
 
 NQ = 43
 FLAG_QUAL_RANGE, FLAG_BAD_BASE, FLAG_RG_RANGE, FLAG_SEGMENTS = 1, 2, 4, 8
+APPLY_BASES_CHECKED = 0x10   # kbbq_apply path flag: skip the base check (include/kbbq_b200.h)
 E_DATA = -4
 E_UNSUPPORTED = -12
 
@@ -97,6 +98,7 @@ SIGNATURES = {
     "kbbq_unsegment_rows": (_i, [_vp, _vp, _i64, _i, _i64, _vp, _vp]),
     "kbbq_build_segmented": (_i, [_vp] * 4 + [_i64, _i, _i, _i] + [_vp] * 4 + [_vp, _sz, _vp, _vp]),
     "kbbq_apply_segmented": (_i, [_vp] * 3 + [_i64, _i, _i, _i] + [_vp] * 5 + [_i, _i, _vp, _vp, _sz, _vp, _vp]),
+    "kbbq_apply_segmented_flags": (_i, [_vp] * 3 + [_i64, _i, _i, _i] + [_vp] * 5 + [_i, _i, _vp, _vp, _sz, _vp, _i, _vp]),
 }
 
 

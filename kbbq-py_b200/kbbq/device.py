@@ -10,6 +10,7 @@ deterministically from the reduced integers (so no broadcast is needed) and appl
 own shard.  Integer sums make the result independent of the number of ranks.
 """
 import ctypes as C
+import weakref
 
 import torch
 
@@ -76,6 +77,9 @@ class DeviceRecalibrator:
         self.workspace = None
         self.ws_reads = -1
         self._ensure_workspace(max_reads)
+        # base arrays built since the last reset (a weak reference and torch's version counter of each): any base
+        # outside ACGTN in them has already set the status word, so applying them again skips the base check
+        self._built = []
 
     @_on_device
     def _ensure_workspace(self, n_reads):
@@ -93,6 +97,26 @@ class DeviceRecalibrator:
     def reset(self):
         self.tables.zero_()
         self.status.zero_()
+        self._built = []
+
+    @staticmethod
+    def _version(t):
+        try:
+            return t._version
+        except RuntimeError:   # inference-mode tensors keep no version counter
+            return None
+
+    def _remember_built(self, seq):
+        v = self._version(seq)
+        self._built = [(r, w) for r, w in self._built if r() is not None and r() is not seq]
+        if v is not None:
+            self._built.append((weakref.ref(seq), v))
+
+    def _bases_checked(self, seq):
+        """True when `seq` is a tensor this recalibrator built since its last reset and that torch has not written
+        to since: the build flagged any base outside ACGTN in this status word, the apply need not look again."""
+        v = self._version(seq)
+        return v is not None and any(r() is seq and w == v for r, w in self._built)
 
     @_on_device
     def build(self, seq, qual, corr, rg=None, second=None, path=0):
@@ -103,6 +127,7 @@ class DeviceRecalibrator:
                                  _p(self.pos_errs), _p(self.pos_total), _p(self.din_errs), _p(self.din_total),
                                  _p(self.workspace), self.ws_bytes, _p(self.status), path, self._stream())
         _native.check(rc)
+        self._remember_built(seq)
 
     @_on_device
     def build_from_bits(self, seq, qual, bits, corr_scratch, rg=None, second=None):
@@ -144,15 +169,17 @@ class DeviceRecalibrator:
                                            _p(self.din_total), _p(self.workspace), self.ws_bytes, _p(self.status),
                                            self._stream())
         _native.check(rc)
+        self._remember_built(sb.seq)
 
     @_on_device
     def apply_segmented(self, sb, out_seg):
         """kbbq_apply on a segmented batch; out_seg: u8 [rows_bound, L] in the segmented order."""
         self._ensure_workspace(sb.rows_bound)
-        rc = self.lib.kbbq_apply_segmented(_p(sb.seq), _p(sb.qual), _p(sb.seg), sb.rows_bound, self.L, self.R, self.minscore,
-                                           _p(self.meanq), _p(self.rgdq), _p(self.qdq), _p(self.posdq), _p(self.dindq),
-                                           NQ, 17, _p(out_seg), _p(self.workspace), self.ws_bytes, _p(self.status),
-                                           self._stream())
+        flags = _native.APPLY_BASES_CHECKED if self._bases_checked(sb.seq) else 0
+        rc = self.lib.kbbq_apply_segmented_flags(_p(sb.seq), _p(sb.qual), _p(sb.seg), sb.rows_bound, self.L, self.R,
+                                                 self.minscore, _p(self.meanq), _p(self.rgdq), _p(self.qdq),
+                                                 _p(self.posdq), _p(self.dindq), NQ, 17, _p(out_seg), _p(self.workspace),
+                                                 self.ws_bytes, _p(self.status), flags, self._stream())
         _native.check(rc)
 
     @_on_device
@@ -180,9 +207,12 @@ class DeviceRecalibrator:
 
     @_on_device
     def apply(self, seq, qual, out, rg=None, second=None, path=0):
-        """Write recalibrated qualities of one batch into `out` (kbbq_apply)."""
+        """Write recalibrated qualities of one batch into `out` (kbbq_apply).  A batch that was not built here since
+        the last reset (or was changed since) has its bases checked: one outside ACGTN raises at check_status()."""
         N = seq.numel() // self.L
         self._ensure_workspace(N)
+        if self._bases_checked(seq):
+            path |= _native.APPLY_BASES_CHECKED
         rc = self.lib.kbbq_apply(_p(seq), _p(qual), _p(rg), _p(second), N, self.L, self.R, self.minscore,
                                  _p(self.meanq), _p(self.rgdq), _p(self.qdq), _p(self.posdq), _p(self.dindq),
                                  NQ, 17, _p(out), _p(self.workspace), self.ws_bytes, _p(self.status), path,

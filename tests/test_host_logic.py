@@ -211,7 +211,8 @@ def test_host_pack_nibbles_matches_numpy():
 def test_shared_memory_plans_fit_for_every_read_length():
     """kbbq_plan_info (host only): every read length the shared-memory kernels claim (4 .. 288) gets a plan that
     fits the 227 KB of a B200 SM, whole warps of consumers + producer warps within 1024 threads, a ring of at least
-    two stages -- for one and for several read groups, build (3 arrays staged) and apply (2)."""
+    two stages -- for one and for several read groups, build (3 arrays staged) and apply (2), in read order and for
+    a segmented batch (arrays | 0x100, KBBQ_PLAN_SEGMENTED)."""
     import ctypes as C
     from kbbq import _native
     lib = _native.lib()
@@ -219,7 +220,7 @@ def test_shared_memory_plans_fit_for_every_read_length():
     planned = 0
     for L in range(4, 300):
         for R in (1, 8):
-            for arrays in (3, 2):
+            for arrays in (3, 2, 3 | 0x100, 2 | 0x100):
                 rc = lib.kbbq_plan_info(L, R, 6, arrays, 0, out)
                 if L > 288:
                     assert rc != 0, (L, R, arrays)     # longer reads take the generic kernels
@@ -233,4 +234,4 @@ def test_shared_memory_plans_fit_for_every_read_length():
                 # two cycle tables of 44 - minscore rows each (row stride a multiple of 128 B covering L cycles)
                 rows, rs = 44 - 6, (4 * ((L + 3) // 4) * 4 + 127) // 128 * 128
                 assert table_bytes >= 2 * rows * rs + rows * 16 * drep * 4, (L, R, arrays)
-    assert planned == 285 * 4
+    assert planned == 285 * 8
