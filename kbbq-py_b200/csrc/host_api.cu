@@ -1,4 +1,5 @@
-// host_api.cu -- host-buffer side of the C ABI: sessions, the whole-path entry points, several GPUs.
+// host_api.cu -- host-buffer side of the C ABI: sessions, the whole-path entry points, several GPUs, and the
+// host-buffer forms of the device-pointer entry points (kbbq_build_host, ...).
 //
 // What recalibrate.recalibrate_fastq (kbbq/recalibrate.py:123-156) does between parsing and printing is two
 // passes over the reads around one small model step.  A SESSION is that path on one device, fed chunk by
@@ -1124,6 +1125,290 @@ int kbbq_recalibrate_host_multi(const uint8_t *seq, const uint8_t *qual, const u
     if (status_out) *status_out = st;
     if (rc) return rc;
     return st ? KBBQ_E_DATA : KBBQ_OK;
+}
+
+}  // extern "C"
+
+// ---- host-buffer forms of the device-pointer entry points: copy in, run, copy back, synchronously ----
+
+namespace {
+
+enum SpanDir { IN, OUT, INOUT, SCRATCH };
+
+// One synchronous call of a device-pointer entry point on host buffers.  The wrapper lists its spans (a host pointer,
+// a byte count, a direction); begin() carves them from one allocation, uploads the IN / INOUT spans and zeroes the OUT
+// spans and the status word; finish() downloads the OUT / INOUT spans and maps a non-zero status to KBBQ_E_DATA.
+// Every span starts 256-byte aligned and is readable up to its 16-byte end, as the TMA ring and the vector
+// calibration kernel need to take their fast paths.  A NULL host pointer gives a NULL device pointer.
+struct HostCall {
+    struct Span {
+        SpanDir dir;
+        void *host;
+        size_t bytes;
+        char *d;
+    };
+    template <class T> struct Dev {  // device pointer of a span, valid once begin() has run
+        const std::vector<Span> *spans;
+        int i;
+        operator T *() const { return i < 0 ? nullptr : (T *)(*spans)[i].d; }
+    };
+
+    int device;
+    bool with_status;
+    std::vector<Span> spans;
+    void *base = nullptr;
+    int *status = nullptr;  // the device status word, with_status only
+
+    HostCall(int device_, bool with_status_) : device(device_), with_status(with_status_) {}
+    HostCall(const HostCall &) = delete;
+    HostCall &operator=(const HostCall &) = delete;
+    ~HostCall() {
+        if (base) cudaFree(base);
+    }
+
+    template <class T> Dev<T> span(SpanDir dir, T *host, size_t bytes) {
+        if (!host && dir != SCRATCH) return {&spans, -1};
+        spans.push_back({dir, (void *)host, bytes, nullptr});
+        return {&spans, (int)spans.size() - 1};
+    }
+    Dev<void> scratch(size_t bytes) { return span<void>(SCRATCH, nullptr, bytes); }
+
+    int begin() {
+        KBBQ_CUDA(cudaSetDevice(device));
+        Carver size(nullptr);
+        for (const Span &s : spans) size.take<char>(s.bytes);
+        if (with_status) size.take<int>(1);
+        KBBQ_CUDA(cudaMalloc(&base, size.off));
+        Carver c(base);
+        for (Span &s : spans) {
+            s.d = c.take<char>(s.bytes);
+            if (!s.bytes) continue;
+            if (s.dir == IN || s.dir == INOUT) KBBQ_CUDA(cudaMemcpy(s.d, s.host, s.bytes, cudaMemcpyHostToDevice));
+            if (s.dir == OUT) KBBQ_CUDA(cudaMemset(s.d, 0, s.bytes));
+        }
+        if (with_status) {
+            status = c.take<int>(1);
+            KBBQ_CUDA(cudaMemset(status, 0, sizeof(int)));
+        }
+        return KBBQ_OK;
+    }
+
+    int finish(int *status_out = nullptr) {
+        for (const Span &s : spans)
+            if (s.bytes && (s.dir == OUT || s.dir == INOUT))
+                KBBQ_CUDA(cudaMemcpy(s.host, s.d, s.bytes, cudaMemcpyDeviceToHost));
+        if (!with_status) return KBBQ_OK;
+        int st = 0;
+        KBBQ_CUDA(cudaMemcpy(&st, status, sizeof(int), cudaMemcpyDeviceToHost));
+        if (status_out) *status_out = st;
+        return st ? KBBQ_E_DATA : KBBQ_OK;
+    }
+};
+
+}  // namespace
+
+extern "C" {
+
+int kbbq_build_host(const uint8_t *seq, const uint8_t *qual, const uint8_t *corr, const uint16_t *rg,
+                    const uint8_t *second, int64_t N, int L, int R, int minscore, int64_t *pos_errs,
+                    int64_t *pos_total, int64_t *din_errs, int64_t *din_total, int *status_out, int device) {
+    if (N < 0 || L < 1 || R < 1 || R > 65535) return KBBQ_E_ARG;
+    if (!pos_errs || !pos_total || !din_errs || !din_total || (N > 0 && (!seq || !qual || !corr))) return KBBQ_E_ARG;
+    const size_t nb = (size_t)N * L, npos = (size_t)R * NQ * 2 * L * 8, ndin = (size_t)R * NQ * 16 * 8;
+    size_t ws_bytes = 0;
+    KBBQ_TRY(kbbq_workspace_bytes(N, L, R, &ws_bytes));
+    HostCall c(device, true);
+    const auto d_seq = c.span(IN, seq, nb);
+    const auto d_qual = c.span(IN, qual, nb);
+    const auto d_corr = c.span(IN, corr, nb);
+    const auto d_rg = c.span(IN, rg, (size_t)N * 2);
+    const auto d_sec = c.span(IN, second, (size_t)N);
+    const auto pe = c.span(OUT, pos_errs, npos);  // fresh tables
+    const auto pt = c.span(OUT, pos_total, npos);
+    const auto de = c.span(OUT, din_errs, ndin);
+    const auto dt = c.span(OUT, din_total, ndin);
+    const auto ws = c.scratch(ws_bytes);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_build(d_seq, d_qual, d_corr, d_rg, d_sec, N, L, R, minscore, pe, pt, de, dt, ws, ws_bytes, c.status, 0,
+                        nullptr));
+    return c.finish(status_out);
+}
+
+int kbbq_apply_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second, int64_t N,
+                    int L, int R, int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
+                    const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual,
+                    int *status_out, int device) {
+    if (N < 0 || L < 1 || R < 1 || R > 65535 || nq < 1 || nq > NQ || ndin1 < 16 || ndin1 > 64) return KBBQ_E_ARG;
+    if (!meanq || !rgdq || !qdq || !posdq || !dindq || (N > 0 && (!seq || !qual || !out_qual))) return KBBQ_E_ARG;
+    const size_t nb = (size_t)N * L, n_q = (size_t)R * nq * 8;
+    size_t ws_bytes = 0;
+    KBBQ_TRY(kbbq_workspace_bytes(N, L, R, &ws_bytes));
+    HostCall c(device, true);
+    const auto d_seq = c.span(IN, seq, nb);
+    const auto d_qual = c.span(IN, qual, nb);
+    const auto d_rg = c.span(IN, rg, (size_t)N * 2);
+    const auto d_sec = c.span(IN, second, (size_t)N);
+    const auto d_meanq = c.span(IN, meanq, (size_t)R * 8);
+    const auto d_rgdq = c.span(IN, rgdq, (size_t)R * 8);
+    const auto d_qdq = c.span(IN, qdq, n_q);
+    const auto d_posdq = c.span(IN, posdq, n_q * 2 * L);
+    const auto d_dindq = c.span(IN, dindq, n_q * ndin1);
+    const auto d_out = c.span(OUT, out_qual, nb);
+    const auto ws = c.scratch(ws_bytes);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_apply(d_seq, d_qual, d_rg, d_sec, N, L, R, minscore, d_meanq, d_rgdq, d_qdq, d_posdq, d_dindq, nq,
+                        ndin1, d_out, ws, ws_bytes, c.status, 0, nullptr));
+    return c.finish(status_out);
+}
+
+int kbbq_get_delta_qs_host(const int64_t *meanq, const int64_t *rg_errs, const int64_t *rg_total,
+                           const int64_t *q_errs, const int64_t *q_total, const int64_t *pos_errs,
+                           const int64_t *pos_total, const int64_t *din_errs, const int64_t *din_total, int R,
+                           int nq, int ncyc, int ndin, int64_t *rgdq, int64_t *qdq, int64_t *posdq,
+                           int64_t *dindq, int device) {
+    if (R < 1 || nq < 1 || ncyc < 0 || ndin < 0) return KBBQ_E_ARG;
+    if (!meanq || !rg_errs || !rg_total || !q_errs || !q_total || !rgdq || !qdq) return KBBQ_E_ARG;
+    if ((ncyc && (!pos_errs || !pos_total || !posdq)) || !dindq || (ndin && (!din_errs || !din_total)))
+        return KBBQ_E_ARG;
+    const size_t nr = (size_t)R * 8, n_q = (size_t)R * nq * 8, n_pos = n_q * ncyc, n_din = n_q * ndin;
+    HostCall c(device, false);
+    const auto d_meanq = c.span(IN, meanq, nr);
+    const auto d_rge = c.span(IN, rg_errs, nr);
+    const auto d_rgt = c.span(IN, rg_total, nr);
+    const auto d_qe = c.span(IN, q_errs, n_q);
+    const auto d_qt = c.span(IN, q_total, n_q);
+    const auto d_pe = c.span(IN, pos_errs, n_pos);
+    const auto d_pt = c.span(IN, pos_total, n_pos);
+    const auto d_de = c.span(IN, din_errs, n_din);
+    const auto d_dt = c.span(IN, din_total, n_din);
+    const auto o_rg = c.span(OUT, rgdq, nr);
+    const auto o_q = c.span(OUT, qdq, n_q);
+    const auto o_pos = c.span(OUT, posdq, n_pos);
+    const auto o_din = c.span(OUT, dindq, n_q * (ndin + 1));
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_get_delta_qs(d_meanq, d_rge, d_rgt, d_qe, d_qt, d_pe, d_pt, d_de, d_dt, R, nq, ncyc, ndin, o_rg, o_q,
+                               o_pos, o_din, nullptr));
+    return c.finish();
+}
+
+int kbbq_delta_q_host(const int64_t *prior_q, const int64_t *numerrs, const int64_t *numtotal, int64_t n,
+                      int64_t *delta, int device) {
+    if (n < 0 || (n > 0 && (!prior_q || !numerrs || !numtotal || !delta))) return KBBQ_E_ARG;
+    if (n == 0) return KBBQ_OK;
+    HostCall c(device, false);
+    const auto d_prior = c.span(IN, prior_q, (size_t)n * 8);
+    const auto d_errs = c.span(IN, numerrs, (size_t)n * 8);
+    const auto d_total = c.span(IN, numtotal, (size_t)n * 8);
+    const auto d_delta = c.span(OUT, delta, (size_t)n * 8);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_delta_q(d_prior, d_errs, d_total, n, d_delta, nullptr));
+    return c.finish();
+}
+
+int kbbq_posterior_q_real_host(const double *prior_q, const int64_t *numerrs, const int64_t *numtotal, int64_t n,
+                               int64_t *posterior, int device) {
+    if (n < 0 || (n > 0 && (!prior_q || !numerrs || !numtotal || !posterior))) return KBBQ_E_ARG;
+    if (n == 0) return KBBQ_OK;
+    HostCall c(device, false);
+    const auto d_prior = c.span(IN, prior_q, (size_t)n * 8);
+    const auto d_errs = c.span(IN, numerrs, (size_t)n * 8);
+    const auto d_total = c.span(IN, numtotal, (size_t)n * 8);
+    const auto d_post = c.span(OUT, posterior, (size_t)n * 8);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_posterior_q_real(d_prior, d_errs, d_total, n, d_post, nullptr));
+    return c.finish();
+}
+
+// Host-buffer forms of the BAM-side entry points: copy, run, copy back (a BAM batch is small next to
+// what the host spends parsing it).
+int kbbq_build_bam_host(const uint8_t *seq, const uint8_t *qual, const uint8_t *err, const uint8_t *skip,
+                        const uint16_t *rg, const uint8_t *flags, const uint16_t *aln_start, const uint16_t *aln_end,
+                        int64_t N, int L, int R, int minscore, int64_t *pos_errs, int64_t *pos_total,
+                        int64_t *din_errs, int64_t *din_total, int *status_out, int device) {
+    if (N < 0 || L < 1 || R < 1 || R > 65535) return KBBQ_E_ARG;
+    if (!pos_errs || !pos_total || !din_errs || !din_total || (N > 0 && (!seq || !qual || !err))) return KBBQ_E_ARG;
+    const size_t nb = (size_t)N * L, npos = (size_t)R * NQ * 2 * L * 8, ndin = (size_t)R * NQ * 16 * 8;
+    size_t ws_bytes = 0;
+    KBBQ_TRY(kbbq_bam_workspace_bytes(N, L, R, &ws_bytes));
+    HostCall c(device, true);
+    const auto d_seq = c.span(IN, seq, nb);
+    const auto d_qual = c.span(IN, qual, nb);
+    const auto d_err = c.span(IN, err, nb);
+    const auto d_skip = c.span(IN, skip, nb);
+    const auto d_rg = c.span(IN, rg, (size_t)N * 2);
+    const auto d_flags = c.span(IN, flags, (size_t)N);
+    const auto d_start = c.span(IN, aln_start, (size_t)N * 2);
+    const auto d_end = c.span(IN, aln_end, (size_t)N * 2);
+    const auto pe = c.span(INOUT, pos_errs, npos);  // the tables accumulate
+    const auto pt = c.span(INOUT, pos_total, npos);
+    const auto de = c.span(INOUT, din_errs, ndin);
+    const auto dt = c.span(INOUT, din_total, ndin);
+    const auto ws = c.scratch(ws_bytes);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_build_bam(d_seq, d_qual, d_err, d_skip, d_rg, d_flags, d_start, d_end, N, L, R, minscore, pe, pt, de,
+                            dt, ws, ws_bytes, c.status, nullptr));
+    return c.finish(status_out);
+}
+
+int kbbq_apply_bam_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *flags, int64_t N,
+                        int L, int R, int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
+                        const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual,
+                        int *status_out, int device) {
+    if (N < 0 || L < 1 || R < 1 || R > 65535 || nq < 1 || ndin1 != 17) return KBBQ_E_ARG;
+    if (!meanq || !rgdq || !qdq || !posdq || !dindq || (N > 0 && (!seq || !qual || !out_qual))) return KBBQ_E_ARG;
+    const size_t nb = (size_t)N * L, n_q = (size_t)R * nq * 8;
+    size_t ws_bytes = 0;
+    KBBQ_TRY(kbbq_bam_workspace_bytes(N, L, R, &ws_bytes));
+    HostCall c(device, true);
+    const auto d_seq = c.span(IN, seq, nb);
+    const auto d_qual = c.span(IN, qual, nb);
+    const auto d_rg = c.span(IN, rg, (size_t)N * 2);
+    const auto d_flags = c.span(IN, flags, (size_t)N);
+    const auto d_meanq = c.span(IN, meanq, (size_t)R * 8);
+    const auto d_rgdq = c.span(IN, rgdq, (size_t)R * 8);
+    const auto d_qdq = c.span(IN, qdq, n_q);
+    const auto d_posdq = c.span(IN, posdq, n_q * 2 * L);
+    const auto d_dindq = c.span(IN, dindq, n_q * ndin1);
+    const auto d_out = c.span(OUT, out_qual, nb);
+    const auto ws = c.scratch(ws_bytes);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_apply_bam(d_seq, d_qual, d_rg, d_flags, N, L, R, minscore, d_meanq, d_rgdq, d_qdq, d_posdq, d_dindq,
+                            nq, ndin1, d_out, ws, ws_bytes, c.status, nullptr));
+    return c.finish(status_out);
+}
+
+int kbbq_calibration_counts_host(const uint8_t *qual, const uint8_t *err, const uint8_t *seq, const uint8_t *corr,
+                                 const uint8_t *skip, int64_t n, int64_t *total, int64_t *errs, int device) {
+    if (n < 0 || !total || !errs || (!err && (!seq || !corr)) || (n > 0 && !qual)) return KBBQ_E_ARG;
+    HostCall c(device, false);
+    const auto d_qual = c.span(IN, qual, (size_t)n);
+    const auto d_err = c.span(IN, err, (size_t)n);
+    const auto d_seq = c.span(IN, err ? nullptr : seq, (size_t)n);  // with an error mask, seq and corr are not read
+    const auto d_corr = c.span(IN, err ? nullptr : corr, (size_t)n);
+    const auto d_skip = c.span(IN, skip, (size_t)n);
+    const auto d_total = c.span(OUT, total, 256 * 8);
+    const auto d_errs = c.span(OUT, errs, 256 * 8);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_calibration_counts(d_qual, d_err, d_seq, d_corr, d_skip, n, d_total, d_errs, nullptr));
+    return c.finish();
+}
+
+int kbbq_marginals_host(const int64_t *pos_errs, const int64_t *pos_total, int L, int R, int64_t *q_errs,
+                        int64_t *q_total, int64_t *rg_errs, int64_t *rg_total, int64_t *meanq, int device) {
+    if (L < 1 || R < 1) return KBBQ_E_ARG;
+    if (!pos_errs || !pos_total || !q_errs || !q_total || !rg_errs || !rg_total || !meanq) return KBBQ_E_ARG;
+    const size_t npos = (size_t)R * NQ * 2 * L * 8, n_q = (size_t)R * NQ * 8, nr = (size_t)R * 8;
+    HostCall c(device, false);
+    const auto pe = c.span(IN, pos_errs, npos);
+    const auto pt = c.span(IN, pos_total, npos);
+    const auto qe = c.span(OUT, q_errs, n_q);
+    const auto qt = c.span(OUT, q_total, n_q);
+    const auto ge = c.span(OUT, rg_errs, nr);
+    const auto gt = c.span(OUT, rg_total, nr);
+    const auto mq = c.span(OUT, meanq, nr);
+    KBBQ_TRY(c.begin());
+    KBBQ_TRY(kbbq_marginals(pe, pt, L, R, qe, qt, ge, gt, mq, nullptr));
+    return c.finish();
 }
 
 }  // extern "C"

@@ -4,11 +4,11 @@
 // kernels take 2 ms).  The corrected reads are only ever compared with the reads
 // (find_corrected_sites, kbbq/recalibrate.py:13-20), so one bit per base carries everything the build
 // needs from them: the host cores reduce (seq, corrected) to a mismatch bit map while the copy engine
-// moves seq and qual, the map (1/8 of the bytes) follows, and expand_corr_kernel (kbbq_b200.cu) turns
+// moves seq and qual, the map (1/8 of the bytes) follows, and expand_corr_kernel (expand.cuh) turns
 // it back into a byte array that differs from seq exactly where the corrected read did.
 // kbbq_host_pack_nibbles goes one step further and folds the read itself into the same pass: 4 bits per
 // base (3-bit base code | mismatch), so that seq + corrected cross PCIe as 0.5 B per base instead of 1.125 and
-// only the qualities travel as they are; expand_nibbles_kernel rebuilds both byte arrays in HBM.
+// only the qualities travel as they are; expand_nibbles_kernel (expand.cuh) rebuilds both byte arrays in HBM.
 // Plain host C++ (no CUDA).  AVX2 when the CPU has it (32 bases per compare + movemask), portable
 // 64-bit SWAR otherwise.
 #include <stddef.h>

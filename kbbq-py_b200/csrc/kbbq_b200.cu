@@ -12,6 +12,7 @@
 #include "build.cuh"
 #include "calib.cuh"
 #include "common.cuh"
+#include "expand.cuh"
 #include "model.cuh"
 #include "prepare.cuh"
 #include "segment.cuh"
@@ -26,7 +27,9 @@ char g_last_cuda_error[256] = "";
 static std::mutex g_const_mu;
 static bool g_const_done[64];
 
-static int upload_constants(int device) {
+static int upload_constants() {
+    int device;
+    KBBQ_CUDA(cudaGetDevice(&device));
     std::lock_guard<std::mutex> lock(g_const_mu);
     if (device >= 0 && device < 64 && g_const_done[device]) return KBBQ_OK;
     KBBQ_CUDA(cudaMemcpyToSymbol(c_lnp, KBBQ_LN_P, sizeof(double) * NQ));
@@ -128,46 +131,84 @@ static bool plan_kernel(int L, int R, int minscore, int narr, int max_smem, Geom
     return false;
 }
 
-template <int KPS>
-static int launch_build_kps(const BuildArgs &a, int grid, size_t smem, cudaStream_t st) {
-    auto kern = build_smem_kernel<KPS, true>;
-    KBBQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, a.g.threads + 32 * a.g.nprod, smem, st>>>(a);  // + the producer warp(s)
+// The shared-memory kernels by groups per thread-group and stage (plan_smem: 1..8); apply also by whether it checks
+// the bases
+static void (*const build_smem_kernels[8])(BuildArgs) = {
+    build_smem_kernel<1, true>, build_smem_kernel<2, true>, build_smem_kernel<3, true>, build_smem_kernel<4, true>,
+    build_smem_kernel<5, true>, build_smem_kernel<6, true>, build_smem_kernel<7, true>, build_smem_kernel<8, true>};
+static void (*const apply_smem_kernels[2][8])(ApplyArgs) = {
+    {apply_smem_kernel<1, false>, apply_smem_kernel<2, false>, apply_smem_kernel<3, false>, apply_smem_kernel<4, false>,
+     apply_smem_kernel<5, false>, apply_smem_kernel<6, false>, apply_smem_kernel<7, false>, apply_smem_kernel<8, false>},
+    {apply_smem_kernel<1, true>, apply_smem_kernel<2, true>, apply_smem_kernel<3, true>, apply_smem_kernel<4, true>,
+     apply_smem_kernel<5, true>, apply_smem_kernel<6, true>, apply_smem_kernel<7, true>, apply_smem_kernel<8, true>}};
+
+template <class Args>
+static int launch_smem(void (*kern)(Args), const Args &a, int grid, cudaStream_t st) {
+    KBBQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.sl.total));
+    kern<<<grid, a.g.threads + 32 * a.g.nprod, a.sl.total, st>>>(a);  // + the producer warp(s)
     KBBQ_LAUNCHED();
     return KBBQ_OK;
-}
-static int launch_build_smem(const BuildArgs &a, int grid, size_t smem, cudaStream_t st) {
-    switch (a.sl.kps) {
-    case 8: return launch_build_kps<8>(a, grid, smem, st);
-    case 7: return launch_build_kps<7>(a, grid, smem, st);
-    case 6: return launch_build_kps<6>(a, grid, smem, st);
-    case 5: return launch_build_kps<5>(a, grid, smem, st);
-    case 4: return launch_build_kps<4>(a, grid, smem, st);
-    case 3: return launch_build_kps<3>(a, grid, smem, st);
-    case 2: return launch_build_kps<2>(a, grid, smem, st);
-    default: return launch_build_kps<1>(a, grid, smem, st);
-    }
 }
 
-template <int KPS>
-static int launch_apply_kps(const ApplyArgs &a, bool validate, int grid, size_t smem, cudaStream_t st) {
-    auto kern = validate ? apply_smem_kernel<KPS, true> : apply_smem_kernel<KPS, false>;
-    KBBQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, a.g.threads + 32 * a.g.nprod, smem, st>>>(a);  // + the producer warp(s)
-    KBBQ_LAUNCHED();
-    return KBBQ_OK;
-}
-static int launch_apply_smem(const ApplyArgs &a, bool validate, int grid, size_t smem, cudaStream_t st) {
-    switch (a.sl.kps) {
-    case 8: return launch_apply_kps<8>(a, validate, grid, smem, st);
-    case 7: return launch_apply_kps<7>(a, validate, grid, smem, st);
-    case 6: return launch_apply_kps<6>(a, validate, grid, smem, st);
-    case 5: return launch_apply_kps<5>(a, validate, grid, smem, st);
-    case 4: return launch_apply_kps<4>(a, validate, grid, smem, st);
-    case 3: return launch_apply_kps<3>(a, validate, grid, smem, st);
-    case 2: return launch_apply_kps<2>(a, validate, grid, smem, st);
-    default: return launch_apply_kps<1>(a, validate, grid, smem, st);
+// What kbbq_build (narr 3) and kbbq_apply (narr 2) share once their arguments are checked: the shared-memory plan,
+// or, when there is none, the generic kernel over the whole batch; then the prepare pass of the shared-memory kernel.
+// generic(r0, n, grid) enqueues the generic kernel over reads [r0, r0 + n).  seg_rows != NULL: a segmented batch of
+// at most N rows (segment.cuh).  On return p->smem says whether the shared-memory kernel is to take reads [0, p->N).
+struct SmemPlan {
+    Geom g;
+    TableCfg tc;
+    StageLayout sl;
+    Workspace w;
+    int sms;
+    int64_t N;
+    bool smem;
+};
+
+template <class Generic>
+static int plan_and_prepare(int narr, bool aligned, int64_t N, int L, int R, int minscore, const uint16_t *rg,
+                            const uint8_t *second, void *workspace, size_t workspace_bytes, int *status, int path,
+                            const unsigned int *seg_rows, cudaStream_t st, const Generic &generic, SmemPlan *p) {
+    const bool segmode = seg_rows != nullptr;
+    int device, max_smem;
+    int rc = current_device_info(&device, &p->sms, &max_smem);
+    if (rc) return rc;
+    p->smem = path != 2 && aligned && plan_kernel(L, R, minscore, narr, max_smem, &p->g, &p->tc, &p->sl, segmode) &&
+              (uint64_t)((N + p->g.G - 1) / p->g.G) < 0xFFFFFFFFull;
+    if (!p->smem) {
+        if (path == 1 || segmode) return KBBQ_E_ARG;
+        return generic(0, N, p->sms * 8);
     }
+    p->w = carve_workspace(workspace, N, L, R);
+    if (!workspace || workspace_bytes < p->w.bytes) return KBBQ_E_WORKSPACE;
+    p->N = N;
+    if (segmode) {
+        seg_prepare_kernel<<<1, 256, 0, st>>>(seg_rows, 2 * R, p->g.G, (unsigned long long)N, p->w.seg, p->w.uni, status);
+        KBBQ_LAUNCHED();
+        return KBBQ_OK;
+    }
+    // One read group: a partial last group would be the only one with untallied rows and cost the
+    // whole batch its header-free fast path; its few reads go through the generic kernel instead.
+    const int64_t tail = (R == 1 && N > p->g.G) ? N % p->g.G : 0;
+    if (tail) {
+        p->N = N - tail;
+        rc = generic(p->N, tail, 1);
+        if (rc) return rc;
+    }
+    return run_prepare(rg, second, p->N, p->g.G, R, p->w, status, p->sms, p->sl.ngs, p->g.gbytes, p->sl.slot, st);
+}
+
+// bam_canon_kernel / bam_uncanon_kernel: one thread per output word; 32-bit thread indices, so very large batches take
+// several launches.  launch(grid, r0, wmax) enqueues the reads from r0 on.
+template <class Launch>
+static int launch_bam_chunks(long long N, int L, const Launch &launch) {
+    const unsigned int wmax = (unsigned int)((3 + L + 3) >> 2);
+    const long long per = std::max<long long>(1, (long long)(0x7FFFFFFFu / wmax) / 256 * 256);  // reads per launch
+    for (long long r0 = 0; r0 < N; r0 += per) {
+        const long long n = std::min<long long>(per, N - r0);
+        launch((unsigned)((n * wmax + BAM_WARPS * 32 - 1) / (BAM_WARPS * 32)), r0, wmax);
+        KBBQ_LAUNCHED();
+    }
+    return KBBQ_OK;
 }
 
 }  // namespace kbbq
@@ -223,7 +264,7 @@ int kbbq_workspace_bytes(int64_t N, int L, int R, size_t *bytes) {
     return KBBQ_OK;
 }
 
-// kbbq_build / kbbq_build_segmented.  seg_rows != NULL: a segmented batch of at most N rows (segment.cuh).
+// kbbq_build / kbbq_build_segmented
 static int build_impl(const uint8_t *seq, const uint8_t *qual, const uint8_t *corr, const uint16_t *rg,
                       const uint8_t *second, int64_t N, int L, int R, int minscore, int64_t *pos_errs,
                       int64_t *pos_total, int64_t *din_errs, int64_t *din_total, void *workspace,
@@ -234,57 +275,30 @@ static int build_impl(const uint8_t *seq, const uint8_t *qual, const uint8_t *co
     if (!seq || !qual || !corr) return KBBQ_E_ARG;
     const bool segmode = seg_rows != nullptr;
     cudaStream_t st = (cudaStream_t)stream;
-    int device, sms, max_smem;
-    int rc = current_device_info(&device, &sms, &max_smem);
-    if (rc) return rc;
-
-    Geom g;
-    TableCfg tc;
-    StageLayout sl;
-    const bool smem_ok = path != 2 && !misaligned(seq, 16) && !misaligned(qual, 16) && !misaligned(corr, 16) &&
-                         plan_kernel(L, R, minscore, 3, max_smem, &g, &tc, &sl, segmode) &&
-                         (uint64_t)((N + g.G - 1) / g.G) < 0xFFFFFFFFull;
-    if (!smem_ok) {
-        if (path == 1 || segmode) return KBBQ_E_ARG;
-        BuildGenericArgs a = {seq, qual, corr, rg, second, N, L, R, minscore,
+    auto generic = [&](int64_t r0, int64_t n, int grid) {
+        BuildGenericArgs a = {seq + r0 * L, qual + r0 * L, corr + r0 * L, rg ? rg + r0 : nullptr,
+                              second ? second + r0 : nullptr, n, L, R, minscore,
                               (unsigned long long *)pos_errs, (unsigned long long *)pos_total,
                               (unsigned long long *)din_errs, (unsigned long long *)din_total, status};
-        build_generic_kernel<<<sms * 8, 256, 0, st>>>(a);
+        build_generic_kernel<<<grid, 256, 0, st>>>(a);
         KBBQ_LAUNCHED();
         return KBBQ_OK;
-    }
-    Workspace w = carve_workspace(workspace, N, L, R);
-    if (!workspace || workspace_bytes < w.bytes) return KBBQ_E_WORKSPACE;
-    if (segmode) {
-        seg_prepare_kernel<<<1, 256, 0, st>>>(seg_rows, 2 * R, g.G, (unsigned long long)N, w.seg, w.uni, status);
-        KBBQ_LAUNCHED();
-    } else {
-        // One read group: a partial last group would be the only one with untallied rows and cost the
-        // whole batch its header-free fast path; its few reads go through the generic kernel instead.
-        const int64_t tail = (R == 1 && N > g.G) ? N % g.G : 0;
-        if (tail) {
-            const int64_t n0 = N - tail;
-            BuildGenericArgs ga = {seq + n0 * L, qual + n0 * L, corr + n0 * L, rg ? rg + n0 : nullptr,
-                                   second ? second + n0 : nullptr, tail, L, R, minscore,
-                                   (unsigned long long *)pos_errs, (unsigned long long *)pos_total,
-                                   (unsigned long long *)din_errs, (unsigned long long *)din_total, status};
-            build_generic_kernel<<<1, 256, 0, st>>>(ga);
-            KBBQ_LAUNCHED();
-            N = n0;
-        }
-        rc = run_prepare(rg, second, N, g.G, R, w, status, sms, sl.ngs, g.gbytes, sl.slot, st);
-        if (rc) return rc;
-    }
+    };
+    const bool aligned = !misaligned(seq, 16) && !misaligned(qual, 16) && !misaligned(corr, 16);
+    SmemPlan p;
+    int rc = plan_and_prepare(3, aligned, N, L, R, minscore, rg, second, workspace, workspace_bytes, status, path,
+                              seg_rows, st, generic, &p);
+    if (rc || !p.smem) return rc;
 
     BuildArgs a;
-    a.seq = seq; a.qual = qual; a.corr = corr; a.total_bytes = N * L; a.g = g; a.t = tc; a.R = R;
+    a.seq = seq; a.qual = qual; a.corr = corr; a.total_bytes = p.N * L; a.g = p.g; a.t = p.tc; a.R = R;
     a.nsub = segmode ? 2 * R : R; a.segmode = segmode ? 1 : 0;
-    a.sl = sl;
-    a.entries = w.entries; a.seg = w.seg; a.uni = w.uni;
+    a.sl = p.sl;
+    a.entries = p.w.entries; a.seg = p.w.seg; a.uni = p.w.uni;
     a.pos_errs = (unsigned long long *)pos_errs; a.pos_total = (unsigned long long *)pos_total;
     a.din_errs = (unsigned long long *)din_errs; a.din_total = (unsigned long long *)din_total;
     a.status = status;
-    return launch_build_smem(a, sms, a.sl.total, st);
+    return launch_smem(build_smem_kernels[a.sl.kps - 1], a, p.sms, st);
 }
 
 int kbbq_build(const uint8_t *seq, const uint8_t *qual, const uint8_t *corr, const uint16_t *rg,
@@ -309,9 +323,7 @@ int kbbq_marginals(const int64_t *pos_errs, const int64_t *pos_total, int L, int
     if (L < 1 || R < 1 || !pos_errs || !pos_total || !q_errs || !q_total || !rg_errs || !rg_total || !meanq)
         return KBBQ_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    int device;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    int rc = upload_constants(device);
+    int rc = upload_constants();
     if (rc) return rc;
     marginals_q_kernel<<<dim3(NQ, R), 128, 0, st>>>((const long long *)pos_errs, (const long long *)pos_total,
                                                    2 * L, (long long *)q_errs, (long long *)q_total);
@@ -326,9 +338,7 @@ int kbbq_delta_q(const int64_t *prior_q, const int64_t *numerrs, const int64_t *
                  int64_t *delta, void *stream) {
     if (n < 0 || (n > 0 && (!prior_q || !numerrs || !numtotal || !delta))) return KBBQ_E_ARG;
     if (n == 0) return KBBQ_OK;
-    int device;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    int rc = upload_constants(device);
+    int rc = upload_constants();
     if (rc) return rc;
     delta_q_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
         (const long long *)prior_q, (const long long *)numerrs, (const long long *)numtotal, n, (long long *)delta);
@@ -340,9 +350,7 @@ int kbbq_posterior_q_real(const double *prior_q, const int64_t *numerrs, const i
                           int64_t *posterior, void *stream) {
     if (n < 0 || (n > 0 && (!prior_q || !numerrs || !numtotal || !posterior))) return KBBQ_E_ARG;
     if (n == 0) return KBBQ_OK;
-    int device;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    int rc = upload_constants(device);
+    int rc = upload_constants();
     if (rc) return rc;
     posterior_q_real_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
         prior_q, (const long long *)numerrs, (const long long *)numtotal, n, (long long *)posterior);
@@ -372,18 +380,6 @@ static BamWorkspace carve_bam_workspace(void *base, long long N, int L, int R) {
     return w;
 }
 
-// one thread per output word; 32-bit thread indices, so very large batches take several launches
-static int launch_bam_canon(const BamCanonArgs &c, cudaStream_t st) {
-    const unsigned int wmax = (unsigned int)((3 + c.L + 3) >> 2);
-    const long long per = std::max<long long>(1, (long long)(0x7FFFFFFFu / wmax) / 256 * 256);
-    for (long long r0 = 0; r0 < c.N; r0 += per) {
-        const long long n = std::min<long long>(per, c.N - r0);
-        bam_canon_kernel<<<(unsigned)((n * wmax + BAM_WARPS * 32 - 1) / (BAM_WARPS * 32)), BAM_WARPS * 32, 0, st>>>(c, r0, wmax);
-        KBBQ_LAUNCHED();
-    }
-    return KBBQ_OK;
-}
-
 int kbbq_bam_workspace_bytes(int64_t N, int L, int R, size_t *bytes) {
     if (N < 0 || L < 1 || R < 1 || R > 65535 || !bytes) return KBBQ_E_ARG;
     *bytes = carve_bam_workspace(nullptr, N, L, R).bytes;
@@ -398,9 +394,9 @@ int kbbq_build_bam(const uint8_t *seq, const uint8_t *qual, const uint8_t *err, 
     if (!pos_errs || !pos_total || !din_errs || !din_total || !status) return KBBQ_E_ARG;
     if (N == 0) return KBBQ_OK;
     if (!seq || !qual || !err) return KBBQ_E_ARG;
-    int device, sms = KBBQ_SM_COUNT_FALLBACK;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const long long blocks = std::min<long long>(((long long)N * L + 255) / 256, (long long)sms * 16);
     if (workspace && minscore >= 1) {  // canonical form + the shared-memory build kernel
@@ -410,7 +406,10 @@ int kbbq_build_bam(const uint8_t *seq, const uint8_t *qual, const uint8_t *err, 
                           w.cseq, w.cqual, w.cthird, w.csecond,
                           (unsigned long long *)pos_errs, (unsigned long long *)pos_total,
                           (unsigned long long *)din_errs, (unsigned long long *)din_total, status};
-        { const int rc_ = launch_bam_canon(c, st); if (rc_) return rc_; }
+        rc = launch_bam_chunks(N, L, [&](unsigned grid, long long r0, unsigned wmax) {
+            bam_canon_kernel<<<grid, BAM_WARPS * 32, 0, st>>>(c, r0, wmax);
+        });
+        if (rc) return rc;
         return kbbq_build(w.cseq, w.cqual, w.cthird, rg, w.csecond, N, L, R, minscore, pos_errs, pos_total, din_errs,
                           din_total, w.inner, w.inner_bytes, status, 0, stream);
     }
@@ -433,9 +432,9 @@ int kbbq_apply_bam(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, 
     if (!meanq || !rgdq || !qdq || !posdq || !dindq || !status) return KBBQ_E_ARG;
     if (N == 0) return KBBQ_OK;
     if (!seq || !qual || !out_qual) return KBBQ_E_ARG;
-    int device, sms = KBBQ_SM_COUNT_FALLBACK;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const long long blocks = std::min<long long>(((long long)N * L + 255) / 256, (long long)sms * 16);
     if (workspace && minscore >= 1 && nq <= NQ) {  // canonical form + the shared-memory apply kernel + flip back
@@ -443,22 +442,17 @@ int kbbq_apply_bam(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, 
         if (workspace_bytes < w.bytes) return KBBQ_E_WORKSPACE;
         BamCanonArgs c = {seq, qual, nullptr, nullptr, rg, flags, nullptr, nullptr, N, L, R, minscore, nq, false,
                           w.cseq, w.cqual, nullptr, w.csecond, nullptr, nullptr, nullptr, nullptr, status};
-        { const int rc_ = launch_bam_canon(c, st); if (rc_) return rc_; }
-        // the canonical reads hold A, C, G, T, N only: bam_canon_kernel has already applied the reference's rule
-        int rc = kbbq_apply(w.cseq, w.cqual, rg, w.csecond, N, L, R, minscore, meanq, rgdq, qdq, posdq, dindq, nq, ndin1,
-                            w.cthird, w.inner, w.inner_bytes, status, KBBQ_APPLY_BASES_CHECKED, stream);
+        rc = launch_bam_chunks(N, L, [&](unsigned grid, long long r0, unsigned wmax) {
+            bam_canon_kernel<<<grid, BAM_WARPS * 32, 0, st>>>(c, r0, wmax);
+        });
         if (rc) return rc;
-        {
-            const unsigned int wmax = (unsigned int)((3 + L + 3) >> 2);
-            const long long per = std::max<long long>(1, (long long)(0x7FFFFFFFu / wmax) / 256 * 256);  // reads per launch
-            for (long long r0 = 0; r0 < N; r0 += per) {
-                const long long n = std::min<long long>(per, N - r0);
-                bam_uncanon_kernel<<<(unsigned)((n * wmax + BAM_WARPS * 32 - 1) / (BAM_WARPS * 32)), BAM_WARPS * 32, 0, st>>>(
-                    w.cthird, flags, N, L, out_qual, r0, wmax);
-                KBBQ_LAUNCHED();
-            }
-        }
-        return KBBQ_OK;
+        // the canonical reads hold A, C, G, T, N only: bam_canon_kernel has already applied the reference's rule
+        rc = kbbq_apply(w.cseq, w.cqual, rg, w.csecond, N, L, R, minscore, meanq, rgdq, qdq, posdq, dindq, nq, ndin1,
+                        w.cthird, w.inner, w.inner_bytes, status, KBBQ_APPLY_BASES_CHECKED, stream);
+        if (rc) return rc;
+        return launch_bam_chunks(N, L, [&](unsigned grid, long long r0, unsigned wmax) {
+            bam_uncanon_kernel<<<grid, BAM_WARPS * 32, 0, st>>>(w.cthird, flags, N, L, out_qual, r0, wmax);
+        });
     }
     ApplyBamArgs a = {seq, qual, rg, flags, out_qual, N, L, R, minscore, nq, ndin1, (const long long *)meanq,
                       (const long long *)rgdq, (const long long *)qdq, (const long long *)posdq,
@@ -474,9 +468,9 @@ int kbbq_calibration_counts(const uint8_t *qual, const uint8_t *err, const uint8
     if (n == 0) return KBBQ_OK;
     if (!qual || (!err && (!seq || !corr))) return KBBQ_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    int device, sms = KBBQ_SM_COUNT_FALLBACK;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
     auto misaligned = [](const void *p) { return p && ((uintptr_t)p & 15u); };
     CalibArgs a = {qual, err, seq, corr, skip, n, (unsigned long long *)total, (unsigned long long *)errs};
     if (misaligned(qual) || misaligned(err) || misaligned(skip) || (!err && (misaligned(seq) || misaligned(corr)))) {
@@ -514,9 +508,7 @@ int kbbq_get_delta_qs(const int64_t *meanq, const int64_t *rg_errs, const int64_
     if (!meanq || !rg_errs || !rg_total || !q_errs || !q_total || !rgdq || !qdq) return KBBQ_E_ARG;
     if ((ncyc && (!pos_errs || !pos_total || !posdq)) || !dindq || (ndin && (!din_errs || !din_total)))
         return KBBQ_E_ARG;
-    int device;
-    KBBQ_CUDA(cudaGetDevice(&device));
-    int rc = upload_constants(device);
+    int rc = upload_constants();
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     DeltaArgs a = {(const long long *)meanq, (const long long *)rg_errs, (const long long *)rg_total,
@@ -545,9 +537,6 @@ static int apply_impl(const uint8_t *seq, const uint8_t *qual, const uint16_t *r
     if (N == 0) return KBBQ_OK;
     if (!seq || !qual || !out_qual) return KBBQ_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    int device, sms, max_smem;
-    int rc = current_device_info(&device, &sms, &max_smem);
-    if (rc) return rc;
     Workspace w = carve_workspace(workspace, N, L, R);
     if (!workspace || workspace_bytes < w.bytes) return KBBQ_E_WORKSPACE;
 
@@ -557,41 +546,25 @@ static int apply_impl(const uint8_t *seq, const uint8_t *qual, const uint16_t *r
         (const long long *)dindq, R, nq, 2 * L, ndin1, w.fold_cyc, w.fold_din);
     KBBQ_LAUNCHED();
 
-    Geom g;
-    TableCfg tc;
-    StageLayout sl;
-    const bool smem_ok = path != 2 && !misaligned(seq, 16) && !misaligned(qual, 16) && !misaligned(out_qual, 4) &&
-                         plan_kernel(L, R, minscore, 2, max_smem, &g, &tc, &sl, segmode) &&
-                         (uint64_t)((N + g.G - 1) / g.G) < 0xFFFFFFFFull;
-    if (!smem_ok) {
-        if (path == 1 || segmode) return KBBQ_E_ARG;
-        ApplyGenericArgs a = {seq, qual, rg, second, out_qual, N, L, R, minscore, nq, w.fold_cyc, w.fold_din, status, validate};
-        apply_generic_kernel<<<sms * 8, 256, 0, st>>>(a);
+    auto generic = [&](int64_t r0, int64_t n, int grid) {
+        ApplyGenericArgs a = {seq + r0 * L, qual + r0 * L, rg ? rg + r0 : nullptr, second ? second + r0 : nullptr,
+                              out_qual + r0 * L, n, L, R, minscore, nq, w.fold_cyc, w.fold_din, status, validate};
+        apply_generic_kernel<<<grid, 256, 0, st>>>(a);
         KBBQ_LAUNCHED();
         return KBBQ_OK;
-    }
-    const int64_t tail = (!segmode && R == 1 && N > g.G) ? N % g.G : 0;  // see kbbq_build
-    if (tail) {
-        const int64_t n0 = N - tail;
-        ApplyGenericArgs ga = {seq + n0 * L, qual + n0 * L, rg ? rg + n0 : nullptr, second ? second + n0 : nullptr,
-                               out_qual + n0 * L, tail, L, R, minscore, nq, w.fold_cyc, w.fold_din, status, validate};
-        apply_generic_kernel<<<1, 256, 0, st>>>(ga);
-        KBBQ_LAUNCHED();
-        N = n0;
-    }
-    if (segmode) {
-        seg_prepare_kernel<<<1, 256, 0, st>>>(seg_rows, 2 * R, g.G, (unsigned long long)N, w.seg, w.uni, status);
-        KBBQ_LAUNCHED();
-    } else {
-        rc = run_prepare(rg, second, N, g.G, R, w, status, sms, sl.ngs, g.gbytes, sl.slot, st);
-        if (rc) return rc;
-    }
+    };
+    const bool aligned = !misaligned(seq, 16) && !misaligned(qual, 16) && !misaligned(out_qual, 4);
+    SmemPlan p;
+    int rc = plan_and_prepare(2, aligned, N, L, R, minscore, rg, second, workspace, workspace_bytes, status, path,
+                              seg_rows, st, generic, &p);
+    if (rc || !p.smem) return rc;
+
     ApplyArgs a;
     a.nsub = segmode ? 2 * R : R; a.segmode = segmode ? 1 : 0;
-    a.seq = seq; a.qual = qual; a.out = out_qual; a.total_bytes = N * L; a.g = g; a.t = tc; a.R = R; a.nq = nq;
-    a.sl = sl;
+    a.seq = seq; a.qual = qual; a.out = out_qual; a.total_bytes = p.N * L; a.g = p.g; a.t = p.tc; a.R = R; a.nq = nq;
+    a.sl = p.sl;
     a.entries = w.entries; a.seg = w.seg; a.uni = w.uni; a.fold_cyc = w.fold_cyc; a.fold_din = w.fold_din; a.status = status;
-    return launch_apply_smem(a, validate, sms, a.sl.total, st);
+    return launch_smem(apply_smem_kernels[validate][a.sl.kps - 1], a, p.sms, st);
 }
 
 int kbbq_apply(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second, int64_t N,
@@ -706,100 +679,6 @@ int kbbq_synth_reads(uint64_t seed, int64_t first_read, int64_t n, int L, int R,
     return KBBQ_OK;
 }
 
-// ------------------------------------------------------------------------------------------------
-// Host-buffer entry points
-// ------------------------------------------------------------------------------------------------
-
-}  // extern "C"
-
-namespace {
-
-struct DevBuf {
-    void *p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    int alloc(size_t n) { KBBQ_CUDA(cudaMalloc(&p, n ? n : 1)); return KBBQ_OK; }
-    template <class T> T *as() { return (T *)p; }
-};
-
-// corr[i] = seq[i] ^ bit i of the mismatch map: a byte array that differs from seq exactly where the
-// corrected read did (host_pack.cpp), which is all the build kernel looks at.  16 bases per thread.
-__global__ void expand_corr_kernel(const uint8_t *seq, const uint32_t *bits, uint8_t *corr, long long n) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long i = t * 16;
-    if (i >= n) return;
-    const uint32_t m = (bits[t >> 1] >> ((t & 1) * 16)) & 0xFFFFu;
-    if (i + 16 <= n) {
-        uint4 v = *reinterpret_cast<const uint4 *>(seq + i);
-        // bits 0..3 of a nibble -> bit 0 of bytes 0..3
-        v.x ^= ((m & 0xFu) * 0x00204081u) & 0x01010101u;
-        v.y ^= (((m >> 4) & 0xFu) * 0x00204081u) & 0x01010101u;
-        v.z ^= (((m >> 8) & 0xFu) * 0x00204081u) & 0x01010101u;
-        v.w ^= (((m >> 12) & 0xFu) * 0x00204081u) & 0x01010101u;
-        *reinterpret_cast<uint4 *>(corr + i) = v;
-    } else {
-        for (int j = 0; i + j < n; ++j) corr[i + j] = seq[i + j] ^ (uint8_t)((m >> j) & 1u);
-    }
-}
-
-// The 4-bit form of (seq, corrected) (host_pack.cpp: kbbq_host_pack_nibbles) back into two byte arrays: seq from
-// the 3-bit base code through a byte-permute table, corr = seq ^ 1 where bit 3 of the nibble says the corrected
-// read differed.  32 bases per thread: one 16-byte load, two 16-byte stores per array.
-__device__ __forceinline__ void expand_nibbles4(uint32_t p16, uint32_t &sw, uint32_t &cw) {
-    // four nibbles = the four selector nibbles of a byte permute over {A C T G | . . . N}
-    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(sw) : "r"(0x47544341u), "r"(0x4E000000u), "r"(p16 & 0x7777u));
-    // bit 3 of nibbles 1, 3 are the sign bits of bytes 0, 1 of p16; those of nibbles 0, 2 after a shift by 4
-    const uint32_t w = (p16 & 0xFFFFu) | (p16 << 20);
-    uint32_t m;
-    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(m) : "r"(w), "r"(0u), "r"(0x9B8Au));
-    cw = sw ^ (m & 0x01010101u);
-}
-
-__global__ void expand_nibbles_kernel(const uint8_t *packed, uint8_t *seq, uint8_t *corr, long long n) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long i = t * 32;
-    if (i >= n) return;
-    if (i + 32 <= n) {
-        const uint4 v = *reinterpret_cast<const uint4 *>(packed + i / 2);
-        const uint32_t in[4] = {v.x, v.y, v.z, v.w};
-        uint32_t s[8], c[8];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            expand_nibbles4(in[k] & 0xFFFFu, s[2 * k], c[2 * k]);
-            expand_nibbles4(in[k] >> 16, s[2 * k + 1], c[2 * k + 1]);
-        }
-        *reinterpret_cast<uint4 *>(seq + i) = make_uint4(s[0], s[1], s[2], s[3]);
-        *reinterpret_cast<uint4 *>(seq + i + 16) = make_uint4(s[4], s[5], s[6], s[7]);
-        *reinterpret_cast<uint4 *>(corr + i) = make_uint4(c[0], c[1], c[2], c[3]);
-        *reinterpret_cast<uint4 *>(corr + i + 16) = make_uint4(c[4], c[5], c[6], c[7]);
-    } else {
-        for (long long j = i; j < n; ++j) {
-            const uint32_t nib = (packed[j >> 1] >> ((j & 1) * 4)) & 0xFu;
-            const uint32_t code = nib & 7u;
-            const uint8_t b = code == 7u ? 'N' : code == 0u ? 'A' : code == 1u ? 'C' : code == 2u ? 'T' : code == 3u ? 'G' : 0;
-            seq[j] = b;
-            corr[j] = b ^ (uint8_t)(nib >> 3);
-        }
-    }
-}
-
-// bump allocator over one device allocation (first pass with base == nullptr measures)
-struct Carver {
-    char *base;
-    size_t off = 0;
-    explicit Carver(void *b) : base((char *)b) {}
-    template <class T> T *take(size_t n_elems) {
-        T *p = base ? (T *)(base + off) : nullptr;
-        off = (off + n_elems * sizeof(T) + 255) / 256 * 256;
-        return p;
-    }
-};
-
-#define KBBQ_TRY(x) do { int rc_ = (x); if (rc_) return rc_; } while (0)
-
-}  // namespace
-
-extern "C" {
-
 int kbbq_expand_mismatch_bits(const uint8_t *seq, const uint32_t *bits, int64_t n, uint8_t *corr, void *stream) {
     if (n < 0 || (n > 0 && (!seq || !bits || !corr))) return KBBQ_E_ARG;
     if (n == 0) return KBBQ_OK;
@@ -815,286 +694,6 @@ int kbbq_expand_nibbles(const uint8_t *packed, int64_t n, uint8_t *seq, uint8_t 
     if (((uintptr_t)packed | (uintptr_t)seq | (uintptr_t)corr) & 15u) return KBBQ_E_ARG;
     expand_nibbles_kernel<<<(unsigned)((n + 32 * 256 - 1) / (32 * 256)), 256, 0, (cudaStream_t)stream>>>(packed, seq, corr, n);
     KBBQ_LAUNCHED();
-    return KBBQ_OK;
-}
-
-int kbbq_build_host(const uint8_t *seq, const uint8_t *qual, const uint8_t *corr, const uint16_t *rg,
-                    const uint8_t *second, int64_t N, int L, int R, int minscore, int64_t *pos_errs,
-                    int64_t *pos_total, int64_t *din_errs, int64_t *din_total, int *status_out, int device) {
-    if (N < 0 || L < 1 || R < 1 || R > 65535) return KBBQ_E_ARG;
-    if (!pos_errs || !pos_total || !din_errs || !din_total) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t npos = (size_t)R * NQ * 2 * L, ndin = (size_t)R * NQ * 16, nb = (size_t)N * L;
-    DevBuf d_seq, d_qual, d_corr, d_rg, d_sec, d_tab, d_ws, d_status;
-    KBBQ_TRY(d_seq.alloc(nb)); KBBQ_TRY(d_qual.alloc(nb)); KBBQ_TRY(d_corr.alloc(nb));
-    KBBQ_TRY(d_tab.alloc((2 * npos + 2 * ndin) * 8));
-    KBBQ_TRY(d_status.alloc(sizeof(int)));
-    size_t ws_bytes = 0;
-    KBBQ_TRY(kbbq_workspace_bytes(N, L, R, &ws_bytes));
-    KBBQ_TRY(d_ws.alloc(ws_bytes));
-    KBBQ_CUDA(cudaMemcpy(d_seq.p, seq, nb, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_qual.p, qual, nb, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_corr.p, corr, nb, cudaMemcpyHostToDevice));
-    if (rg) { KBBQ_TRY(d_rg.alloc((size_t)N * 2)); KBBQ_CUDA(cudaMemcpy(d_rg.p, rg, (size_t)N * 2, cudaMemcpyHostToDevice)); }
-    if (second) { KBBQ_TRY(d_sec.alloc((size_t)N)); KBBQ_CUDA(cudaMemcpy(d_sec.p, second, (size_t)N, cudaMemcpyHostToDevice)); }
-    KBBQ_CUDA(cudaMemset(d_tab.p, 0, (2 * npos + 2 * ndin) * 8));
-    KBBQ_CUDA(cudaMemset(d_status.p, 0, sizeof(int)));
-    int64_t *pe = d_tab.as<int64_t>(), *pt = pe + npos, *de = pt + npos, *dt = de + ndin;
-    KBBQ_TRY(kbbq_build(d_seq.as<uint8_t>(), d_qual.as<uint8_t>(), d_corr.as<uint8_t>(), rg ? d_rg.as<uint16_t>() : nullptr,
-                        second ? d_sec.as<uint8_t>() : nullptr, N, L, R, minscore, pe, pt, de, dt, d_ws.p, ws_bytes,
-                        d_status.as<int>(), 0, nullptr));
-    KBBQ_CUDA(cudaMemcpy(pos_errs, pe, npos * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(pos_total, pt, npos * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(din_errs, de, ndin * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(din_total, dt, ndin * 8, cudaMemcpyDeviceToHost));
-    int st_host = 0;
-    KBBQ_CUDA(cudaMemcpy(&st_host, d_status.p, sizeof(int), cudaMemcpyDeviceToHost));
-    if (status_out) *status_out = st_host;
-    return st_host ? KBBQ_E_DATA : KBBQ_OK;
-}
-
-int kbbq_apply_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second, int64_t N,
-                    int L, int R, int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
-                    const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual,
-                    int *status_out, int device) {
-    if (N < 0 || L < 1 || R < 1 || R > 65535 || nq < 1 || nq > NQ || ndin1 < 16 || ndin1 > 64) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t nb = (size_t)N * L;
-    const size_t n_q = (size_t)R * nq, n_pos = n_q * 2 * L, n_din = n_q * ndin1;
-    DevBuf d_seq, d_qual, d_out, d_rg, d_sec, d_dq, d_ws, d_status;
-    KBBQ_TRY(d_seq.alloc(nb)); KBBQ_TRY(d_qual.alloc(nb)); KBBQ_TRY(d_out.alloc(nb));
-    KBBQ_TRY(d_dq.alloc((2 * (size_t)R + n_q + n_pos + n_din) * 8));
-    KBBQ_TRY(d_status.alloc(sizeof(int)));
-    size_t ws_bytes = 0;
-    KBBQ_TRY(kbbq_workspace_bytes(N, L, R, &ws_bytes));
-    KBBQ_TRY(d_ws.alloc(ws_bytes));
-    int64_t *d_meanq = d_dq.as<int64_t>(), *d_rgdq = d_meanq + R, *d_qdq = d_rgdq + R, *d_posdq = d_qdq + n_q,
-            *d_dindq = d_posdq + n_pos;
-    KBBQ_CUDA(cudaMemcpy(d_seq.p, seq, nb, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_qual.p, qual, nb, cudaMemcpyHostToDevice));
-    if (rg) { KBBQ_TRY(d_rg.alloc((size_t)N * 2)); KBBQ_CUDA(cudaMemcpy(d_rg.p, rg, (size_t)N * 2, cudaMemcpyHostToDevice)); }
-    if (second) { KBBQ_TRY(d_sec.alloc((size_t)N)); KBBQ_CUDA(cudaMemcpy(d_sec.p, second, (size_t)N, cudaMemcpyHostToDevice)); }
-    KBBQ_CUDA(cudaMemcpy(d_meanq, meanq, (size_t)R * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_rgdq, rgdq, (size_t)R * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_qdq, qdq, n_q * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_posdq, posdq, n_pos * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(d_dindq, dindq, n_din * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemset(d_status.p, 0, sizeof(int)));
-    KBBQ_TRY(kbbq_apply(d_seq.as<uint8_t>(), d_qual.as<uint8_t>(), rg ? d_rg.as<uint16_t>() : nullptr,
-                        second ? d_sec.as<uint8_t>() : nullptr, N, L, R, minscore, d_meanq, d_rgdq, d_qdq, d_posdq,
-                        d_dindq, nq, ndin1, d_out.as<uint8_t>(), d_ws.p, ws_bytes, d_status.as<int>(), 0, nullptr));
-    KBBQ_CUDA(cudaMemcpy(out_qual, d_out.p, nb, cudaMemcpyDeviceToHost));
-    int st_host = 0;
-    KBBQ_CUDA(cudaMemcpy(&st_host, d_status.p, sizeof(int), cudaMemcpyDeviceToHost));
-    if (status_out) *status_out = st_host;
-    return st_host ? KBBQ_E_DATA : KBBQ_OK;
-}
-
-int kbbq_get_delta_qs_host(const int64_t *meanq, const int64_t *rg_errs, const int64_t *rg_total,
-                           const int64_t *q_errs, const int64_t *q_total, const int64_t *pos_errs,
-                           const int64_t *pos_total, const int64_t *din_errs, const int64_t *din_total, int R,
-                           int nq, int ncyc, int ndin, int64_t *rgdq, int64_t *qdq, int64_t *posdq,
-                           int64_t *dindq, int device) {
-    if (R < 1 || nq < 1 || ncyc < 0 || ndin < 0) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t n_q = (size_t)R * nq, n_pos = n_q * ncyc, n_din = n_q * ndin, n_din1 = n_q * (ndin + 1);
-    const size_t in_elems = 3 * (size_t)R + 2 * n_q + 2 * n_pos + 2 * n_din;
-    const size_t out_elems = (size_t)R + n_q + n_pos + n_din1;
-    DevBuf d;
-    KBBQ_TRY(d.alloc((in_elems + out_elems) * 8));
-    int64_t *p = d.as<int64_t>();
-    int64_t *d_meanq = p; p += R;
-    int64_t *d_rge = p; p += R;
-    int64_t *d_rgt = p; p += R;
-    int64_t *d_qe = p; p += n_q;
-    int64_t *d_qt = p; p += n_q;
-    int64_t *d_pe = p; p += n_pos;
-    int64_t *d_pt = p; p += n_pos;
-    int64_t *d_de = p; p += n_din;
-    int64_t *d_dt = p; p += n_din;
-    int64_t *o_rg = p; p += R;
-    int64_t *o_q = p; p += n_q;
-    int64_t *o_pos = p; p += n_pos;
-    int64_t *o_din = p;
-    const struct { int64_t *dst; const int64_t *src; size_t n; } ups[] = {
-        {d_meanq, meanq, (size_t)R}, {d_rge, rg_errs, (size_t)R}, {d_rgt, rg_total, (size_t)R}, {d_qe, q_errs, n_q},
-        {d_qt, q_total, n_q}, {d_pe, pos_errs, n_pos}, {d_pt, pos_total, n_pos}, {d_de, din_errs, n_din},
-        {d_dt, din_total, n_din}};
-    for (auto &u : ups)
-        if (u.n) KBBQ_CUDA(cudaMemcpy(u.dst, u.src, u.n * 8, cudaMemcpyHostToDevice));
-    KBBQ_TRY(kbbq_get_delta_qs(d_meanq, d_rge, d_rgt, d_qe, d_qt, d_pe, d_pt, d_de, d_dt, R, nq, ncyc, ndin, o_rg, o_q,
-                               o_pos, o_din, nullptr));
-    KBBQ_CUDA(cudaMemcpy(rgdq, o_rg, (size_t)R * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(qdq, o_q, n_q * 8, cudaMemcpyDeviceToHost));
-    if (n_pos) KBBQ_CUDA(cudaMemcpy(posdq, o_pos, n_pos * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(dindq, o_din, n_din1 * 8, cudaMemcpyDeviceToHost));
-    return KBBQ_OK;
-}
-
-int kbbq_delta_q_host(const int64_t *prior_q, const int64_t *numerrs, const int64_t *numtotal, int64_t n,
-                      int64_t *delta, int device) {
-    if (n < 0) return KBBQ_E_ARG;
-    if (n == 0) return KBBQ_OK;
-    KBBQ_CUDA(cudaSetDevice(device));
-    DevBuf d;
-    KBBQ_TRY(d.alloc((size_t)n * 4 * 8));
-    int64_t *p = d.as<int64_t>();
-    KBBQ_CUDA(cudaMemcpy(p, prior_q, (size_t)n * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(p + n, numerrs, (size_t)n * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(p + 2 * n, numtotal, (size_t)n * 8, cudaMemcpyHostToDevice));
-    KBBQ_TRY(kbbq_delta_q(p, p + n, p + 2 * n, n, p + 3 * n, nullptr));
-    KBBQ_CUDA(cudaMemcpy(delta, p + 3 * n, (size_t)n * 8, cudaMemcpyDeviceToHost));
-    return KBBQ_OK;
-}
-
-int kbbq_posterior_q_real_host(const double *prior_q, const int64_t *numerrs, const int64_t *numtotal, int64_t n,
-                               int64_t *posterior, int device) {
-    if (n < 0) return KBBQ_E_ARG;
-    if (n == 0) return KBBQ_OK;
-    KBBQ_CUDA(cudaSetDevice(device));
-    DevBuf d;
-    KBBQ_TRY(d.alloc((size_t)n * 4 * 8));
-    int64_t *p = d.as<int64_t>();
-    KBBQ_CUDA(cudaMemcpy(p, prior_q, (size_t)n * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(p + n, numerrs, (size_t)n * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(p + 2 * n, numtotal, (size_t)n * 8, cudaMemcpyHostToDevice));
-    KBBQ_TRY(kbbq_posterior_q_real(reinterpret_cast<const double *>(p), p + n, p + 2 * n, n, p + 3 * n, nullptr));
-    KBBQ_CUDA(cudaMemcpy(posterior, p + 3 * n, (size_t)n * 8, cudaMemcpyDeviceToHost));
-    return KBBQ_OK;
-}
-
-// Host-buffer forms of the BAM-side entry points: copy, run, copy back (a BAM batch is small next to
-// what the host spends parsing it).
-int kbbq_build_bam_host(const uint8_t *seq, const uint8_t *qual, const uint8_t *err, const uint8_t *skip,
-                        const uint16_t *rg, const uint8_t *flags, const uint16_t *aln_start, const uint16_t *aln_end,
-                        int64_t N, int L, int R, int minscore, int64_t *pos_errs, int64_t *pos_total,
-                        int64_t *din_errs, int64_t *din_total, int *status_out, int device) {
-    if (N < 0 || L < 1 || R < 1 || R > 65535) return KBBQ_E_ARG;
-    if (!pos_errs || !pos_total || !din_errs || !din_total) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t npos = (size_t)R * NQ * 2 * L, ndin = (size_t)R * NQ * 16, nb = (size_t)N * L;
-    Carver c(nullptr);
-    auto carve = [&](Carver &cv, uint8_t **ds, uint8_t **dq, uint8_t **de, uint8_t **dk, uint16_t **dr, uint8_t **df,
-                     uint16_t **d0, uint16_t **d1, int64_t **dt, int **dst) {
-        *ds = cv.take<uint8_t>(nb); *dq = cv.take<uint8_t>(nb); *de = cv.take<uint8_t>(nb); *dk = cv.take<uint8_t>(nb);
-        *dr = cv.take<uint16_t>((size_t)N); *df = cv.take<uint8_t>((size_t)N);
-        *d0 = cv.take<uint16_t>((size_t)N); *d1 = cv.take<uint16_t>((size_t)N);
-        *dt = cv.take<int64_t>(2 * npos + 2 * ndin); *dst = cv.take<int>(64);
-    };
-    uint8_t *ds, *dq, *de, *dk, *df; uint16_t *dr, *d0, *d1; int64_t *dt; int *dst;
-    carve(c, &ds, &dq, &de, &dk, &dr, &df, &d0, &d1, &dt, &dst);
-    DevBuf buf;
-    KBBQ_TRY(buf.alloc(c.off));
-    Carver c2(buf.p);
-    carve(c2, &ds, &dq, &de, &dk, &dr, &df, &d0, &d1, &dt, &dst);
-    auto up = [&](void *d, const void *h, size_t n) { return h && n ? cudaMemcpy(d, h, n, cudaMemcpyHostToDevice) : cudaSuccess; };
-    KBBQ_CUDA(up(ds, seq, nb)); KBBQ_CUDA(up(dq, qual, nb)); KBBQ_CUDA(up(de, err, nb)); KBBQ_CUDA(up(dk, skip, nb));
-    KBBQ_CUDA(up(dr, rg, (size_t)N * 2)); KBBQ_CUDA(up(df, flags, (size_t)N));
-    KBBQ_CUDA(up(d0, aln_start, (size_t)N * 2)); KBBQ_CUDA(up(d1, aln_end, (size_t)N * 2));
-    KBBQ_CUDA(cudaMemcpy(dt, pos_errs, npos * 8, cudaMemcpyHostToDevice));   // the tables accumulate
-    KBBQ_CUDA(cudaMemcpy(dt + npos, pos_total, npos * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(dt + 2 * npos, din_errs, ndin * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(dt + 2 * npos + ndin, din_total, ndin * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemset(dst, 0, sizeof(int)));
-    size_t ws_bytes = 0;
-    KBBQ_TRY(kbbq_bam_workspace_bytes(N, L, R, &ws_bytes));
-    DevBuf ws;
-    KBBQ_TRY(ws.alloc(ws_bytes));
-    KBBQ_TRY(kbbq_build_bam(ds, dq, de, skip ? dk : nullptr, rg ? dr : nullptr, flags ? df : nullptr,
-                            aln_start ? d0 : nullptr, aln_end ? d1 : nullptr, N, L, R, minscore, dt, dt + npos,
-                            dt + 2 * npos, dt + 2 * npos + ndin, ws.p, ws_bytes, dst, nullptr));
-    KBBQ_CUDA(cudaMemcpy(pos_errs, dt, npos * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(pos_total, dt + npos, npos * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(din_errs, dt + 2 * npos, ndin * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(din_total, dt + 2 * npos + ndin, ndin * 8, cudaMemcpyDeviceToHost));
-    int st = 0;
-    KBBQ_CUDA(cudaMemcpy(&st, dst, sizeof(int), cudaMemcpyDeviceToHost));
-    if (status_out) *status_out = st;
-    return st ? KBBQ_E_DATA : KBBQ_OK;
-}
-
-int kbbq_apply_bam_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *flags, int64_t N,
-                        int L, int R, int minscore, const int64_t *meanq, const int64_t *rgdq, const int64_t *qdq,
-                        const int64_t *posdq, const int64_t *dindq, int nq, int ndin1, uint8_t *out_qual,
-                        int *status_out, int device) {
-    if (N < 0 || L < 1 || R < 1 || R > 65535 || nq < 1 || ndin1 != 17) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t nb = (size_t)N * L, n_q = (size_t)R * nq;
-    uint8_t *ds, *dq, *dout, *df; uint16_t *dr; int64_t *dm; int *dst;
-    DevBuf buf;
-    for (int pass = 0; pass < 2; ++pass) {
-        Carver cv(pass ? buf.p : nullptr);
-        ds = cv.take<uint8_t>(nb); dq = cv.take<uint8_t>(nb); dout = cv.take<uint8_t>(nb);
-        dr = cv.take<uint16_t>((size_t)N); df = cv.take<uint8_t>((size_t)N);
-        dm = cv.take<int64_t>(2 * (size_t)R + n_q * (1 + 2 * (size_t)L + ndin1)); dst = cv.take<int>(64);
-        if (!pass) KBBQ_TRY(buf.alloc(cv.off));
-    }
-    int64_t *d_meanq = dm, *d_rgdq = dm + R, *d_qdq = d_rgdq + R, *d_posdq = d_qdq + n_q, *d_dindq = d_posdq + n_q * 2 * L;
-    auto up = [&](void *d, const void *h, size_t n) { return h && n ? cudaMemcpy(d, h, n, cudaMemcpyHostToDevice) : cudaSuccess; };
-    KBBQ_CUDA(up(ds, seq, nb)); KBBQ_CUDA(up(dq, qual, nb));
-    KBBQ_CUDA(up(dr, rg, (size_t)N * 2)); KBBQ_CUDA(up(df, flags, (size_t)N));
-    KBBQ_CUDA(up(d_meanq, meanq, (size_t)R * 8)); KBBQ_CUDA(up(d_rgdq, rgdq, (size_t)R * 8));
-    KBBQ_CUDA(up(d_qdq, qdq, n_q * 8)); KBBQ_CUDA(up(d_posdq, posdq, n_q * 2 * L * 8));
-    KBBQ_CUDA(up(d_dindq, dindq, n_q * ndin1 * 8));
-    KBBQ_CUDA(cudaMemset(dst, 0, sizeof(int)));
-    size_t ws_bytes = 0;
-    KBBQ_TRY(kbbq_bam_workspace_bytes(N, L, R, &ws_bytes));
-    DevBuf ws;
-    KBBQ_TRY(ws.alloc(ws_bytes));
-    KBBQ_TRY(kbbq_apply_bam(ds, dq, rg ? dr : nullptr, flags ? df : nullptr, N, L, R, minscore, d_meanq, d_rgdq, d_qdq,
-                            d_posdq, d_dindq, nq, ndin1, dout, ws.p, ws_bytes, dst, nullptr));
-    if (nb) KBBQ_CUDA(cudaMemcpy(out_qual, dout, nb, cudaMemcpyDeviceToHost));
-    int st = 0;
-    KBBQ_CUDA(cudaMemcpy(&st, dst, sizeof(int), cudaMemcpyDeviceToHost));
-    if (status_out) *status_out = st;
-    return st ? KBBQ_E_DATA : KBBQ_OK;
-}
-
-int kbbq_calibration_counts_host(const uint8_t *qual, const uint8_t *err, const uint8_t *seq, const uint8_t *corr,
-                                 const uint8_t *skip, int64_t n, int64_t *total, int64_t *errs, int device) {
-    if (n < 0 || !total || !errs) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t nb = ((size_t)n + 15) / 16 * 16;
-    const int narr = 1 + (err ? 1 : 2) + (skip ? 1 : 0);
-    DevBuf d;
-    KBBQ_TRY(d.alloc(nb * narr + 2 * 256 * 8));
-    uint8_t *p = d.as<uint8_t>();
-    int64_t *cnt = reinterpret_cast<int64_t *>(p + nb * narr);
-    KBBQ_CUDA(cudaMemset(cnt, 0, 2 * 256 * 8));
-    uint8_t *dq = p, *de = nullptr, *ds = nullptr, *dc = nullptr, *dk = nullptr;
-    size_t o = nb;
-    KBBQ_CUDA(cudaMemcpy(dq, qual, (size_t)n, cudaMemcpyHostToDevice));
-    if (err) { de = p + o; o += nb; KBBQ_CUDA(cudaMemcpy(de, err, (size_t)n, cudaMemcpyHostToDevice)); }
-    else {
-        if (!seq || !corr) return KBBQ_E_ARG;
-        ds = p + o; o += nb; dc = p + o; o += nb;
-        KBBQ_CUDA(cudaMemcpy(ds, seq, (size_t)n, cudaMemcpyHostToDevice));
-        KBBQ_CUDA(cudaMemcpy(dc, corr, (size_t)n, cudaMemcpyHostToDevice));
-    }
-    if (skip) { dk = p + o; KBBQ_CUDA(cudaMemcpy(dk, skip, (size_t)n, cudaMemcpyHostToDevice)); }
-    KBBQ_TRY(kbbq_calibration_counts(dq, de, ds, dc, dk, n, cnt, cnt + 256, nullptr));
-    KBBQ_CUDA(cudaMemcpy(total, cnt, 256 * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(errs, cnt + 256, 256 * 8, cudaMemcpyDeviceToHost));
-    return KBBQ_OK;
-}
-
-int kbbq_marginals_host(const int64_t *pos_errs, const int64_t *pos_total, int L, int R, int64_t *q_errs,
-                        int64_t *q_total, int64_t *rg_errs, int64_t *rg_total, int64_t *meanq, int device) {
-    if (L < 1 || R < 1) return KBBQ_E_ARG;
-    KBBQ_CUDA(cudaSetDevice(device));
-    const size_t npos = (size_t)R * NQ * 2 * L, n_q = (size_t)R * NQ;
-    DevBuf d;
-    KBBQ_TRY(d.alloc((2 * npos + 2 * n_q + 3 * (size_t)R) * 8));
-    int64_t *pe = d.as<int64_t>(), *pt = pe + npos, *qe = pt + npos, *qt = qe + n_q, *ge = qt + n_q, *gt = ge + R,
-            *mq = gt + R;
-    KBBQ_CUDA(cudaMemcpy(pe, pos_errs, npos * 8, cudaMemcpyHostToDevice));
-    KBBQ_CUDA(cudaMemcpy(pt, pos_total, npos * 8, cudaMemcpyHostToDevice));
-    KBBQ_TRY(kbbq_marginals(pe, pt, L, R, qe, qt, ge, gt, mq, nullptr));
-    KBBQ_CUDA(cudaMemcpy(q_errs, qe, n_q * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(q_total, qt, n_q * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(rg_errs, ge, (size_t)R * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(rg_total, gt, (size_t)R * 8, cudaMemcpyDeviceToHost));
-    KBBQ_CUDA(cudaMemcpy(meanq, mq, (size_t)R * 8, cudaMemcpyDeviceToHost));
     return KBBQ_OK;
 }
 

@@ -165,6 +165,11 @@ def i64(a):
     return np.ascontiguousarray(a, dtype=np.int64)
 
 
+def _opt(a, dtype=np.uint8):
+    """An optional array argument: None stays None (NULL), anything else becomes a contiguous array of `dtype`."""
+    return None if a is None else np.ascontiguousarray(a, dtype=dtype)
+
+
 def plan_info(L, R=1, minscore=6, arrays=3, max_smem=0):
     """Shared-memory plan of the build (arrays=3) / apply (arrays=2) kernel, or None for the generic path."""
     out = (C.c_int * 10)()
@@ -177,20 +182,24 @@ def plan_info(L, R=1, minscore=6, arrays=3, max_smem=0):
 DEVICE = int(os.environ.get("KBBQ_DEVICE", os.environ.get("LOCAL_RANK", "0")))
 
 
+def _dev(device):
+    """The device of a call: `device`, or DEVICE when it is None."""
+    return DEVICE if device is None else int(device)
+
+
 # ---- host-buffer wrappers (numpy in, numpy out) ---------------------------------------------
 
 def build_host(seq, qual, corr, rg, second, L, R, minscore=6, device=None):
     seq, qual, corr = u8(seq).ravel(), u8(qual).ravel(), u8(corr).ravel()
     N = seq.size // L
     assert seq.size == qual.size == corr.size == N * L
-    rg = None if rg is None else np.ascontiguousarray(rg, dtype=np.uint16)
-    second = None if second is None else u8(second)
+    rg = _opt(rg, np.uint16)
+    second = _opt(second)
     pe, pt = np.zeros((R, NQ, 2 * L), np.int64), np.zeros((R, NQ, 2 * L), np.int64)
     de, dt = np.zeros((R, NQ, 16), np.int64), np.zeros((R, NQ, 16), np.int64)
     st = C.c_int(0)
     rc = lib().kbbq_build_host(ptr(seq), ptr(qual), ptr(corr), ptr(rg), ptr(second), N, L, R, minscore,
-                               ptr(pe), ptr(pt), ptr(de), ptr(dt), C.byref(st),
-                               DEVICE if device is None else device)
+                               ptr(pe), ptr(pt), ptr(de), ptr(dt), C.byref(st), _dev(device))
     check(rc, st.value)
     return pe, pt, de, dt
 
@@ -202,15 +211,14 @@ def marginals_host(pos_errs, pos_total, device=None):
     q_e, q_t = np.zeros((R, NQ), np.int64), np.zeros((R, NQ), np.int64)
     g_e, g_t, mq = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
     check(lib().kbbq_marginals_host(ptr(pos_errs), ptr(pos_total), L2 // 2, R, ptr(q_e), ptr(q_t),
-                                    ptr(g_e), ptr(g_t), ptr(mq), DEVICE if device is None else device))
+                                    ptr(g_e), ptr(g_t), ptr(mq), _dev(device)))
     return mq, g_e, g_t, q_e, q_t
 
 
 def delta_q_host(prior_q, numerrs, numtotal, device=None):
     prior_q, numerrs, numtotal = i64(prior_q), i64(numerrs), i64(numtotal)
     out = np.zeros(prior_q.shape, np.int64)
-    check(lib().kbbq_delta_q_host(ptr(prior_q), ptr(numerrs), ptr(numtotal), prior_q.size, ptr(out),
-                                  DEVICE if device is None else device))
+    check(lib().kbbq_delta_q_host(ptr(prior_q), ptr(numerrs), ptr(numtotal), prior_q.size, ptr(out), _dev(device)))
     return out
 
 
@@ -220,34 +228,30 @@ def posterior_q_real_host(prior_q, numerrs, numtotal, device=None):
     numerrs, numtotal = i64(numerrs), i64(numtotal)
     out = np.zeros(prior_q.shape, np.int64)
     check(lib().kbbq_posterior_q_real_host(ptr(prior_q), ptr(numerrs), ptr(numtotal), prior_q.size, ptr(out),
-                                           DEVICE if device is None else device))
+                                           _dev(device)))
     return out
 
 
 def calibration_counts_host(qual, err=None, seq=None, corr=None, skip=None, device=None):
     """-> (total int64[256], errs int64[256]): bases and errors per quality, skipped bases left out."""
     qual = u8(qual).ravel()
-    arrs = [None if a is None else u8(a).ravel() for a in (err, seq, corr, skip)]
+    arrs = [_opt(a) for a in (err, seq, corr, skip)]
     for a in arrs:
         assert a is None or a.size == qual.size
     total, errs = np.zeros(256, np.int64), np.zeros(256, np.int64)
     check(lib().kbbq_calibration_counts_host(ptr(qual), *[ptr(a) for a in arrs], qual.size, ptr(total), ptr(errs),
-                                             DEVICE if device is None else device))
+                                             _dev(device)))
     return total, errs
-
-
-def _u16(a):
-    return None if a is None else np.ascontiguousarray(a, dtype=np.uint16)
 
 
 def build_bam_host(seq, qual, err, skip, rg, flags, aln_start, aln_end, L, R, minscore=6, tables=None, device=None):
     """BAM-side tally on packed host arrays (kbbq_build_bam_host); `tables` = (pe, pt, de, dt) to add to."""
     seq, qual, err = u8(seq).ravel(), u8(qual).ravel(), u8(err).ravel()
-    skip = None if skip is None else u8(skip).ravel()
+    skip = _opt(skip)
     N = seq.size // L
     assert seq.size == qual.size == err.size == N * L
-    flags = None if flags is None else u8(flags)
-    rg, aln_start, aln_end = _u16(rg), _u16(aln_start), _u16(aln_end)
+    flags = _opt(flags)
+    rg, aln_start, aln_end = _opt(rg, np.uint16), _opt(aln_start, np.uint16), _opt(aln_end, np.uint16)
     if tables is None:
         tables = (np.zeros((R, NQ, 2 * L), np.int64), np.zeros((R, NQ, 2 * L), np.int64),
                   np.zeros((R, NQ, 16), np.int64), np.zeros((R, NQ, 16), np.int64))
@@ -255,7 +259,7 @@ def build_bam_host(seq, qual, err, skip, rg, flags, aln_start, aln_end, L, R, mi
     st = C.c_int(0)
     rc = lib().kbbq_build_bam_host(ptr(seq), ptr(qual), ptr(err), ptr(skip), ptr(rg), ptr(flags), ptr(aln_start),
                                    ptr(aln_end), N, L, R, minscore, ptr(pe), ptr(pt), ptr(de), ptr(dt), C.byref(st),
-                                   DEVICE if device is None else device)
+                                   _dev(device))
     check(rc, st.value)
     return pe, pt, de, dt
 
@@ -263,16 +267,15 @@ def build_bam_host(seq, qual, err, skip, rg, flags, aln_start, aln_end, L, R, mi
 def apply_bam_host(seq, qual, rg, flags, L, R, meanq, rgdq, qdq, posdq, dindq, minscore=6, device=None):
     seq, qual = u8(seq).ravel(), u8(qual).ravel()
     N = seq.size // L
-    flags = None if flags is None else u8(flags)
-    rg = _u16(rg)
+    flags = _opt(flags)
+    rg = _opt(rg, np.uint16)
     meanq, rgdq, qdq, posdq, dindq = [i64(a) for a in (meanq, rgdq, qdq, posdq, dindq)]
     nq, ndin1 = qdq.shape[1], dindq.shape[2]
     assert posdq.shape == (R, nq, 2 * L) and dindq.shape[:2] == (R, nq)
     out = np.zeros((N, L), np.uint8)
     st = C.c_int(0)
     rc = lib().kbbq_apply_bam_host(ptr(seq), ptr(qual), ptr(rg), ptr(flags), N, L, R, minscore, ptr(meanq), ptr(rgdq),
-                                   ptr(qdq), ptr(posdq), ptr(dindq), nq, ndin1, ptr(out), C.byref(st),
-                                   DEVICE if device is None else device)
+                                   ptr(qdq), ptr(posdq), ptr(dindq), nq, ndin1, ptr(out), C.byref(st), _dev(device))
     check(rc, st.value)
     return out
 
@@ -285,15 +288,15 @@ def get_delta_qs_host(meanq, rg_errs, rg_total, q_errs, q_total, pos_errs, pos_t
     rgdq, qdq = np.zeros(R, np.int64), np.zeros((R, nq), np.int64)
     posdq, dindq = np.zeros((R, nq, ncyc), np.int64), np.zeros((R, nq, ndin + 1), np.int64)
     check(lib().kbbq_get_delta_qs_host(*[ptr(a) for a in arrs], R, nq, ncyc, ndin, ptr(rgdq), ptr(qdq),
-                                       ptr(posdq), ptr(dindq), DEVICE if device is None else device))
+                                       ptr(posdq), ptr(dindq), _dev(device)))
     return rgdq, qdq, posdq, dindq
 
 
 def apply_host(seq, qual, rg, second, L, R, meanq, rgdq, qdq, posdq, dindq, minscore=6, device=None):
     seq, qual = u8(seq).ravel(), u8(qual).ravel()
     N = seq.size // L
-    rg = None if rg is None else np.ascontiguousarray(rg, dtype=np.uint16)
-    second = None if second is None else u8(second)
+    rg = _opt(rg, np.uint16)
+    second = _opt(second)
     meanq, rgdq, qdq, posdq, dindq = [i64(a) for a in (meanq, rgdq, qdq, posdq, dindq)]
     nq, ndin1 = qdq.shape[1], dindq.shape[2]
     assert posdq.shape == (R, nq, 2 * L) and dindq.shape[:2] == (R, nq)
@@ -301,7 +304,7 @@ def apply_host(seq, qual, rg, second, L, R, meanq, rgdq, qdq, posdq, dindq, mins
     st = C.c_int(0)
     rc = lib().kbbq_apply_host(ptr(seq), ptr(qual), ptr(rg), ptr(second), N, L, R, minscore, ptr(meanq),
                                ptr(rgdq), ptr(qdq), ptr(posdq), ptr(dindq), nq, ndin1, ptr(out),
-                               C.byref(st), DEVICE if device is None else device)
+                               C.byref(st), _dev(device))
     check(rc, st.value)
     return out
 
@@ -325,8 +328,8 @@ def recalibrate_host(seq, qual, corr, rg, second, L, R, minscore=6, want_tables=
     devices: several GPUs of this box share the reads (kbbq_recalibrate_host_multi); the result is the same."""
     seq, qual, corr = u8(seq).ravel(), u8(qual).ravel(), u8(corr).ravel()
     N = seq.size // L
-    rg = None if rg is None else np.ascontiguousarray(rg, dtype=np.uint16)
-    second = None if second is None else u8(second)
+    rg = _opt(rg, np.uint16)
+    second = _opt(second)
     if out is None:
         out = np.zeros((N, L), np.uint8)
     tables = deltas = None
@@ -365,7 +368,7 @@ class Session:
 
     def __init__(self, L, R=1, minscore=6, chunk_reads=0, resident_reads=0, device=None, host_threads=0):
         self.L, self.R = int(L), int(R)
-        self.device = DEVICE if device is None else int(device)
+        self.device = _dev(device)
         h = C.c_void_p()
         check(lib().kbbq_session_create(self.device, self.L, self.R, minscore, chunk_reads, resident_reads,
                                         host_threads, C.byref(h)))
@@ -397,8 +400,8 @@ class Session:
     def build_chunk(self, seq, qual, corr, rg=None, second=None, keep=False):
         seq, qual, corr = u8(seq).ravel(), u8(qual).ravel(), u8(corr).ravel()
         n = seq.size // self.L
-        rg = None if rg is None else np.ascontiguousarray(rg, dtype=np.uint16)
-        second = None if second is None else u8(second)
+        rg = _opt(rg, np.uint16)
+        second = _opt(second)
         check(lib().kbbq_session_build_chunk(self.h, ptr(seq), ptr(qual), ptr(corr), ptr(rg), ptr(second), n, int(keep)))
 
     def build_range(self, seq, qual, corr, rg=None, second=None):
@@ -406,8 +409,8 @@ class Session:
         them (kbbq_session_build_range).  Returns the number of chunks added."""
         seq, qual, corr = u8(seq).ravel(), u8(qual).ravel(), u8(corr).ravel()
         n = seq.size // self.L
-        rg = None if rg is None else np.ascontiguousarray(rg, dtype=np.uint16)
-        second = None if second is None else u8(second)
+        rg = _opt(rg, np.uint16)
+        second = _opt(second)
         check(lib().kbbq_session_build_range(self.h, ptr(seq), ptr(qual), ptr(corr), ptr(rg), ptr(second), n))
         return -(-n // self.chunk_reads)
 
@@ -443,8 +446,8 @@ class Session:
     def apply_chunk(self, seq, qual, rg, second, out):
         seq, qual = u8(seq).ravel(), u8(qual).ravel()
         n = seq.size // self.L
-        rg = None if rg is None else np.ascontiguousarray(rg, dtype=np.uint16)
-        second = None if second is None else u8(second)
+        rg = _opt(rg, np.uint16)
+        second = _opt(second)
         assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"] and out.size >= n * self.L
         self._keep.append(out)
         check(lib().kbbq_session_apply_chunk(self.h, ptr(seq), ptr(qual), ptr(rg), ptr(second), n, ptr(out)))

@@ -4,9 +4,9 @@
     python tools/sass_listing.py profiles/r1_sass
 
 writes <prefix>_<kernel>.txt (instructions only, encodings stripped) for the instantiations the BASELINE configs
-run -- 150 bp, one read group or a segmented batch: build_smem_kernel<3,true>, apply_smem_kernel<4>; 250 bp:
-build<2,true>, apply<3>; the work-list walk of rows in read order with several read groups: build<1,true>,
-apply<2>; build<4,true> is the plan round 1 ran at 150 bp -- plus <prefix>_summary.txt with a mnemonic histogram of each: the lines to
+run -- 150 bp, one read group or a segmented batch: build_smem_kernel<3,true>, apply_smem_kernel<4,true>; 250 bp:
+build<2,true>, apply<3,true>; the work-list walk of rows in read order with several read groups: build<1,true>,
+apply<2,true>; build<4,true> is the plan round 1 ran at 150 bp -- plus <prefix>_summary.txt with a mnemonic histogram of each: the lines to
 look for are UBLKCP (TMA bulk copy), SYNCS (mbarrier), ATOMS / REDS (shared-memory reductions), IDP
 (4-way byte dot product), PRMT, LDS, STG.
 """
@@ -21,11 +21,11 @@ SO = os.path.join(ROOT, "kbbq-py_b200", "kbbq", "libkbbq_b200.so")
 WANT = {
     "_ZN4kbbq17build_smem_kernelILi3ELb1EEEvNS_9BuildArgsE": "build_smem_kernel_kps3",
     "_ZN4kbbq17build_smem_kernelILi4ELb1EEEvNS_9BuildArgsE": "build_smem_kernel_kps4",
-    "_ZN4kbbq17apply_smem_kernelILi4EEEvNS_9ApplyArgsE": "apply_smem_kernel_kps4",
+    "_ZN4kbbq17apply_smem_kernelILi4ELb1EEEvNS_9ApplyArgsE": "apply_smem_kernel_kps4",
     "_ZN4kbbq17build_smem_kernelILi2ELb1EEEvNS_9BuildArgsE": "build_smem_kernel_kps2",
-    "_ZN4kbbq17apply_smem_kernelILi3EEEvNS_9ApplyArgsE": "apply_smem_kernel_kps3",
+    "_ZN4kbbq17apply_smem_kernelILi3ELb1EEEvNS_9ApplyArgsE": "apply_smem_kernel_kps3",
     "_ZN4kbbq17build_smem_kernelILi1ELb1EEEvNS_9BuildArgsE": "build_smem_kernel_kps1",
-    "_ZN4kbbq17apply_smem_kernelILi2EEEvNS_9ApplyArgsE": "apply_smem_kernel_kps2",
+    "_ZN4kbbq17apply_smem_kernelILi2ELb1EEEvNS_9ApplyArgsE": "apply_smem_kernel_kps2",
 }
 
 
