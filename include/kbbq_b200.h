@@ -57,6 +57,7 @@ extern "C" {
 #define KBBQ_FLAG_BAD_BASE 2   /* a base outside ACGTN: TypeError in Dinucleotide.vecget */
 #define KBBQ_FLAG_RG_RANGE 4   /* rg[i] >= R */
 #define KBBQ_FLAG_SEGMENTS 8   /* kbbq_*_segmented: malformed span table (not sorted / not 16-row aligned / past rows_bound) */
+#define KBBQ_FLAG_KMER_FULL 16 /* kbbq_kmer_count / kbbq_kmer_flag: a probe walked the whole k-mer table */
 
 int kbbq_abi_version(void);
 const char *kbbq_strerror(int code);
@@ -447,6 +448,54 @@ int kbbq_host_pack_nibbles(const uint8_t *seq, const uint8_t *corr, int64_t n, u
 /* The device side: seq_dev from the base codes, corr_dev = a byte array that differs from seq_dev exactly where
  * bit 3 of the nibble is set.  All three pointers 16-byte aligned. */
 int kbbq_expand_nibbles(const uint8_t *packed_dev, int64_t n, uint8_t *seq_dev, uint8_t *corr_dev, void *stream);
+
+/*
+ * Sequencing errors from the reads' own k-mer spectrum: the mismatch map of a batch without a corrected file
+ * (DESIGN.md, "Errors from k-mer counts").  For k in 1..31, window j of a read covers bases [j, j + k); it is valid
+ * when all k bases are A, C, G or T (uppercase); its key is min(forward code, reverse-complement code), first base in
+ * the most significant 2 bits (A 0, C 1, G 2, T 3).  count(key) = the valid windows of the batch with that key, both
+ * strands on one key, exact.  A window is solid when count >= t.  A base no solid window covers is uncovered unless
+ * its read has no solid window at all (such a read is left alone).  Every maximal run [a, b] of uncovered bases flags
+ * a and b when it is inside the read, b when it starts the read, a when it ends the read; a flagged base that is not
+ * A/C/G/T is not flagged.  The flags are the 1-bit map of kbbq_host_mismatch_bits (bit i of the flattened batch in
+ * word i / 32, LSB first), which kbbq_expand_mismatch_bits turns into the corrected reads kbbq_build takes.
+ *
+ * The counts live in an open-addressing table of `capacity` 16-byte slots {u64 key, u64 count} (capacity a power of
+ * two, table_dev 16-byte aligned).  kbbq_kmer_table_bytes: the default capacity for N reads of length L, the smallest
+ * power of two >= 1.5 x the number of windows N * max(0, L - k + 1), and its bytes.  kbbq_kmer_clear empties a table.
+ * kbbq_kmer_count ADDS the windows of a batch (chunks and repeated calls accumulate); a probe that finds no free slot
+ * in the whole table raises KBBQ_FLAG_KMER_FULL and stops.  kbbq_kmer_histogram writes hist_dev u64[256]: hist[c] =
+ * number of distinct keys with count c, counts above 255 in hist[255], hist[0] = 0.  kbbq_kmer_flag writes all
+ * ceil(N * L / 32) words of bits_dev for the threshold t = min_count >= 1 (resolve an automatic threshold with
+ * kbbq_kmer_min_count first).  Device pointers, asynchronous on `stream`, no allocation; L up to what one warp's
+ * L words of shared memory allow.
+ */
+int kbbq_kmer_table_bytes(int64_t N, int L, int k, uint64_t *capacity, size_t *bytes);
+int kbbq_kmer_clear(void *table_dev, uint64_t capacity, void *stream);
+int kbbq_kmer_count(const uint8_t *seq_dev, int64_t N, int L, int k, void *table_dev, uint64_t capacity,
+                    int *status_dev, void *stream);
+int kbbq_kmer_histogram(const void *table_dev, uint64_t capacity, uint64_t *hist_dev, void *stream);
+int kbbq_kmer_flag(const uint8_t *seq_dev, int64_t N, int L, int k, const void *table_dev, uint64_t capacity,
+                   int min_count, uint32_t *bits_dev, int *status_dev, void *stream);
+/* The automatic threshold: the smallest c in 2..254 with hist[c] <= hist[c + 1] (the first valley of the spectrum),
+ * 255 when there is none.  Host only, no device.  KBBQ_E_ARG for a NULL hist. */
+int kbbq_kmer_min_count(const uint64_t *hist);
+
+/*
+ * Host-buffer forms, synchronous.  kbbq_kmer_errors_host: the map of N reads of length L (bits_out ceil(N * L / 32)
+ * words; hist_out u64[256] may be NULL) with t = min_count when > 0, else kbbq_kmer_min_count of the batch's histogram
+ * (*min_count_used, may be NULL).  kbbq_recalibrate_kmer_host: kbbq_recalibrate_host with that map in place of a
+ * corrected file -- upload, clear + count + histogram, threshold, flag, then kbbq_expand_mismatch_bits, kbbq_build,
+ * kbbq_marginals, kbbq_get_delta_qs and kbbq_apply; tables_host / deltas_host (optional) as kbbq_recalibrate_host's.
+ * KBBQ_E_UNSUPPORTED when the reads and the default table do not fit the device's free memory; KBBQ_E_DATA with
+ * KBBQ_FLAG_KMER_FULL in the status (kbbq_kmer_errors_host has no other flag to report) when the table fills.
+ */
+int kbbq_kmer_errors_host(const uint8_t *seq, int64_t N, int L, int k, int min_count, uint32_t *bits_out,
+                          uint64_t *hist_out, int *min_count_used, int device);
+int kbbq_recalibrate_kmer_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second,
+                               int64_t N, int L, int R, int minscore, int k, int min_count, uint8_t *out_qual,
+                               int64_t *tables_host, int64_t *deltas_host, int *min_count_used, int *status_out,
+                               int device);
 
 /* Number of kernel launches this library has issued since load (bench.py's gpu_launches). */
 int64_t kbbq_launch_count(void);

@@ -1173,12 +1173,25 @@ struct HostCall {
     }
     Dev<void> scratch(size_t bytes) { return span<void>(SCRATCH, nullptr, bytes); }
 
-    int begin() {
-        KBBQ_CUDA(cudaSetDevice(device));
+    size_t bytes() const {
         Carver size(nullptr);
         for (const Span &s : spans) size.take<char>(s.bytes);
         if (with_status) size.take<int>(1);
-        KBBQ_CUDA(cudaMalloc(&base, size.off));
+        return size.off;
+    }
+
+    // *ok = the spans fit the device's free memory now
+    int fits(bool *ok) {
+        KBBQ_CUDA(cudaSetDevice(device));
+        size_t free_b = 0, total_b = 0;
+        KBBQ_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        *ok = bytes() <= free_b;
+        return KBBQ_OK;
+    }
+
+    int begin() {
+        KBBQ_CUDA(cudaSetDevice(device));
+        KBBQ_CUDA(cudaMalloc(&base, bytes()));
         Carver c(base);
         for (Span &s : spans) {
             s.d = c.take<char>(s.bytes);
@@ -1409,6 +1422,113 @@ int kbbq_marginals_host(const int64_t *pos_errs, const int64_t *pos_total, int L
     KBBQ_TRY(c.begin());
     KBBQ_TRY(kbbq_marginals(pe, pt, L, R, qe, qt, ge, gt, mq, nullptr));
     return c.finish();
+}
+
+}  // extern "C"
+
+// ---- errors from k-mer counts on host buffers (kmer.cuh) ----
+
+namespace {
+
+// clear + count + histogram, the threshold on the host, then the flags.  A full table stops before the flags:
+// *status = KBBQ_FLAG_KMER_FULL and KBBQ_E_DATA.
+int kmer_errors_dev(const uint8_t *seq, int64_t N, int L, int k, int min_count, void *table, uint64_t cap,
+                    uint64_t *d_hist, uint32_t *bits, int *d_status, uint64_t *hist, int *t, int *status) {
+    KBBQ_TRY(kbbq_kmer_clear(table, cap, nullptr));
+    KBBQ_TRY(kbbq_kmer_count(seq, N, L, k, table, cap, d_status, nullptr));
+    KBBQ_TRY(kbbq_kmer_histogram(table, cap, d_hist, nullptr));
+    KBBQ_CUDA(cudaMemcpy(hist, d_hist, 256 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    KBBQ_CUDA(cudaMemcpy(status, d_status, sizeof(int), cudaMemcpyDeviceToHost));
+    if (*status) return KBBQ_E_DATA;
+    *t = min_count > 0 ? min_count : kbbq_kmer_min_count(hist);
+    return kbbq_kmer_flag(seq, N, L, k, table, cap, *t, bits, d_status, nullptr);
+}
+
+}  // namespace
+
+extern "C" {
+
+int kbbq_kmer_errors_host(const uint8_t *seq, int64_t N, int L, int k, int min_count, uint32_t *bits_out,
+                          uint64_t *hist_out, int *min_count_used, int device) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 0 || (N > 0 && (!seq || !bits_out))) return KBBQ_E_ARG;
+    uint64_t cap = 0;
+    size_t table_bytes = 0;
+    KBBQ_TRY(kbbq_kmer_table_bytes(N, L, k, &cap, &table_bytes));
+    const size_t nb = (size_t)N * L;
+    HostCall c(device, true);
+    const auto d_seq = c.span(IN, seq, nb);
+    const auto d_bits = c.span(OUT, bits_out, (nb + 31) / 32 * 4);
+    const auto d_hist = c.scratch(256 * sizeof(uint64_t));
+    const auto table = c.scratch(table_bytes);
+    bool ok = false;
+    KBBQ_TRY(c.fits(&ok));
+    if (!ok) return KBBQ_E_UNSUPPORTED;
+    KBBQ_TRY(c.begin());
+    uint64_t hist[256];
+    int t = 0, st = 0;
+    KBBQ_TRY(kmer_errors_dev(d_seq, N, L, k, min_count, table, cap, (uint64_t *)(void *)d_hist, d_bits, c.status, hist,
+                             &t, &st));
+    if (hist_out) memcpy(hist_out, hist, sizeof(hist));
+    if (min_count_used) *min_count_used = t;
+    return c.finish();
+}
+
+int kbbq_recalibrate_kmer_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second,
+                               int64_t N, int L, int R, int minscore, int k, int min_count, uint8_t *out_qual,
+                               int64_t *tables_host, int64_t *deltas_host, int *min_count_used, int *status_out,
+                               int device) {
+    if (N < 0 || L < 1 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ || k < 1 || k > 31 || min_count < 0)
+        return KBBQ_E_ARG;
+    if (N > 0 && (!seq || !qual || !out_qual)) return KBBQ_E_ARG;
+    uint64_t cap = 0;
+    size_t table_bytes = 0, ws_bytes = 0;
+    KBBQ_TRY(kbbq_kmer_table_bytes(N, L, k, &cap, &table_bytes));
+    KBBQ_TRY(kbbq_workspace_bytes(N, L, R, &ws_bytes));
+    const size_t nb = (size_t)N * L, npos = (size_t)R * NQ * 2 * L, ndin = (size_t)R * NQ * 16;
+    const size_t ntab = 2 * npos + 2 * ndin, nmodel = carve_model(nullptr, L, R).elems;
+    HostCall c(device, true);
+    const auto d_seq = c.span(IN, seq, nb);
+    const auto d_qual = c.span(IN, qual, nb);
+    const auto d_rg = c.span(IN, rg, (size_t)N * 2);
+    const auto d_sec = c.span(IN, second, (size_t)N);
+    const auto d_out = c.span(OUT, out_qual, nb);
+    const auto d_bits = c.scratch((nb + 31) / 32 * 4);
+    const auto d_corr = c.scratch(nb);
+    const auto d_hist = c.scratch(256 * sizeof(uint64_t));
+    const auto d_tab = c.scratch(ntab * 8);
+    const auto d_model = c.scratch(nmodel * 8);
+    const auto ws = c.scratch(ws_bytes);
+    const auto table = c.scratch(table_bytes);
+    bool ok = false;
+    KBBQ_TRY(c.fits(&ok));
+    if (!ok) return KBBQ_E_UNSUPPORTED;
+    KBBQ_TRY(c.begin());
+    uint64_t hist[256];
+    int t = 0, st = 0;
+    const int rc = kmer_errors_dev(d_seq, N, L, k, min_count, table, cap, (uint64_t *)(void *)d_hist,
+                                   (uint32_t *)(void *)d_bits, c.status, hist, &t, &st);
+    if (rc == KBBQ_E_DATA && status_out) *status_out = st;
+    KBBQ_TRY(rc);
+    if (min_count_used) *min_count_used = t;
+    // from here on kbbq_recalibrate_host's steps on one batch, with the map in place of the corrected reads
+    int64_t *pe = (int64_t *)(void *)d_tab, *pt = pe + npos, *de = pt + npos, *dt = de + ndin;
+    const ModelPtrs mp = carve_model((int64_t *)(void *)d_model, L, R);
+    uint8_t *corr = (uint8_t *)(void *)d_corr;
+    KBBQ_CUDA(cudaMemset(pe, 0, ntab * 8));
+    KBBQ_TRY(kbbq_expand_mismatch_bits(d_seq, (uint32_t *)(void *)d_bits, (int64_t)nb, corr, nullptr));
+    KBBQ_TRY(kbbq_build(d_seq, d_qual, corr, d_rg, d_sec, N, L, R, minscore, pe, pt, de, dt, ws, ws_bytes, c.status, 0,
+                        nullptr));
+    KBBQ_TRY(kbbq_marginals(pe, pt, L, R, mp.q_errs, mp.q_total, mp.rg_errs, mp.rg_total, mp.meanq, nullptr));
+    KBBQ_TRY(kbbq_get_delta_qs(mp.meanq, mp.rg_errs, mp.rg_total, mp.q_errs, mp.q_total, pe, pt, de, dt, R, NQ, 2 * L,
+                               16, mp.rgdq, mp.qdq, mp.posdq, mp.dindq, nullptr));
+    // the build has checked these very bases into the same status word
+    KBBQ_TRY(kbbq_apply(d_seq, d_qual, d_rg, d_sec, N, L, R, minscore, mp.meanq, mp.rgdq, mp.qdq, mp.posdq, mp.dindq, NQ,
+                        17, d_out, ws, ws_bytes, c.status, KBBQ_APPLY_BASES_CHECKED, nullptr));
+    if (tables_host) KBBQ_CUDA(cudaMemcpy(tables_host, pe, ntab * 8, cudaMemcpyDeviceToHost));
+    if (deltas_host)
+        KBBQ_CUDA(cudaMemcpy(deltas_host, mp.meanq, ((size_t)2 * R + (size_t)R * NQ * (1 + 2 * L + 17)) * 8,
+                             cudaMemcpyDeviceToHost));
+    return c.finish(status_out);
 }
 
 }  // extern "C"

@@ -13,6 +13,7 @@
 #include "calib.cuh"
 #include "common.cuh"
 #include "expand.cuh"
+#include "kmer.cuh"
 #include "model.cuh"
 #include "prepare.cuh"
 #include "segment.cuh"
@@ -695,6 +696,87 @@ int kbbq_expand_nibbles(const uint8_t *packed, int64_t n, uint8_t *seq, uint8_t 
     expand_nibbles_kernel<<<(unsigned)((n + 32 * 256 - 1) / (32 * 256)), 256, 0, (cudaStream_t)stream>>>(packed, seq, corr, n);
     KBBQ_LAUNCHED();
     return KBBQ_OK;
+}
+
+// ---- k-mer errors (kmer.cuh) ----
+
+static bool kmer_table_ok(const void *table, uint64_t capacity) {
+    return table && !misaligned(table, 16) && capacity >= 1 && (capacity & (capacity - 1)) == 0;
+}
+
+int kbbq_kmer_table_bytes(int64_t N, int L, int k, uint64_t *capacity, size_t *bytes) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !capacity) return KBBQ_E_ARG;
+    const uint64_t windows = (uint64_t)N * (uint64_t)std::max(0, L - k + 1);
+    const uint64_t need = windows + (windows + 1) / 2;   // ceil(1.5 x windows)
+    if (need > (1ull << 59)) return KBBQ_E_ARG;
+    uint64_t cap = 1;
+    while (cap < need) cap <<= 1;
+    *capacity = cap;
+    if (bytes) *bytes = (size_t)(cap * 16);
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_clear(void *table, uint64_t capacity, void *stream) {
+    if (!kmer_table_ok(table, capacity)) return KBBQ_E_ARG;
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    const uint64_t blocks = std::min<uint64_t>((capacity + 255) / 256, (uint64_t)sms * 16);
+    kmer_clear_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((ulonglong2 *)table, capacity);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_count(const uint8_t *seq, int64_t N, int L, int k, void *table, uint64_t capacity, int *status,
+                    void *stream) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !status || !kmer_table_ok(table, capacity)) return KBBQ_E_ARG;
+    if (N == 0 || L < k) return KBBQ_OK;
+    if (!seq) return KBBQ_E_ARG;
+    kmer_count_kernel<<<(unsigned)((N + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        seq, N, L, k, (unsigned long long *)table, capacity - 1, status);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_histogram(const void *table, uint64_t capacity, uint64_t *hist, void *stream) {
+    if (!kmer_table_ok(table, capacity) || !hist) return KBBQ_E_ARG;
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    KBBQ_CUDA(cudaMemsetAsync(hist, 0, 256 * sizeof(uint64_t), (cudaStream_t)stream));
+    const uint64_t blocks = std::min<uint64_t>((capacity + 255) / 256, (uint64_t)sms * 8);
+    kmer_hist_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((const ulonglong2 *)table, capacity,
+                                                                         (unsigned long long *)hist);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_flag(const uint8_t *seq, int64_t N, int L, int k, const void *table, uint64_t capacity, int min_count,
+                   uint32_t *bits, int *status, void *stream) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 1 || !status || !kmer_table_ok(table, capacity))
+        return KBBQ_E_ARG;
+    if (N == 0) return KBBQ_OK;
+    if (!seq || !bits) return KBBQ_E_ARG;
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    // a warp assembles the L words of its 32 reads in shared memory: 4 warps a block while that stays under 48 KB
+    const int warps = std::max(1, std::min(4, 49152 / (4 * L)));
+    const size_t smem = (size_t)warps * L * 4;
+    if (smem > (size_t)max_smem) return KBBQ_E_ARG;
+    if (smem > 49152) KBBQ_CUDA(cudaFuncSetAttribute(kmer_flag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t blocks = (N + 32 * warps - 1) / (32 * warps);
+    kmer_flag_kernel<<<(unsigned)blocks, 32 * warps, smem, (cudaStream_t)stream>>>(
+        seq, N, L, k, (const ulonglong2 *)table, capacity - 1, (unsigned long long)min_count, bits, status);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_min_count(const uint64_t *hist) {
+    if (!hist) return KBBQ_E_ARG;
+    for (int c = 2; c <= 254; ++c)
+        if (hist[c] <= hist[c + 1]) return c;
+    return 255;
 }
 
 }  // extern "C"

@@ -1,0 +1,172 @@
+// kmer.cuh -- sequencing errors from the reads' own k-mer spectrum (kbbq_kmer_*, include/kbbq_b200.h).
+//
+// The rule (DESIGN.md, "Errors from k-mer counts"): a window of k bases is valid when all of them are A/C/G/T; its key
+// is the smaller of its forward and reverse-complement 2-bit codes (first base in the most significant bits).  count(x)
+// is the number of valid windows of the batch with key x; a window is solid when count >= t.  A base is uncovered when
+// no solid window covers it; in every maximal run [a, b] of uncovered bases, an inner run flags a and b, a run at the
+// read start flags b, a run at the read end flags a, and a run that is the whole read (no solid window) flags nothing.
+// A flagged byte that is not A/C/G/T is not flagged.
+//
+// Table: open addressing over `capacity` (a power of two) 16-byte slots {u64 key, u64 count}, empty key = all ones
+// (keys have 62 bits, so it cannot occur), home slot = splitmix64(key) & (capacity - 1), linear probing.  Insert: CAS
+// the key into an empty slot, then add 1 to the count -- one 32-byte sector per probe.  A probe that has walked the
+// whole table raises KBBQ_FLAG_KMER_FULL and gives up.  The counts, and so the flags, do not depend on where a key
+// lands, so any schedule gives the same bits.
+#pragma once
+#include "common.cuh"
+
+namespace kbbq {
+
+constexpr unsigned long long KMER_EMPTY = ~0ull;
+
+__device__ __forceinline__ unsigned long long kmer_mix(unsigned long long x) {   // splitmix64 finaliser
+    x ^= x >> 30;
+    x *= 0xBF58476D1CE4E5B9ull;
+    x ^= x >> 27;
+    x *= 0x94D049BB133111EBull;
+    x ^= x >> 31;
+    return x;
+}
+
+// A=0 C=1 G=2 T=3, anything else (N, lowercase) -1
+__device__ __forceinline__ int kmer_code(uint8_t b) {
+    return b == 'A' ? 0 : b == 'C' ? 1 : b == 'G' ? 2 : b == 'T' ? 3 : -1;
+}
+
+// Rolling codes of the window that ends at the base just pushed.  valid() once the last k bases were all A/C/G/T.
+struct KmerRoll {
+    unsigned long long fwd = 0, rc = 0, mask;
+    int shift, k, run = 0;
+    __device__ KmerRoll(int k_) : mask((1ull << (2 * k_)) - 1), shift(2 * (k_ - 1)), k(k_) {}
+    __device__ __forceinline__ void push(uint8_t b) {
+        const int c = kmer_code(b);
+        if (c < 0) { run = 0; return; }
+        fwd = ((fwd << 2) | (unsigned)c) & mask;
+        rc = (rc >> 2) | ((unsigned long long)(3 - c) << shift);
+        ++run;
+    }
+    __device__ __forceinline__ bool valid() const { return run >= k; }
+    __device__ __forceinline__ unsigned long long key() const { return fwd < rc ? fwd : rc; }
+};
+
+__global__ void kmer_clear_kernel(ulonglong2 *table, unsigned long long capacity) {
+    for (unsigned long long s = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; s < capacity;
+         s += (unsigned long long)gridDim.x * blockDim.x)
+        table[s] = make_ulonglong2(KMER_EMPTY, 0ull);
+}
+
+// One thread per read: roll the codes along the read, one insert per valid window.  Counts accumulate.
+__global__ void kmer_count_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *table,
+                                  unsigned long long mask, int *status) {
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= N) return;
+    const uint8_t *s = seq + r * L;
+    KmerRoll roll(k);
+    for (int e = 0; e < L; ++e) {
+        roll.push(s[e]);
+        if (!roll.valid()) continue;
+        const unsigned long long key = roll.key();
+        unsigned long long slot = kmer_mix(key) & mask;
+        bool done = false;
+        for (unsigned long long p = 0; p <= mask; ++p) {
+            unsigned long long *kp = table + 2 * slot;
+            unsigned long long cur = __ldcg(kp);   // a key never changes once set: a stale EMPTY only costs the CAS
+            if (cur == KMER_EMPTY) {
+                cur = atomicCAS(kp, KMER_EMPTY, key);
+                if (cur == KMER_EMPTY) cur = key;
+            }
+            if (cur == key) {
+                atomicAdd(kp + 1, 1ull);
+                done = true;
+                break;
+            }
+            slot = (slot + 1) & mask;
+        }
+        if (!done) {
+            atomicOr(status, KBBQ_FLAG_KMER_FULL);
+            return;
+        }
+    }
+}
+
+// 256-bin histogram of the counts of the occupied slots (count >= 255 in bin 255), privatised in shared memory.
+__global__ void kmer_hist_kernel(const ulonglong2 *table, unsigned long long capacity, unsigned long long *hist) {
+    __shared__ unsigned int h[256];
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) h[i] = 0;
+    __syncthreads();
+    for (unsigned long long s = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; s < capacity;
+         s += (unsigned long long)gridDim.x * blockDim.x) {
+        const ulonglong2 v = __ldg(table + s);
+        if (v.x != KMER_EMPTY && v.y) atomicAdd(&h[v.y < 255 ? v.y : 255], 1u);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < 256; i += blockDim.x)
+        if (h[i]) atomicAdd(hist + i, (unsigned long long)h[i]);
+}
+
+__device__ __forceinline__ unsigned long long kmer_lookup(const ulonglong2 *table, unsigned long long mask,
+                                                          unsigned long long key, bool *full) {
+    unsigned long long slot = kmer_mix(key) & mask;
+    for (unsigned long long p = 0; p <= mask; ++p) {
+        const ulonglong2 v = __ldg(table + slot);
+        if (v.x == key) return v.y;
+        if (v.x == KMER_EMPTY) return 0;
+        slot = (slot + 1) & mask;
+    }
+    *full = true;
+    return 0;
+}
+
+// One thread per read, one warp per 32 consecutive reads.  Each window's count is looked up once; base i is covered
+// when the last solid window that starts at or before i starts at i - k + 1 or later (the running form of "one of the
+// k windows over i is solid").  A base's coverage is final once the window that starts at it has been looked up, so
+// the run rule runs one window behind the lookups.  The 32 reads of a warp are 32 L bits = L whole words of the
+// map, starting at word (first read / 32) * L: the warp assembles them in shared memory and stores whole words.
+__global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
+                                 unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
+    extern __shared__ uint32_t kmer_words[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long r0 = ((long long)blockIdx.x * (blockDim.x >> 5) + warp) * 32;
+    if (r0 >= N) return;
+    uint32_t *wb = kmer_words + (size_t)warp * L;
+    for (int w = lane; w < L; w += 32) wb[w] = 0;
+    __syncwarp();
+    const long long r = r0 + lane;
+    if (r < N && L >= k) {
+        const uint8_t *s = seq + r * L;
+        const int base_bit = lane * L;
+        auto flag = [&](int i) {
+            if (kmer_code(s[i]) >= 0) atomicOr(&wb[(base_bit + i) >> 5], 1u << ((base_bit + i) & 31));
+        };
+        int last = -L - k;   // start of the last solid window so far
+        int run = -1;        // start of the open uncovered run, -1: none
+        auto settle = [&](int i) {   // coverage of base i is final
+            if (last < i - k + 1) {
+                if (run < 0) run = i;
+            } else if (run >= 0) {
+                if (run > 0) flag(run);   // an inner run flags both ends, one at the read start only its end
+                flag(i - 1);
+                run = -1;
+            }
+        };
+        KmerRoll roll(k);
+        bool full = false;
+        for (int e = 0; e < L; ++e) {
+            roll.push(s[e]);
+            if (e < k - 1) continue;
+            const int j = e - k + 1;
+            if (roll.valid() && kmer_lookup(table, mask, roll.key(), &full) >= t) last = j;
+            settle(j);
+        }
+        for (int i = L - k + 1; i < L; ++i) settle(i);
+        if (run > 0) flag(run);   // a run at the read end flags its start; a run of the whole read flags nothing
+        if (full) atomicOr(status, KBBQ_FLAG_KMER_FULL);
+    }
+    __syncwarp();
+    const long long nreads = N - r0 < 32 ? N - r0 : 32;
+    const int nwords = (int)((nreads * L + 31) / 32);
+    uint32_t *out = bits + (r0 / 32) * L;
+    for (int w = lane; w < nwords; w += 32) out[w] = wb[w];
+}
+
+}  // namespace kbbq

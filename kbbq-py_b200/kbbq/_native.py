@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(HERE, "libkbbq_b200.so")
 
 NQ = 43
 FLAG_QUAL_RANGE, FLAG_BAD_BASE, FLAG_RG_RANGE, FLAG_SEGMENTS = 1, 2, 4, 8
+FLAG_KMER_FULL = 16
 APPLY_BASES_CHECKED = 0x10   # kbbq_apply path flag: skip the base check (include/kbbq_b200.h)
 E_DATA = -4
 E_UNSUPPORTED = -12
@@ -99,6 +100,14 @@ SIGNATURES = {
     "kbbq_build_segmented": (_i, [_vp] * 4 + [_i64, _i, _i, _i] + [_vp] * 4 + [_vp, _sz, _vp, _vp]),
     "kbbq_apply_segmented": (_i, [_vp] * 3 + [_i64, _i, _i, _i] + [_vp] * 5 + [_i, _i, _vp, _vp, _sz, _vp, _vp]),
     "kbbq_apply_segmented_flags": (_i, [_vp] * 3 + [_i64, _i, _i, _i] + [_vp] * 5 + [_i, _i, _vp, _vp, _sz, _vp, _i, _vp]),
+    "kbbq_kmer_table_bytes": (_i, [_i64, _i, _i, C.POINTER(C.c_uint64), C.POINTER(_sz)]),
+    "kbbq_kmer_clear": (_i, [_vp, C.c_uint64, _vp]),
+    "kbbq_kmer_count": (_i, [_vp, _i64, _i, _i, _vp, C.c_uint64, _vp, _vp]),
+    "kbbq_kmer_histogram": (_i, [_vp, C.c_uint64, _vp, _vp]),
+    "kbbq_kmer_flag": (_i, [_vp, _i64, _i, _i, _vp, C.c_uint64, _i, _vp, _vp, _vp]),
+    "kbbq_kmer_min_count": (_i, [_vp]),
+    "kbbq_kmer_errors_host": (_i, [_vp, _i64, _i, _i, _i, _vp, _vp, C.POINTER(_i), _i]),
+    "kbbq_recalibrate_kmer_host": (_i, [_vp] * 4 + [_i64, _i, _i, _i, _i, _i] + [_vp] * 3 + [C.POINTER(_i), C.POINTER(_i), _i]),
 }
 
 
@@ -147,6 +156,8 @@ def raise_for_status(status):
         raise IndexError("read group index out of range")
     if status & FLAG_SEGMENTS:
         raise ValueError("malformed span table of a segmented batch")
+    if status & FLAG_KMER_FULL:
+        raise MemoryError("the k-mer table is full")
 
 
 def ptr(a):
@@ -348,6 +359,68 @@ def recalibrate_host(seq, qual, corr, rg, second, L, R, minscore=6, want_tables=
     tabs = (tables[:npos].reshape(R, NQ, 2 * L), tables[npos:2 * npos].reshape(R, NQ, 2 * L),
             tables[2 * npos:2 * npos + ndin].reshape(R, NQ, 16), tables[2 * npos + ndin:].reshape(R, NQ, 16))
     return out, tabs, split_deltas(deltas, L, R)
+
+
+def kmer_table_bytes(N, L, k):
+    """-> (capacity, bytes) of the default k-mer table for N reads of length L."""
+    cap, nbytes = C.c_uint64(0), C.c_size_t(0)
+    check(lib().kbbq_kmer_table_bytes(N, L, k, C.byref(cap), C.byref(nbytes)))
+    return cap.value, nbytes.value
+
+
+def kmer_min_count(hist):
+    """The automatic threshold of a 256-bin count histogram (kbbq_kmer_min_count)."""
+    hist = np.ascontiguousarray(hist, dtype=np.uint64)
+    assert hist.size == 256
+    return int(lib().kbbq_kmer_min_count(ptr(hist)))
+
+
+def _kmer_check(rc, status, N, L, k, device):
+    if rc == E_UNSUPPORTED:
+        nbytes = kmer_table_bytes(N, L, k)[1]
+        raise ValueError("%d reads x %d bp with a %.1f GB k-mer table (k = %d) do not fit the free memory of GPU %d"
+                         % (N, L, nbytes / 1e9, k, device))
+    check(rc, status)
+
+
+def kmer_errors_host(seq, L, k=23, min_count=0, device=None):
+    """Errors from the batch's k-mer counts (kbbq_kmer_errors_host) -> (bits u32[ceil(N*L/32)], hist u64[256], t)."""
+    seq = u8(seq).ravel()
+    N = seq.size // L
+    assert seq.size == N * L
+    bits = np.zeros((N * L + 31) // 32, np.uint32)
+    hist = np.zeros(256, np.uint64)
+    t = C.c_int(0)
+    dev = _dev(device)
+    rc = lib().kbbq_kmer_errors_host(ptr(seq), N, L, k, min_count, ptr(bits), ptr(hist), C.byref(t), dev)
+    _kmer_check(rc, FLAG_KMER_FULL, N, L, k, dev)   # a full table is the only data error of this entry point
+    return bits, hist, t.value
+
+
+def recalibrate_kmer_host(seq, qual, rg, second, L, R, minscore=6, k=23, min_count=0, want_tables=False, device=None):
+    """The whole path with the errors found from the reads' k-mer counts (kbbq_recalibrate_kmer_host)
+    -> (out_qual [N, L] u8, t), or (out_qual, t, tables, deltas) as recalibrate_host's with want_tables."""
+    seq, qual = u8(seq).ravel(), u8(qual).ravel()
+    N = seq.size // L
+    assert seq.size == qual.size == N * L
+    rg = _opt(rg, np.uint16)
+    second = _opt(second)
+    out = np.zeros((N, L), np.uint8)
+    tables = deltas = None
+    if want_tables:
+        tables = np.zeros(2 * R * NQ * 2 * L + 2 * R * NQ * 16, np.int64)
+        deltas = np.zeros(2 * R + R * NQ * (1 + 2 * L + 17), np.int64)
+    t, st = C.c_int(0), C.c_int(0)
+    dev = _dev(device)
+    rc = lib().kbbq_recalibrate_kmer_host(ptr(seq), ptr(qual), ptr(rg), ptr(second), N, L, R, minscore, k, min_count,
+                                          ptr(out), ptr(tables), ptr(deltas), C.byref(t), C.byref(st), dev)
+    _kmer_check(rc, st.value, N, L, k, dev)
+    if not want_tables:
+        return out, t.value
+    npos, ndin = R * NQ * 2 * L, R * NQ * 16
+    tabs = (tables[:npos].reshape(R, NQ, 2 * L), tables[npos:2 * npos].reshape(R, NQ, 2 * L),
+            tables[2 * npos:2 * npos + ndin].reshape(R, NQ, 16), tables[2 * npos + ndin:].reshape(R, NQ, 16))
+    return out, t.value, tabs, split_deltas(deltas, L, R)
 
 
 def split_deltas(deltas, L, R):

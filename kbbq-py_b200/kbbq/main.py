@@ -10,7 +10,17 @@ from kbbq import recalibrate as re
 
 def recalibrate(args):
     re.recalibrate(bam=args.bam, fastq=args.fastq, infer_rg=args.infer_rg,
-                   use_oq=args.use_oq, set_oq=args.set_oq, gatkreport=args.gatkreport)
+                   use_oq=args.use_oq, set_oq=args.set_oq, gatkreport=args.gatkreport,
+                   reads=args.reads, kmer_size=args.kmer_size, min_count=args.min_count)
+
+
+def _int_in(lo, hi):
+    def parse(text):
+        v = int(text)
+        if not lo <= v <= hi:
+            raise argparse.ArgumentTypeError("%d is not in %d..%d" % (v, lo, hi))
+        return v
+    return parse
 
 
 def _out_of_scope(name):
@@ -34,6 +44,13 @@ def main():
     recalibrate_input.add_argument('-b', '--bam', help='BAM to recalibrate')
     recalibrate_input.add_argument('-f', '--fastq', nargs=2,
                                    help='FASTQ file to recalibrate and a corrected version from your favorite error corrector.')
+    recalibrate_input.add_argument('-r', '--reads',
+                                   help='FASTQ file to recalibrate, its errors found on the GPU from its own k-mer counts.')
+    recalibrate_parser.add_argument('-k', '--kmer-size', type=_int_in(1, 31), default=23,
+                                    help='k-mer length of --reads (1..31, default 23).')
+    recalibrate_parser.add_argument('--min-count', type=_int_in(0, 2 ** 31 - 1), default=0,
+                                    help='Count from which a k-mer of --reads is trusted; 0 (default) takes the first '
+                                         'valley of the count histogram.')
     recalibrate_parser.add_argument('-u', '--use-oq', action='store_true', help=oq_help)
     recalibrate_parser.add_argument('-s', '--set-oq', action='store_true',
                                     help='Set the \'OQ\' flag prior to recalibration. Only works when producing BAM output.')

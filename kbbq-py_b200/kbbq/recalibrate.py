@@ -189,19 +189,51 @@ def recalibrate_fastq(fastq, infer_rg=False, devices=None):
     w.write(''.join(chunks))
 
 
+def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None):
+    """Recalibrate the reads of one FASTQ file with the errors found from their own k-mer counts (kbbq.kmer); FASTQ to
+    stdout as recalibrate_fastq prints it.  The whole file is one batch on the first of `devices`."""
+    from . import fastx
+    if not 1 <= k <= 31:
+        raise ValueError("k must be in 1..31, got %d" % k)
+    if min_count < 0:
+        raise ValueError("min_count must be >= 0, got %d" % min_count)
+    reads = fastx.NativeFastq(path)
+    try:
+        if reads.N == 0:
+            return
+        seq, qual = reads.pack()   # ValueError for reads of unequal length, as on the -f path
+        rg, second, keys = reads.infer(infer_rg)
+        L, R = reads.L, max(1, len(keys))
+        out, _ = _native.recalibrate_kmer_host(seq, qual, rg, second, L, R, 6, k, min_count,
+                                               device=_native.device_list(devices)[0])
+        fd = _stdout_fd()
+        if fd is not None:
+            reads.write(fd, out)
+            return
+        txt = (out + np.uint8(33)).astype(np.uint8)
+        sys.stdout.write(''.join('@%s\n%s\n+\n%s\n' % (reads.name(i), seq[i].tobytes().decode(),
+                                                      txt[i].tobytes().decode('latin-1')) for i in range(reads.N)))
+    finally:
+        reads.close()
+
+
 def recalibrate_bam(bam, use_oq=False, set_oq=False):
     """Not implemented in the reference either (kbbq/recalibrate.py:158-164)."""
     raise NotImplementedError('Recalibrating a bam is not yet implemented. \
         Try converting your BAM to a FASTQ file with the samtools fastq command.')
 
 
-def recalibrate(bam, fastq, infer_rg=False, use_oq=False, set_oq=False, gatkreport=None, devices=None):
-    """reference: kbbq/recalibrate.py:166-174 (devices: see recalibrate_fastq)."""
+def recalibrate(bam, fastq, infer_rg=False, use_oq=False, set_oq=False, gatkreport=None, devices=None, reads=None,
+                kmer_size=23, min_count=0):
+    """reference: kbbq/recalibrate.py:166-174 (devices: see recalibrate_fastq).  reads: one FASTQ file whose errors
+    come from its own k-mer counts (recalibrate_reads) instead of a corrected twin."""
     if gatkreport is not None:
         raise NotImplementedError('GATKreport reading / creation is not yet supported.')
     elif bam is not None:
         recalibrate_bam(bam, use_oq, set_oq)
     elif fastq is not None:
         recalibrate_fastq(fastq, infer_rg=infer_rg, devices=devices)
+    elif reads is not None:
+        recalibrate_reads(reads, infer_rg=infer_rg, k=kmer_size, min_count=min_count, devices=devices)
     else:
         raise ValueError("A BAM or FASTQ file should be provided for recalibration.")

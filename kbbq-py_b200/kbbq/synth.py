@@ -53,6 +53,59 @@ def _synth_block(seed, first_read, n, L, R):
     return seq, q.astype(np.uint8), corr, rg, sec.astype(np.uint8)
 
 
+def genome_reads(seed, genome_len, n_reads, L, sub_rate=0.01, n_rate=0.0, block=1 << 20):
+    """Reads sampled from a random genome, for the k-mer error path (kbbq.kmer): unlike synth_reads, whose bases are
+    iid, these repeat each other's k-mers as real reads do.
+
+    A seeded numpy stream draws a uniform random genome of `genome_len` bases.  Reads come in pairs (read 2i named
+    r<i>/1, read 2i + 1 r<i>/2): a fragment of L to 2L bases at a uniform position, read 1 its first L bases, read 2
+    the reverse complement of its last L.  Every base is then replaced by one of the three other bases with
+    probability `sub_rate` (a sequencing error) or by N with probability `n_rate`.  Qualities: 25..40 on correct
+    bases, 2..20 on errors, 2 on N.
+    -> seq u8[n, L], qual u8[n, L], errors bool[n, L] (the substitutions), second u8[n]."""
+    if n_reads and genome_len < 2 * L:
+        raise ValueError("genome_len must be at least 2 L")
+    rng = np.random.default_rng(seed)
+    genome = rng.integers(0, 4, genome_len, dtype=np.uint8)
+    acgt = np.frombuffer(b"ACGT", dtype=np.uint8)
+    seq = np.empty((n_reads, L), np.uint8)
+    qual = np.empty((n_reads, L), np.uint8)
+    err = np.empty((n_reads, L), bool)
+    second = (np.arange(n_reads) & 1).astype(np.uint8)
+    cols = np.arange(L)
+    block += block & 1   # the two reads of a pair share a block
+    for lo in range(0, n_reads, block):
+        hi = min(n_reads, lo + block)
+        n = hi - lo
+        pair = (np.arange(lo, hi) >> 1)
+        npairs = int(pair[-1] - pair[0] + 1)
+        frag = rng.integers(L, 2 * L + 1, npairs)
+        start = rng.integers(0, genome_len - frag + 1)
+        frag, start = frag[pair - pair[0]], start[pair - pair[0]]
+        is2 = second[lo:hi].astype(bool)
+        first = np.where(is2, start + frag - L, start)
+        codes = genome[first[:, None] + cols[None, :]]
+        codes[is2] = 3 - codes[is2][:, ::-1]   # read 2: the reverse complement of the fragment's end
+        e = rng.random((n, L)) < sub_rate
+        shift = rng.integers(1, 4, (n, L), dtype=np.uint8)
+        codes = np.where(e, (codes + shift) & 3, codes)
+        isn = rng.random((n, L)) < n_rate
+        seq[lo:hi] = np.where(isn, np.uint8(ord("N")), acgt[codes])
+        q = np.where(e, rng.integers(2, 21, (n, L)), rng.integers(25, 41, (n, L)))
+        qual[lo:hi] = np.where(isn, 2, q)
+        err[lo:hi] = e & ~isn
+    return seq, qual, err, second
+
+
+def write_reads_fastq(path, seq, qual, second):
+    """One FASTQ file of genome_reads' pairs, named r<i>/1 and r<i>/2."""
+    n, L = seq.shape
+    with open(path, "wb") as f:
+        for i in range(n):
+            f.write(b"@r%d/%d\n%s\n+\n%s\n" % (i // 2, int(second[i]) + 1, seq[i].tobytes(),
+                                               (qual[i] + 33).astype(np.uint8).tobytes()))
+
+
 def write_fastq(path_uncorr, path_corr, seq, qual, corr, rg, second, infer_rg=True):
     """Write the packed reads as the two FASTQ files `kbbq recalibrate -f` takes, named per
     docs/cli/fastq_input.rst of the reference (name/1_RG:Z:<rg>)."""
