@@ -57,7 +57,7 @@ extern "C" {
 #define KBBQ_FLAG_BAD_BASE 2   /* a base outside ACGTN: TypeError in Dinucleotide.vecget */
 #define KBBQ_FLAG_RG_RANGE 4   /* rg[i] >= R */
 #define KBBQ_FLAG_SEGMENTS 8   /* kbbq_*_segmented: malformed span table (not sorted / not 16-row aligned / past rows_bound) */
-#define KBBQ_FLAG_KMER_FULL 16 /* kbbq_kmer_count / kbbq_kmer_flag: a probe walked the whole k-mer table */
+#define KBBQ_FLAG_KMER_FULL 16 /* kbbq_kmer_count / _sieve / _flag: a probe walked the whole k-mer table */
 
 int kbbq_abi_version(void);
 const char *kbbq_strerror(int code);
@@ -496,6 +496,68 @@ int kbbq_recalibrate_kmer_host(const uint8_t *seq, const uint8_t *qual, const ui
                                int64_t N, int L, int R, int minscore, int k, int min_count, uint8_t *out_qual,
                                int64_t *tables_host, int64_t *deltas_host, int *min_count_used, int *status_out,
                                int device);
+
+/*
+ * The same counts for inputs of any size: a SIEVED table that only has to hold the keys seen at least twice, filled in
+ * two passes over all the reads (DESIGN.md §10, "Streaming").  Slots, hash, probing and empty key as above.
+ *   kbbq_kmer_sieve          pass A: per valid window one 64-bit atomicOr of a few bits into one word of filter_dev
+ *                            (filter_words u64, a power of two, zeroed before the first chunk); when the word already
+ *                            held them all, the key is put in the table with count 0.  Every key with count >= 2 ends
+ *                            up in the table whatever the schedule; a key seen once only through a false positive.
+ *                            A full table raises KBBQ_FLAG_KMER_FULL.
+ *   kbbq_kmer_count_present  pass B: adds 1 to the count of every window whose key is in the table, and the number of
+ *                            valid windows to *windows_dev (u64, zeroed before the first chunk).  A probe that walks a
+ *                            table with no empty slot raises KBBQ_FLAG_KMER_FULL.
+ * Both passes stop probing once KBBQ_FLAG_KMER_FULL is in status_dev: a full table costs no more than a usable one.
+ *   kbbq_kmer_histogram_sieved  hist_dev u64[256] equal to kbbq_kmer_histogram's of the exact table: bins 2..255 from
+ *                            the table, hist[1] = windows - the sum of the counts >= 2.
+ *   kbbq_kmer_flag_sieved    the flags for any t = min_count >= 1: t >= 2 is kbbq_kmer_flag (an absent key has count
+ *                            <= 1 < t); t = 1 marks every valid window solid without a lookup.
+ * The histogram, threshold and flags equal those of the exact table bit for bit; which false-positive singletons the
+ * table holds depends on the schedule.  Device pointers, asynchronous on `stream`, no allocation.
+ * kbbq_kmer_stream_plan (host only): sizes for a file of `windows` windows within budget_bytes -- the filter the
+ * largest power of two with 8 F <= min(windows, budget / 4) bytes (at least 1 word), the table the exact rule's
+ * capacity (kbbq_kmer_table_bytes) or, when that does not fit, the largest power of two with 16 cap <= budget - 8 F.
+ * KBBQ_E_UNSUPPORTED when not even min(exact capacity, KBBQ_KMER_MIN_SLOTS) slots fit.  The sizes never change the
+ * result, only the memory and whether the table can fill.
+ */
+#define KBBQ_KMER_MIN_SLOTS 65536
+int kbbq_kmer_stream_plan(uint64_t windows, uint64_t budget_bytes, uint64_t *filter_words, uint64_t *capacity);
+int kbbq_kmer_sieve(const uint8_t *seq_dev, int64_t N, int L, int k, void *filter_dev, uint64_t filter_words,
+                    void *table_dev, uint64_t capacity, int *status_dev, void *stream);
+int kbbq_kmer_count_present(const uint8_t *seq_dev, int64_t N, int L, int k, void *table_dev, uint64_t capacity,
+                            uint64_t *windows_dev, int *status_dev, void *stream);
+int kbbq_kmer_histogram_sieved(const void *table_dev, uint64_t capacity, const uint64_t *windows_dev, uint64_t *hist_dev,
+                               void *stream);
+int kbbq_kmer_flag_sieved(const uint8_t *seq_dev, int64_t N, int L, int k, const void *table_dev, uint64_t capacity,
+                          int min_count, uint32_t *bits_dev, int *status_dev, void *stream);
+
+/*
+ * `kbbq recalibrate -r` through a streaming session (resident_reads_cap = 0), chunk by chunk from host memory, in the
+ * session's streams and staging slots (a chunk's bytes go up while the previous chunk's kernel runs):
+ *   kmer_begin      allocate and clear the filter and the table for k-mers of length k (filter_words / capacity 0:
+ *                   kbbq_kmer_stream_plan of `windows`, the windows of the whole input, within 90 % of the free device
+ *                   memory; KBBQ_E_UNSUPPORTED when that does not fit)
+ *   kmer_sieve      pass A of a chunk of n <= chunk_reads reads (seq: n * L bytes), every chunk of the input
+ *   kmer_count      pass B of a chunk, every chunk again; the first call releases the filter, and returns
+ *                   KBBQ_E_DATA (KBBQ_FLAG_KMER_FULL in the status word) when the table filled in pass A
+ *   kmer_threshold  wait, build the histogram (hist_out u64[256], may be NULL) and take t = min_count when > 0, else
+ *                   kbbq_kmer_min_count (*t_used, may be NULL).  KBBQ_E_DATA with KBBQ_FLAG_KMER_FULL in the status
+ *                   word (kbbq_session_sync) when the table filled.
+ *   build_chunk_kmer  pass 1 of the build with the flags of the chunk as its mismatch map: seq crosses as bytes,
+ *                   then flag, kbbq_expand_mismatch_bits and the build of kbbq_session_build_chunk
+ * then kbbq_session_model and kbbq_session_apply_chunk as for any streaming session.  Calls out of this order (and
+ * on a session that keeps chunks resident) return KBBQ_E_ARG, as do kbbq_session_build_chunk / _build_range /
+ * _apply_chunk between kmer_begin and kmer_threshold; kbbq_session_reset releases the k-mer buffers.
+ */
+int kbbq_session_kmer_begin(kbbq_session *s, int k, int64_t windows, uint64_t filter_words, uint64_t capacity);
+int kbbq_session_kmer_sieve(kbbq_session *s, const uint8_t *seq, int64_t n);
+int kbbq_session_kmer_count(kbbq_session *s, const uint8_t *seq, int64_t n);
+int kbbq_session_kmer_threshold(kbbq_session *s, int min_count, uint64_t *hist_out, int *t_used);
+int kbbq_session_build_chunk_kmer(kbbq_session *s, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg,
+                                  const uint8_t *second, int64_t n);
+/* sizes the session's k-mer buffers were given (0 before kmer_begin) */
+int kbbq_session_kmer_sizes(const kbbq_session *s, uint64_t *filter_words, uint64_t *capacity);
 
 /* Number of kernel launches this library has issued since load (bench.py's gpu_launches). */
 int64_t kbbq_launch_count(void);

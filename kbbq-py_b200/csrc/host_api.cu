@@ -17,6 +17,11 @@
 // tables summed over NVLink peer memory (one kernel per device reads every peer's table and writes the sum),
 // through pinned host memory when the devices cannot reach each other.  Every kernel launched here goes through
 // the device-pointer entry points of kbbq_b200.cu.
+//
+// `kbbq recalibrate -r` streams through the same session: kbbq_session_kmer_sieve x n and kbbq_session_kmer_count x n
+// fill a sieved k-mer table (kmer.cuh) in the same slots and streams, kbbq_session_kmer_threshold takes the exact
+// histogram, and kbbq_session_build_chunk_kmer is pass 1 with the map flagged on the device in place of the corrected
+// reads.
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -90,6 +95,9 @@ __global__ void sum_tables_kernel(PeerTables p, int n, long long *out, size_t el
 
 enum { PACK_NONE = 0, PACK_BITS = 1, PACK_NIBBLES = 2 };
 
+// where a session is in `kbbq recalibrate -r` (kbbq_session_kmer_*): the calls must come in this order
+enum { KMER_NONE = 0, KMER_SIEVE, KMER_COUNT, KMER_READY };
+
 struct UpSlot {   // one upload in flight: the chunk as the host has it (read order)
     uint8_t *seq = nullptr, *qual = nullptr, *corr = nullptr, *sec = nullptr;
     uint16_t *rg = nullptr;
@@ -139,6 +147,14 @@ struct kbbq_session {
     int64_t built = 0, applied = 0;
     bool summed = false;    // the model reads d_sum (tables of several sessions added up) instead of d_tab
     int64_t h2d_bytes = 0, d2h_bytes = 0;
+    // the sieved k-mer table of kbbq_session_kmer_*: the filter (released when pass B starts), and one allocation of
+    // table, window count, histogram and the map of a chunk
+    int kmer_stage = KMER_NONE, kmer_k = 0, kmer_t = 0;
+    int64_t kmer_chunks = 0;
+    uint64_t filter_words = 0, kmer_cap = 0;
+    void *kmer_filter = nullptr, *kmer_base = nullptr, *kmer_table = nullptr;
+    uint64_t *kmer_windows = nullptr, *kmer_hist = nullptr;
+    uint32_t *kmer_bits = nullptr;
     std::mutex mu;
 
     ~kbbq_session() {
@@ -146,6 +162,8 @@ struct kbbq_session {
         for (auto s : {s_up, s_comp, s_down}) if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
         for (auto &u : up) { if (u.uploaded) cudaEventDestroy(u.uploaded); if (u.consumed) cudaEventDestroy(u.consumed); }
         for (auto &o : down) { if (o.applied) cudaEventDestroy(o.applied); if (o.drained) cudaEventDestroy(o.drained); }
+        if (kmer_filter) cudaFree(kmer_filter);
+        if (kmer_base) cudaFree(kmer_base);
         if (base) cudaFree(base);
         if (pinned) cudaFreeHost(pinned);
     }
@@ -280,11 +298,26 @@ int session_create(int device, int L, int R, int minscore, int64_t C, int64_t M,
     return KBBQ_OK;
 }
 
-// Forget the tables and chunks of the previous run (the device memory stays).
+// Free the k-mer buffers once the compute stream is done with them.
+int kmer_release(kbbq_session *S) {
+    if (S->kmer_filter || S->kmer_base) KBBQ_CUDA(cudaStreamSynchronize(S->s_comp));
+    if (S->kmer_filter) KBBQ_CUDA(cudaFree(S->kmer_filter));
+    if (S->kmer_base) KBBQ_CUDA(cudaFree(S->kmer_base));
+    S->kmer_filter = S->kmer_base = S->kmer_table = nullptr;
+    S->kmer_windows = S->kmer_hist = nullptr;
+    S->kmer_bits = nullptr;
+    S->filter_words = S->kmer_cap = 0;
+    S->kmer_stage = KMER_NONE;
+    S->kmer_chunks = 0;
+    return KBBQ_OK;
+}
+
+// Forget the tables and chunks of the previous run (the device memory stays; the k-mer buffers go).
 int session_reset(kbbq_session *S) {
     KBBQ_CUDA(cudaSetDevice(S->device));
     KBBQ_CUDA(cudaStreamSynchronize(S->s_up));
     KBBQ_CUDA(cudaStreamSynchronize(S->s_down));
+    KBBQ_TRY(kmer_release(S));
     KBBQ_CUDA(cudaMemsetAsync(S->d_tab, 0, S->ntab * 8, S->s_comp));
     KBBQ_CUDA(cudaMemsetAsync(S->d_status, 0, sizeof(int), S->s_comp));
     S->built = S->applied = 0;
@@ -331,29 +364,34 @@ bool chunk_args_ok(const kbbq_session *S, int64_t k, int64_t n, bool keep) {
 }
 
 // Pass 1 of chunk k, first half: enqueue the copies that come straight from the caller's memory (the qualities,
-// read groups and mate flags; the reads too unless they travel as nibbles).  Nothing waits for the device.
+// read groups and mate flags; the reads too unless they travel as nibbles -- and always on the k-mer path, whose map
+// is made on the device from the reads).  Nothing waits for the device.
 int build_chunk_upload(kbbq_session *S, int64_t k, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg,
-                       const uint8_t *second, int64_t n, bool keep) {
+                       const uint8_t *second, int64_t n, bool keep, bool kmer = false) {
     if (!chunk_args_ok(S, k, n, keep) || !seq || !qual) return KBBQ_E_ARG;
     const ChunkPlace p = chunk_place(S, k, keep, rg != nullptr, second != nullptr);
     KBBQ_CUDA(cudaStreamWaitEvent(S->s_up, p.u->consumed, 0));   // the slot's previous chunk has been built
-    return upload_reads(S, S->pack == PACK_NIBBLES ? nullptr : seq, qual, rg, second, n, p.d_seq, p.d_qual, p.d_rg, p.d_sec);
+    return upload_reads(S, S->pack == PACK_NIBBLES && !kmer ? nullptr : seq, qual, rg, second, n, p.d_seq, p.d_qual,
+                        p.d_rg, p.d_sec);
 }
 
 // Second half: the host cores pack (seq, corrected) of the chunk while the copy engine is busy with what
 // build_chunk_upload queued (of this chunk and, in run_build_pass, of the next one too), the packed form follows,
 // and the compute stream expands it, segments the rows when there are several read groups, and builds.  The only
-// wait is for the pinned packing slot (two chunks back).
+// wait is for the pinned packing slot (two chunks back).  corr == NULL: the k-mer path -- nothing more goes up, the
+// map is flagged from the session's k-mer table and expanded on the device.
 int build_chunk_finish(kbbq_session *S, int64_t k, const uint8_t *seq, const uint8_t *corr, bool has_rg, bool has_second,
                        int64_t n, bool keep) {
-    if (!chunk_args_ok(S, k, n, keep) || !seq || !corr) return KBBQ_E_ARG;
+    const bool kmer = corr == nullptr;
+    if (!chunk_args_ok(S, k, n, keep) || !seq || (kmer && S->kmer_stage != KMER_READY)) return KBBQ_E_ARG;
     const ChunkPlace p = chunk_place(S, k, keep, has_rg, has_second);
     UpSlot &u = *p.u;
     Resident *r = p.r;
     const int L = S->L, R = S->R;
     const size_t nb = (size_t)n * L;
     if (r) r->n = n;
-    if (S->pack) {
+    if (kmer) {
+    } else if (S->pack) {
         KBBQ_CUDA(cudaEventSynchronize(u.uploaded));           // the slot's packed chunk of two chunks back is on the device
         size_t bb;
         if (S->pack == PACK_NIBBLES) {
@@ -373,7 +411,11 @@ int build_chunk_finish(kbbq_session *S, int64_t k, const uint8_t *seq, const uin
     }
     KBBQ_CUDA(cudaEventRecord(u.uploaded, S->s_up));
     KBBQ_CUDA(cudaStreamWaitEvent(S->s_comp, u.uploaded, 0));
-    if (S->pack == PACK_NIBBLES) KBBQ_TRY(kbbq_expand_nibbles((const uint8_t *)u.bits, (int64_t)nb, p.d_seq, u.corr, S->s_comp));
+    if (kmer) {
+        KBBQ_TRY(kbbq_kmer_flag_sieved(p.d_seq, n, L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_t, S->kmer_bits,
+                                       S->d_status, S->s_comp));
+        KBBQ_TRY(kbbq_expand_mismatch_bits(p.d_seq, S->kmer_bits, (int64_t)nb, u.corr, S->s_comp));
+    } else if (S->pack == PACK_NIBBLES) KBBQ_TRY(kbbq_expand_nibbles((const uint8_t *)u.bits, (int64_t)nb, p.d_seq, u.corr, S->s_comp));
     else if (S->pack == PACK_BITS) KBBQ_TRY(kbbq_expand_mismatch_bits(p.d_seq, u.bits, (int64_t)nb, u.corr, S->s_comp));
     const size_t npos = (size_t)R * NQ * 2 * L, ndin = (size_t)R * NQ * 16;
     int64_t *pe = S->d_tab, *pt = pe + npos, *de = pt + npos, *dt = de + ndin;
@@ -396,9 +438,12 @@ int build_chunk_finish(kbbq_session *S, int64_t k, const uint8_t *seq, const uin
 }
 
 // Pass 1 of one chunk in one go.
+// between kbbq_session_kmer_begin and kbbq_session_kmer_threshold only the k-mer passes may run on a session
+bool kmer_counting(const kbbq_session *S) { return S->kmer_stage == KMER_SIEVE || S->kmer_stage == KMER_COUNT; }
+
 int build_chunk_async(kbbq_session *S, const uint8_t *seq, const uint8_t *qual, const uint8_t *corr, const uint16_t *rg,
                       const uint8_t *second, int64_t n, bool keep) {
-    if (n < 0 || n > S->C) return KBBQ_E_ARG;
+    if (n < 0 || n > S->C || kmer_counting(S)) return KBBQ_E_ARG;
     if (n == 0) return KBBQ_OK;
     if (!seq || !qual || !corr) return KBBQ_E_ARG;
     const int64_t k = S->built;
@@ -406,6 +451,112 @@ int build_chunk_async(kbbq_session *S, const uint8_t *seq, const uint8_t *qual, 
     S->built++;
     KBBQ_TRY(build_chunk_upload(S, k, seq, qual, rg, second, n, keep));
     return build_chunk_finish(S, k, seq, corr, rg != nullptr, second != nullptr, n, keep);
+}
+
+// ---- kbbq recalibrate -r through a streaming session (kbbq_session_kmer_*, DESIGN.md §10 "Streaming") ----
+
+int kmer_begin(kbbq_session *S, int k, int64_t windows, uint64_t F, uint64_t cap) {
+    auto pow2 = [](uint64_t x) { return x >= 1 && (x & (x - 1)) == 0; };
+    if (k < 1 || k > 31 || windows < 0 || S->kmer_stage != KMER_NONE || S->M > 0) return KBBQ_E_ARG;   // streaming only
+    if ((F == 0) != (cap == 0) || (F && (!pow2(F) || !pow2(cap)))) return KBBQ_E_ARG;
+    if (!F) {
+        size_t free_b = 0, total_b = 0;
+        KBBQ_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        KBBQ_TRY(kbbq_kmer_stream_plan((uint64_t)windows, (uint64_t)(0.9 * (double)free_b), &F, &cap));
+    }
+    const size_t bits_words = ((size_t)S->C * S->L + 31) / 32 + 4;
+    Carver c(nullptr);
+    c.take<ulonglong2>(cap);
+    c.take<uint64_t>(1);
+    c.take<uint64_t>(256);
+    c.take<uint32_t>(bits_words);
+    // a request the device cannot hold is a size problem (KBBQ_E_UNSUPPORTED), not a CUDA failure
+    auto alloc = [&](void **p, size_t bytes) -> int {
+        const cudaError_t e = cudaMalloc(p, bytes);
+        if (e == cudaSuccess) return KBBQ_OK;
+        cudaGetLastError();
+        *p = nullptr;
+        kmer_release(S);
+        return e == cudaErrorMemoryAllocation ? KBBQ_E_UNSUPPORTED : KBBQ_E_CUDA;
+    };
+    KBBQ_TRY(alloc(&S->kmer_filter, F * 8));
+    KBBQ_TRY(alloc(&S->kmer_base, c.off));
+    Carver d(S->kmer_base);
+    S->kmer_table = d.take<ulonglong2>(cap);
+    S->kmer_windows = d.take<uint64_t>(1);
+    S->kmer_hist = d.take<uint64_t>(256);
+    S->kmer_bits = d.take<uint32_t>(bits_words);
+    S->filter_words = F;
+    S->kmer_cap = cap;
+    S->kmer_k = k;
+    S->kmer_chunks = 0;
+    KBBQ_CUDA(cudaMemsetAsync(S->kmer_filter, 0, F * 8, S->s_comp));
+    KBBQ_CUDA(cudaMemsetAsync(S->kmer_windows, 0, 8, S->s_comp));
+    KBBQ_TRY(kbbq_kmer_clear(S->kmer_table, cap, S->s_comp));
+    S->kmer_stage = KMER_SIEVE;
+    return KBBQ_OK;
+}
+
+// Pass A (count = false) or B of one chunk: its bytes go up into a staging slot while the previous chunk's kernel runs.
+int kmer_chunk(kbbq_session *S, const uint8_t *seq, int64_t n, bool count, UpSlot **slot) {
+    *slot = nullptr;
+    const bool in_order = S->kmer_stage == KMER_SIEVE || (count && S->kmer_stage == KMER_COUNT);
+    if (!in_order) return KBBQ_E_ARG;
+    if (n < 0 || n > S->C || (n > 0 && !seq)) return KBBQ_E_ARG;
+    if (count && S->kmer_stage == KMER_SIEVE) {   // pass A is over: its filter is not needed any more
+        int st = 0;
+        KBBQ_CUDA(cudaMemcpyAsync(&st, S->d_status, sizeof(int), cudaMemcpyDeviceToHost, S->s_comp));
+        KBBQ_CUDA(cudaStreamSynchronize(S->s_comp));
+        KBBQ_CUDA(cudaFree(S->kmer_filter));
+        S->kmer_filter = nullptr;
+        S->kmer_stage = KMER_COUNT;
+        // a table that filled in pass A is reported here, before pass B; one that fills in pass B stops its kernels
+        // (kmer.cuh) and is reported by kbbq_session_kmer_threshold
+        if (st & KBBQ_FLAG_KMER_FULL) return KBBQ_E_DATA;
+    }
+    if (n == 0) return KBBQ_OK;
+    UpSlot &u = S->up[S->kmer_chunks++ & 1];
+    const size_t nb = (size_t)n * S->L;
+    KBBQ_CUDA(cudaStreamWaitEvent(S->s_up, u.consumed, 0));
+    KBBQ_CUDA(cudaMemcpyAsync(u.seq, seq, nb, cudaMemcpyHostToDevice, S->s_up));
+    S->h2d_bytes += (int64_t)nb;
+    KBBQ_CUDA(cudaEventRecord(u.uploaded, S->s_up));
+    KBBQ_CUDA(cudaStreamWaitEvent(S->s_comp, u.uploaded, 0));
+    if (count)
+        KBBQ_TRY(kbbq_kmer_count_present(u.seq, n, S->L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_windows,
+                                         S->d_status, S->s_comp));
+    else
+        KBBQ_TRY(kbbq_kmer_sieve(u.seq, n, S->L, S->kmer_k, S->kmer_filter, S->filter_words, S->kmer_table, S->kmer_cap,
+                                 S->d_status, S->s_comp));
+    KBBQ_CUDA(cudaEventRecord(u.consumed, S->s_comp));
+    *slot = &u;
+    return KBBQ_OK;
+}
+
+int kmer_threshold(kbbq_session *S, int min_count, uint64_t *hist_out, int *t_used) {
+    if (S->kmer_stage != KMER_COUNT || min_count < 0) return KBBQ_E_ARG;
+    uint64_t hist[256];
+    int st = 0;
+    KBBQ_TRY(kbbq_kmer_histogram_sieved(S->kmer_table, S->kmer_cap, S->kmer_windows, S->kmer_hist, S->s_comp));
+    KBBQ_CUDA(cudaMemcpyAsync(hist, S->kmer_hist, sizeof(hist), cudaMemcpyDeviceToHost, S->s_comp));
+    KBBQ_CUDA(cudaMemcpyAsync(&st, S->d_status, sizeof(int), cudaMemcpyDeviceToHost, S->s_comp));
+    KBBQ_CUDA(cudaStreamSynchronize(S->s_comp));
+    if (st & KBBQ_FLAG_KMER_FULL) return KBBQ_E_DATA;
+    S->kmer_t = min_count > 0 ? min_count : kbbq_kmer_min_count(hist);
+    S->kmer_stage = KMER_READY;
+    if (hist_out) memcpy(hist_out, hist, sizeof(hist));
+    if (t_used) *t_used = S->kmer_t;
+    return KBBQ_OK;
+}
+
+int build_chunk_kmer_async(kbbq_session *S, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg,
+                           const uint8_t *second, int64_t n) {
+    if (S->kmer_stage != KMER_READY || n < 0 || n > S->C) return KBBQ_E_ARG;
+    if (n == 0) return KBBQ_OK;
+    if (!seq || !qual) return KBBQ_E_ARG;
+    const int64_t k = S->built++;
+    KBBQ_TRY(build_chunk_upload(S, k, seq, qual, rg, second, n, false, true));
+    return build_chunk_finish(S, k, seq, nullptr, rg != nullptr, second != nullptr, n, false);
 }
 
 int model_async(kbbq_session *S) {
@@ -453,7 +604,7 @@ int apply_resident_async(kbbq_session *S, int64_t k, uint8_t *out_host) {
 // pass 2 of a chunk that is not resident: the reads are sent again
 int apply_chunk_async(kbbq_session *S, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second,
                       int64_t n, uint8_t *out_host) {
-    if (n < 0 || n > S->C || !S->up[0].seq) return KBBQ_E_ARG;
+    if (n < 0 || n > S->C || !S->up[0].seq || kmer_counting(S)) return KBBQ_E_ARG;
     if (n == 0) return KBBQ_OK;
     if (!seq || !qual || !out_host) return KBBQ_E_ARG;
     UpSlot &u = S->up[S->applied & 1];
@@ -628,9 +779,56 @@ int kbbq_session_build_range(kbbq_session *s, const uint8_t *seq, const uint8_t 
                              const uint16_t *rg, const uint8_t *second, int64_t n) {
     if (!s || n < 0 || (n > 0 && (!seq || !qual || !corr))) return KBBQ_E_ARG;
     std::lock_guard<std::mutex> lock(s->mu);
+    if (kmer_counting(s)) return KBBQ_E_ARG;
     KBBQ_CUDA(cudaSetDevice(s->device));
     KBBQ_TRY(run_build_pass(s, seq, qual, corr, rg, second, n));
     KBBQ_CUDA(cudaStreamSynchronize(s->s_up));   // the caller may reuse its buffers
+    return KBBQ_OK;
+}
+
+int kbbq_session_kmer_begin(kbbq_session *s, int k, int64_t windows, uint64_t filter_words, uint64_t capacity) {
+    if (!s) return KBBQ_E_ARG;
+    std::lock_guard<std::mutex> lock(s->mu);
+    KBBQ_CUDA(cudaSetDevice(s->device));
+    return kmer_begin(s, k, windows, filter_words, capacity);
+}
+
+static int session_kmer_chunk(kbbq_session *s, const uint8_t *seq, int64_t n, bool count) {
+    if (!s) return KBBQ_E_ARG;
+    std::lock_guard<std::mutex> lock(s->mu);
+    KBBQ_CUDA(cudaSetDevice(s->device));
+    UpSlot *u = nullptr;
+    KBBQ_TRY(kmer_chunk(s, seq, n, count, &u));
+    if (u) KBBQ_CUDA(cudaEventSynchronize(u->uploaded));   // the caller may reuse its buffer
+    return KBBQ_OK;
+}
+
+int kbbq_session_kmer_sieve(kbbq_session *s, const uint8_t *seq, int64_t n) { return session_kmer_chunk(s, seq, n, false); }
+
+int kbbq_session_kmer_count(kbbq_session *s, const uint8_t *seq, int64_t n) { return session_kmer_chunk(s, seq, n, true); }
+
+int kbbq_session_kmer_threshold(kbbq_session *s, int min_count, uint64_t *hist_out, int *t_used) {
+    if (!s) return KBBQ_E_ARG;
+    std::lock_guard<std::mutex> lock(s->mu);
+    KBBQ_CUDA(cudaSetDevice(s->device));
+    return kmer_threshold(s, min_count, hist_out, t_used);
+}
+
+int kbbq_session_build_chunk_kmer(kbbq_session *s, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg,
+                                  const uint8_t *second, int64_t n) {
+    if (!s) return KBBQ_E_ARG;
+    std::lock_guard<std::mutex> lock(s->mu);
+    KBBQ_CUDA(cudaSetDevice(s->device));
+    const int64_t k = s->built;
+    KBBQ_TRY(build_chunk_kmer_async(s, seq, qual, rg, second, n));
+    if (n > 0) KBBQ_CUDA(cudaEventSynchronize(s->up[k & 1].uploaded));   // the caller may reuse its buffers
+    return KBBQ_OK;
+}
+
+int kbbq_session_kmer_sizes(const kbbq_session *s, uint64_t *filter_words, uint64_t *capacity) {
+    if (!s) return KBBQ_E_ARG;
+    if (filter_words) *filter_words = s->filter_words;
+    if (capacity) *capacity = s->kmer_cap;
     return KBBQ_OK;
 }
 

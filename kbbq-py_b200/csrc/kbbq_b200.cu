@@ -704,13 +704,19 @@ static bool kmer_table_ok(const void *table, uint64_t capacity) {
     return table && !misaligned(table, 16) && capacity >= 1 && (capacity & (capacity - 1)) == 0;
 }
 
-int kbbq_kmer_table_bytes(int64_t N, int L, int k, uint64_t *capacity, size_t *bytes) {
-    if (N < 0 || L < 1 || k < 1 || k > 31 || !capacity) return KBBQ_E_ARG;
-    const uint64_t windows = (uint64_t)N * (uint64_t)std::max(0, L - k + 1);
+// the default capacity: the smallest power of two >= 1.5 x windows; 0 when that is past 2^59
+static uint64_t kmer_exact_capacity(uint64_t windows) {
     const uint64_t need = windows + (windows + 1) / 2;   // ceil(1.5 x windows)
-    if (need > (1ull << 59)) return KBBQ_E_ARG;
+    if (need > (1ull << 59)) return 0;
     uint64_t cap = 1;
     while (cap < need) cap <<= 1;
+    return cap;
+}
+
+int kbbq_kmer_table_bytes(int64_t N, int L, int k, uint64_t *capacity, size_t *bytes) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !capacity) return KBBQ_E_ARG;
+    const uint64_t cap = kmer_exact_capacity((uint64_t)N * (uint64_t)std::max(0, L - k + 1));
+    if (!cap) return KBBQ_E_ARG;
     *capacity = cap;
     if (bytes) *bytes = (size_t)(cap * 16);
     return KBBQ_OK;
@@ -764,9 +770,9 @@ int kbbq_kmer_flag(const uint8_t *seq, int64_t N, int L, int k, const void *tabl
     const int warps = std::max(1, std::min(4, 49152 / (4 * L)));
     const size_t smem = (size_t)warps * L * 4;
     if (smem > (size_t)max_smem) return KBBQ_E_ARG;
-    if (smem > 49152) KBBQ_CUDA(cudaFuncSetAttribute(kmer_flag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem > 49152) KBBQ_CUDA(cudaFuncSetAttribute(kmer_flag_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t blocks = (N + 32 * warps - 1) / (32 * warps);
-    kmer_flag_kernel<<<(unsigned)blocks, 32 * warps, smem, (cudaStream_t)stream>>>(
+    kmer_flag_kernel<false><<<(unsigned)blocks, 32 * warps, smem, (cudaStream_t)stream>>>(
         seq, N, L, k, (const ulonglong2 *)table, capacity - 1, (unsigned long long)min_count, bits, status);
     KBBQ_LAUNCHED();
     return KBBQ_OK;
@@ -777,6 +783,92 @@ int kbbq_kmer_min_count(const uint64_t *hist) {
     for (int c = 2; c <= 254; ++c)
         if (hist[c] <= hist[c + 1]) return c;
     return 255;
+}
+
+// ---- the sieved table (kmer.cuh, DESIGN.md §10 "Streaming") ----
+
+static bool pow2(uint64_t x) { return x >= 1 && (x & (x - 1)) == 0; }
+
+int kbbq_kmer_stream_plan(uint64_t windows, uint64_t budget_bytes, uint64_t *filter_words, uint64_t *capacity) {
+    if (!filter_words || !capacity) return KBBQ_E_ARG;
+    const uint64_t exact = kmer_exact_capacity(windows);
+    if (!exact) return KBBQ_E_ARG;
+    // filter: the largest power of two with 8 F <= min(W, budget / 4) bytes (one byte per window), at least one word
+    const uint64_t fbytes = std::min(windows, budget_bytes / 4);
+    uint64_t F = 1;
+    while (F <= (1ull << 40) && 16 * F <= fbytes) F <<= 1;
+    // table: the exact rule's capacity, or the largest power of two that fits what the filter leaves
+    const uint64_t min_cap = std::min<uint64_t>(exact, KBBQ_KMER_MIN_SLOTS);
+    if (budget_bytes < 8 * F || (budget_bytes - 8 * F) / 16 < min_cap) return KBBQ_E_UNSUPPORTED;
+    const uint64_t slots = (budget_bytes - 8 * F) / 16;
+    uint64_t cap = min_cap;
+    while (cap < exact && 2 * cap <= slots) cap <<= 1;
+    *filter_words = F;
+    *capacity = cap;
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_sieve(const uint8_t *seq, int64_t N, int L, int k, void *filter, uint64_t filter_words, void *table,
+                    uint64_t capacity, int *status, void *stream) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !status || !kmer_table_ok(table, capacity) || !filter ||
+        misaligned(filter, 8) || !pow2(filter_words))
+        return KBBQ_E_ARG;
+    if (N == 0 || L < k) return KBBQ_OK;
+    if (!seq) return KBBQ_E_ARG;
+    kmer_sieve_kernel<<<(unsigned)((N + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        seq, N, L, k, (unsigned long long *)filter, filter_words - 1, (unsigned long long *)table, capacity - 1, status);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_count_present(const uint8_t *seq, int64_t N, int L, int k, void *table, uint64_t capacity,
+                            uint64_t *windows, int *status, void *stream) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !status || !windows || misaligned(windows, 8) ||
+        !kmer_table_ok(table, capacity))
+        return KBBQ_E_ARG;
+    if (N == 0 || L < k) return KBBQ_OK;
+    if (!seq) return KBBQ_E_ARG;
+    kmer_count_present_kernel<<<(unsigned)((N + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        seq, N, L, k, (unsigned long long *)table, capacity - 1, (unsigned long long *)windows, status);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_histogram_sieved(const void *table, uint64_t capacity, const uint64_t *windows, uint64_t *hist,
+                               void *stream) {
+    if (!kmer_table_ok(table, capacity) || !hist || !windows || misaligned(windows, 8)) return KBBQ_E_ARG;
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    KBBQ_CUDA(cudaMemsetAsync(hist, 0, 256 * sizeof(uint64_t), st));
+    const uint64_t blocks = std::min<uint64_t>((capacity + 255) / 256, (uint64_t)sms * 8);
+    kmer_hist_sieved_kernel<<<(unsigned)blocks, 256, 0, st>>>((const ulonglong2 *)table, capacity,
+                                                              (unsigned long long *)hist);
+    KBBQ_LAUNCHED();
+    kmer_hist_tail_kernel<<<1, 1, 0, st>>>((const unsigned long long *)windows, (unsigned long long *)hist);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_flag_sieved(const uint8_t *seq, int64_t N, int L, int k, const void *table, uint64_t capacity,
+                          int min_count, uint32_t *bits, int *status, void *stream) {
+    if (min_count != 1) return kbbq_kmer_flag(seq, N, L, k, table, capacity, min_count, bits, status, stream);
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !status || !kmer_table_ok(table, capacity)) return KBBQ_E_ARG;
+    if (N == 0) return KBBQ_OK;
+    if (!seq || !bits) return KBBQ_E_ARG;
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    const int warps = std::max(1, std::min(4, 49152 / (4 * L)));   // as kbbq_kmer_flag
+    const size_t smem = (size_t)warps * L * 4;
+    if (smem > (size_t)max_smem) return KBBQ_E_ARG;
+    if (smem > 49152) KBBQ_CUDA(cudaFuncSetAttribute(kmer_flag_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t blocks = (N + 32 * warps - 1) / (32 * warps);
+    kmer_flag_kernel<true><<<(unsigned)blocks, 32 * warps, smem, (cudaStream_t)stream>>>(
+        seq, N, L, k, (const ulonglong2 *)table, capacity - 1, 1ull, bits, status);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
 }
 
 }  // extern "C"

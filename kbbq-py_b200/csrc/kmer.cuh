@@ -12,6 +12,16 @@
 // the key into an empty slot, then add 1 to the count -- one 32-byte sector per probe.  A probe that has walked the
 // whole table raises KBBQ_FLAG_KMER_FULL and gives up.  The counts, and so the flags, do not depend on where a key
 // lands, so any schedule gives the same bits.
+//
+// Sieved table (DESIGN.md §10, "Streaming"): the same slots, filled in two passes over all reads so that the table
+// only has to hold the keys seen at least twice.  Pass A (kmer_sieve_kernel) ORs a pattern of bits into ONE 64-bit
+// word of a filter per window and inserts the key with count 0 when the word already held the whole pattern; the
+// occurrences of a key meet at one word and the atomics on it are serialised, so every occurrence after the first sees
+// the full pattern: every key with count >= 2 is in the table, whatever the schedule (a key seen once lands there only
+// through a false positive).  Pass B (kmer_count_present_kernel) adds 1 to the keys present and counts the valid
+// windows W.  Then h[c] for c >= 2 is binned from the table and h[1] = W - sum of the counts >= 2
+// (kmer_hist_sieved_kernel + kmer_hist_tail_kernel): the exact histogram, so the exact threshold and, for t >= 2,
+// the exact flags from the unchanged kmer_flag_kernel (an absent key has count <= 1 < t); t = 1 needs no lookup.
 #pragma once
 #include "common.cuh"
 
@@ -122,6 +132,8 @@ __device__ __forceinline__ unsigned long long kmer_lookup(const ulonglong2 *tabl
 // k windows over i is solid").  A base's coverage is final once the window that starts at it has been looked up, so
 // the run rule runs one window behind the lookups.  The 32 reads of a warp are 32 L bits = L whole words of the
 // map, starting at word (first read / 32) * L: the warp assembles them in shared memory and stores whole words.
+// ALL_SOLID: every valid window is solid (t = 1 on a sieved table, where a key seen once may be absent); no lookups.
+template <bool ALL_SOLID>
 __global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
                                  unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
     extern __shared__ uint32_t kmer_words[];
@@ -155,7 +167,7 @@ __global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, 
             roll.push(s[e]);
             if (e < k - 1) continue;
             const int j = e - k + 1;
-            if (roll.valid() && kmer_lookup(table, mask, roll.key(), &full) >= t) last = j;
+            if (roll.valid() && (ALL_SOLID || kmer_lookup(table, mask, roll.key(), &full) >= t)) last = j;
             settle(j);
         }
         for (int i = L - k + 1; i < L; ++i) settle(i);
@@ -167,6 +179,131 @@ __global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, 
     const int nwords = (int)((nreads * L + 31) / 32);
     uint32_t *out = bits + (r0 / 32) * L;
     for (int w = lane; w < nwords; w += 32) out[w] = wb[w];
+}
+
+// Filter word and bit pattern of a key for the sieve: splitmix64 of the key plus a constant, so independent of the
+// home slot (splitmix64 of the key).  Word: the low bits; pattern: five bit positions from the top 30 bits.
+__device__ __forceinline__ void kmer_sieve_hash(unsigned long long key, unsigned long long fmask, unsigned long long *w,
+                                                unsigned long long *pattern) {
+    const unsigned long long h = kmer_mix(key + 0x9E3779B97F4A7C15ull);
+    *w = h & fmask;
+    *pattern = (1ull << ((h >> 34) & 63)) | (1ull << ((h >> 40) & 63)) | (1ull << ((h >> 46) & 63)) |
+               (1ull << ((h >> 52) & 63)) | (1ull << (h >> 58));
+}
+
+// Whether some thread has found the table full: a table without an empty slot makes every probe for an absent key
+// walk all of it, so once the flag is up the passes stop probing (the host then reports KBBQ_E_DATA).
+__device__ __forceinline__ bool kmer_table_full(const int *status) {
+    return (*(const volatile int *)status & KBBQ_FLAG_KMER_FULL) != 0;
+}
+
+// Pass A.  One thread per read as kmer_count_kernel; per valid window one 64-bit atomicOr on one filter word, and
+// when the old word held the whole pattern, the key is claimed (count 0) or found in the table.  A thread stops once
+// the table is full.
+__global__ void kmer_sieve_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *filter,
+                                  unsigned long long fmask, unsigned long long *table, unsigned long long mask,
+                                  int *status) {
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= N) return;
+    const uint8_t *s = seq + r * L;
+    KmerRoll roll(k);
+    for (int e = 0; e < L; ++e) {
+        roll.push(s[e]);
+        if (!roll.valid()) continue;
+        const unsigned long long key = roll.key();
+        unsigned long long w, pattern;
+        kmer_sieve_hash(key, fmask, &w, &pattern);
+        if ((atomicOr(filter + w, pattern) & pattern) != pattern) continue;   // first sight (or so it seems)
+        if (kmer_table_full(status)) return;
+        unsigned long long slot = kmer_mix(key) & mask;
+        bool done = false;
+        for (unsigned long long p = 0; p <= mask; ++p) {
+            unsigned long long *kp = table + 2 * slot;
+            unsigned long long cur = __ldcg(kp);
+            if (cur == KMER_EMPTY) {
+                cur = atomicCAS(kp, KMER_EMPTY, key);
+                if (cur == KMER_EMPTY) cur = key;
+            }
+            if (cur == key) {
+                done = true;
+                break;
+            }
+            slot = (slot + 1) & mask;
+        }
+        if (!done) {
+            atomicOr(status, KBBQ_FLAG_KMER_FULL);
+            return;
+        }
+    }
+}
+
+// Pass B.  One thread per read: a key present in the table gets 1 added, an absent one nothing (its count is <= 1).
+// The valid windows of the batch are added to *windows: a warp sum, one atomic per warp.  A probe that walks the
+// whole table (no empty slot: every absent key would cost `capacity` loads) raises KBBQ_FLAG_KMER_FULL, and a thread
+// stops once the flag is up; W is then incomplete, but the table is reported full anyway.
+__global__ void kmer_count_present_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *table,
+                                          unsigned long long mask, unsigned long long *windows, int *status) {
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned int valid = 0;
+    if (r < N) {
+        const uint8_t *s = seq + r * L;
+        KmerRoll roll(k);
+        for (int e = 0; e < L; ++e) {
+            roll.push(s[e]);
+            if (!roll.valid()) continue;
+            if (kmer_table_full(status)) break;   // not return: the whole warp takes part in the sum below
+            ++valid;
+            const unsigned long long key = roll.key();
+            unsigned long long slot = kmer_mix(key) & mask;
+            bool done = false;
+            for (unsigned long long p = 0; p <= mask; ++p) {
+                unsigned long long *kp = table + 2 * slot;
+                const unsigned long long cur = __ldcg(kp);   // no key is inserted in this pass
+                if (cur == key) atomicAdd(kp + 1, 1ull);
+                if (cur == key || cur == KMER_EMPTY) {
+                    done = true;
+                    break;
+                }
+                slot = (slot + 1) & mask;
+            }
+            if (!done) {
+                atomicOr(status, KBBQ_FLAG_KMER_FULL);
+                break;
+            }
+        }
+    }
+    valid = __reduce_add_sync(0xffffffffu, valid);
+    if ((threadIdx.x & 31) == 0 && valid) atomicAdd(windows, (unsigned long long)valid);
+}
+
+// h[c] for c >= 2 from the slots of a sieved table (count >= 255 in bin 255, as kmer_hist_kernel bins), and the sum of
+// those counts, unclipped, into hist[1]; the singletons a false positive let in are not binned.  kmer_hist_tail_kernel
+// then turns hist[1] into W - that sum: the number of keys seen once.
+__global__ void kmer_hist_sieved_kernel(const ulonglong2 *table, unsigned long long capacity, unsigned long long *hist) {
+    __shared__ unsigned int h[256];
+    __shared__ unsigned long long sum;
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) h[i] = 0;
+    if (threadIdx.x == 0) sum = 0;
+    __syncthreads();
+    unsigned long long mine = 0;
+    for (unsigned long long s = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; s < capacity;
+         s += (unsigned long long)gridDim.x * blockDim.x) {
+        const ulonglong2 v = __ldg(table + s);
+        if (v.x != KMER_EMPTY && v.y >= 2) {
+            atomicAdd(&h[v.y < 255 ? v.y : 255], 1u);
+            mine += v.y;
+        }
+    }
+    for (int o = 16; o; o >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, o);
+    if ((threadIdx.x & 31) == 0 && mine) atomicAdd(&sum, mine);
+    __syncthreads();
+    for (int i = 2 + threadIdx.x; i < 256; i += blockDim.x)
+        if (h[i]) atomicAdd(hist + i, (unsigned long long)h[i]);
+    if (threadIdx.x == 0 && sum) atomicAdd(hist + 1, sum);
+}
+
+__global__ void kmer_hist_tail_kernel(const unsigned long long *windows, unsigned long long *hist) {
+    hist[1] = *windows - hist[1];
 }
 
 }  // namespace kbbq

@@ -108,11 +108,27 @@ SIGNATURES = {
     "kbbq_kmer_min_count": (_i, [_vp]),
     "kbbq_kmer_errors_host": (_i, [_vp, _i64, _i, _i, _i, _vp, _vp, C.POINTER(_i), _i]),
     "kbbq_recalibrate_kmer_host": (_i, [_vp] * 4 + [_i64, _i, _i, _i, _i, _i] + [_vp] * 3 + [C.POINTER(_i), C.POINTER(_i), _i]),
+    "kbbq_kmer_stream_plan": (_i, [C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "kbbq_kmer_sieve": (_i, [_vp, _i64, _i, _i, _vp, C.c_uint64, _vp, C.c_uint64, _vp, _vp]),
+    "kbbq_kmer_count_present": (_i, [_vp, _i64, _i, _i, _vp, C.c_uint64, _vp, _vp, _vp]),
+    "kbbq_kmer_histogram_sieved": (_i, [_vp, C.c_uint64, _vp, _vp, _vp]),
+    "kbbq_kmer_flag_sieved": (_i, [_vp, _i64, _i, _i, _vp, C.c_uint64, _i, _vp, _vp, _vp]),
+    "kbbq_session_kmer_begin": (_i, [_vp, _i, _i64, C.c_uint64, C.c_uint64]),
+    "kbbq_session_kmer_sieve": (_i, [_vp, _vp, _i64]),
+    "kbbq_session_kmer_count": (_i, [_vp, _vp, _i64]),
+    "kbbq_session_kmer_threshold": (_i, [_vp, _i, _vp, C.POINTER(_i)]),
+    "kbbq_session_build_chunk_kmer": (_i, [_vp] * 5 + [_i64]),
+    "kbbq_session_kmer_sizes": (_i, [_vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
 }
 
 
 class KbbqNativeError(RuntimeError):
     """The CUDA library is missing, or a CUDA / argument error came back from it."""
+
+
+class DoesNotFit(ValueError):
+    """The reads and the k-mer table of a single-batch call do not fit the GPU's free memory (KBBQ_E_UNSUPPORTED):
+    the streamed path (Session.kmer_*) handles such inputs."""
 
 
 def lib():
@@ -375,10 +391,21 @@ def kmer_min_count(hist):
     return int(lib().kbbq_kmer_min_count(ptr(hist)))
 
 
+def kmer_stream_plan(windows, budget_bytes):
+    """-> (filter_words, capacity) of a sieved k-mer table for `windows` windows within budget_bytes
+    (kbbq_kmer_stream_plan); ValueError when not even the smallest table fits."""
+    f, cap = C.c_uint64(0), C.c_uint64(0)
+    rc = lib().kbbq_kmer_stream_plan(windows, budget_bytes, C.byref(f), C.byref(cap))
+    if rc == E_UNSUPPORTED:
+        raise ValueError("a sieved k-mer table for %d windows does not fit %.3f GB" % (windows, budget_bytes / 1e9))
+    check(rc)
+    return f.value, cap.value
+
+
 def _kmer_check(rc, status, N, L, k, device):
     if rc == E_UNSUPPORTED:
         nbytes = kmer_table_bytes(N, L, k)[1]
-        raise ValueError("%d reads x %d bp with a %.1f GB k-mer table (k = %d) do not fit the free memory of GPU %d"
+        raise DoesNotFit("%d reads x %d bp with a %.1f GB k-mer table (k = %d) do not fit the free memory of GPU %d"
                          % (N, L, nbytes / 1e9, k, device))
     check(rc, status)
 
@@ -535,3 +562,59 @@ class Session:
         a, b = C.c_int64(), C.c_int64()
         check(lib().kbbq_session_traffic(self.h, C.byref(a), C.byref(b)))
         return a.value, b.value
+
+    # ---- `kbbq recalibrate -r` in chunks: a sieved k-mer table (include/kbbq_b200.h, kbbq_session_kmer_*) ----
+
+    def kmer_begin(self, k, windows, filter_words=0, capacity=0):
+        """Allocate and clear the filter and the table for k-mers of length k; 0 sizes them by kbbq_kmer_stream_plan
+        of `windows` (the input's windows) from the free memory.  ValueError when that does not fit."""
+        self.k = int(k)
+        rc = lib().kbbq_session_kmer_begin(self.h, self.k, int(windows), filter_words, capacity)
+        if rc == E_UNSUPPORTED:
+            what = ("%d filter words and %d slots (%.2f GB)" % (filter_words, capacity, (8 * filter_words + 16 * capacity) / 1e9)
+                    if filter_words else "the smallest sieved table for %d windows" % windows)
+            raise ValueError("k-mer table (k = %d): %s do not fit the free memory of GPU %d" % (self.k, what, self.device))
+        check(rc)
+
+    def kmer_sizes(self):
+        """-> (filter_words, capacity) the k-mer buffers were given."""
+        f, cap = C.c_uint64(0), C.c_uint64(0)
+        check(lib().kbbq_session_kmer_sizes(self.h, C.byref(f), C.byref(cap)))
+        return f.value, cap.value
+
+    def kmer_sieve(self, seq):
+        """Pass A over one chunk (every chunk of the input)."""
+        seq = u8(seq).ravel()
+        check(lib().kbbq_session_kmer_sieve(self.h, ptr(seq), seq.size // self.L))
+
+    def kmer_count(self, seq):
+        """Pass B over one chunk (every chunk again, after pass A).  MemoryError, naming the table's size, when the
+        table filled in pass A."""
+        seq = u8(seq).ravel()
+        rc = lib().kbbq_session_kmer_count(self.h, ptr(seq), seq.size // self.L)
+        if rc == E_DATA:
+            self._kmer_full()
+        check(rc)
+
+    def _kmer_full(self):
+        f, cap = self.kmer_sizes()
+        raise MemoryError("the sieved k-mer table (k = %d) of %d slots (%.2f GB) is full: more distinct repeated "
+                          "k-mers than it holds" % (self.k, cap, 16 * cap / 1e9))
+
+    def kmer_threshold(self, min_count=0):
+        """-> (t, hist u64[256]): the exact histogram and the threshold (min_count when > 0, else the first valley).
+        MemoryError, naming the table's size, when it filled."""
+        hist = np.zeros(256, np.uint64)
+        t = C.c_int(0)
+        rc = lib().kbbq_session_kmer_threshold(self.h, int(min_count), ptr(hist), C.byref(t))
+        if rc == E_DATA:
+            self._kmer_full()
+        check(rc)
+        return t.value, hist
+
+    def build_chunk_kmer(self, seq, qual, rg=None, second=None):
+        """Pass 1 of the build for a chunk, its errors flagged from the k-mer table."""
+        seq, qual = u8(seq).ravel(), u8(qual).ravel()
+        rg = _opt(rg, np.uint16)
+        second = _opt(second)
+        check(lib().kbbq_session_build_chunk_kmer(self.h, ptr(seq), ptr(qual), ptr(rg), ptr(second), seq.size // self.L))

@@ -61,6 +61,38 @@ def _stdout_fd():
     return fd
 
 
+def _packed_batches(total, batch_reads, pack):
+    """pack(lo, m) for the batches [lo, lo + m) of reads [0, total), in order; the next batch is tokenised on a worker
+    thread (native code, GIL released) while the caller hands this one to the GPU, so host memory holds two."""
+    from concurrent.futures import ThreadPoolExecutor
+    starts = list(range(0, total, batch_reads))
+    if not starts:
+        return
+    with ThreadPoolExecutor(1) as pool:
+        nxt = pool.submit(pack, starts[0], min(batch_reads, total - starts[0]))
+        for i in range(len(starts)):
+            cur = nxt.result()
+            if i + 1 < len(starts):
+                nxt = pool.submit(pack, starts[i + 1], min(batch_reads, total - starts[i + 1]))
+            yield cur
+
+
+def _apply_pass(sess, reads, rg, second, batch_reads):
+    """Pass 2 of a streaming session whose model is built: every read of `reads` packed again, applied and printed."""
+    L = reads.L
+    fd = _stdout_fd()
+    for lo, m, seq, qual in _packed_batches(reads.N, batch_reads, lambda lo, m: (lo, m) + reads.pack(lo, m)):
+        out = np.empty((m, L), np.uint8)
+        sess.apply_chunk(seq, qual, rg[lo:lo + m], second[lo:lo + m], out)
+        sess.sync()   # raises the reference's exception for bad input; `out` is complete
+        if fd is not None:
+            reads.write(fd, out, lo, m)
+        else:
+            txt = (out + np.uint8(33)).astype(np.uint8)
+            sys.stdout.write(''.join('@%s\n%s\n+\n%s\n' % (reads.name(lo + i), seq[i].tobytes().decode(),
+                                                          txt[i].tobytes().decode('latin-1')) for i in range(m)))
+
+
 def _recalibrate_fastq_streamed(fastq, infer_rg, batch_reads, devices=None):
     """The two passes of kbbq/recalibrate.py:123-156 over batches of `batch_reads` reads through a session
     (kbbq_session_*, csrc/host_api.cu): pass 1 packs a batch from the indexed files and hands it to the session,
@@ -78,43 +110,14 @@ def _recalibrate_fastq_streamed(fastq, infer_rg, batch_reads, devices=None):
         raise ValueError("operands could not be broadcast together: reads of unequal length")
     rg, second, keys = reads.infer(infer_rg)
     L, R = reads.L, max(1, len(keys))
-    from concurrent.futures import ThreadPoolExecutor
     device = _native.device_list(devices)[0]
-
-    def pack(lo, hi_total, with_corr):
-        m = min(batch_reads, hi_total - lo)
-        seq, qual = reads.pack(lo, m)
-        return lo, m, seq, qual, (fixed.pack(lo, m)[0] if with_corr else None)
-
-    def batches(total, with_corr):
-        # the next batch is tokenised (native code, GIL released) while the GPU works on this one
-        starts = list(range(0, total, batch_reads))
-        if not starts:
-            return
-        with ThreadPoolExecutor(1) as pool:
-            nxt = pool.submit(pack, starts[0], total, with_corr)
-            for i in range(len(starts)):
-                cur = nxt.result()
-                if i + 1 < len(starts):
-                    nxt = pool.submit(pack, starts[i + 1], total, with_corr)
-                yield cur
-
     with _native.Session(L, R, 6, chunk_reads=batch_reads, resident_reads=0, device=device) as sess:
-        for lo, m, seq, qual, corr in batches(n_build, True):
+        for lo, m, seq, qual, corr in _packed_batches(n_build, batch_reads,
+                                                      lambda lo, m: (lo, m) + reads.pack(lo, m) + fixed.pack(lo, m)[:1]):
             sess.build_chunk(seq, qual, corr, rg[lo:lo + m], second[lo:lo + m])
         fixed.close()
         sess.model()
-        fd = _stdout_fd()
-        for lo, m, seq, qual, _ in batches(reads.N, False):
-            out = np.empty((m, L), np.uint8)
-            sess.apply_chunk(seq, qual, rg[lo:lo + m], second[lo:lo + m], out)
-            sess.sync()   # raises the reference's exception for bad input; `out` is complete
-            if fd is not None:
-                reads.write(fd, out, lo, m)
-            else:
-                txt = (out + np.uint8(33)).astype(np.uint8)
-                sys.stdout.write(''.join('@%s\n%s\n+\n%s\n' % (reads.name(lo + i), seq[i].tobytes().decode(),
-                                                              txt[i].tobytes().decode('latin-1')) for i in range(m)))
+        _apply_pass(sess, reads, rg, second, batch_reads)
     reads.close()
 
 
@@ -189,23 +192,62 @@ def recalibrate_fastq(fastq, infer_rg=False, devices=None):
     w.write(''.join(chunks))
 
 
+def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device):
+    """recalibrate_reads through a streaming session, for files of any size (DESIGN.md §10, "Streaming"): two passes
+    over every batch fill a sieved k-mer table that only holds the k-mers seen at least twice (A: sieve, B: count),
+    the threshold is taken from its histogram -- the exact one --, a third pass flags and builds, the model runs once
+    and a fourth pass applies and prints, as _recalibrate_fastq_streamed does.  Host memory holds two batches (plus
+    the index of the file); the output is the single-batch path's, byte for byte."""
+    if reads.L < 0:
+        raise ValueError("%s: reads of unequal length are not supported on this path" % reads.path)
+    rg, second, keys = reads.infer(infer_rg)
+    N, L, R = reads.N, reads.L, max(1, len(keys))
+
+    def seq_only(lo, m):
+        return reads.pack(lo, m)[0]
+
+    with _native.Session(L, R, 6, chunk_reads=batch_reads, resident_reads=0, device=device) as sess:
+        sess.kmer_begin(k, N * max(0, L - k + 1))
+        for seq in _packed_batches(N, batch_reads, seq_only):
+            sess.kmer_sieve(seq)
+        for seq in _packed_batches(N, batch_reads, seq_only):
+            sess.kmer_count(seq)
+        sess.kmer_threshold(min_count)
+        for lo, m, seq, qual in _packed_batches(N, batch_reads, lambda lo, m: (lo, m) + reads.pack(lo, m)):
+            sess.build_chunk_kmer(seq, qual, rg[lo:lo + m], second[lo:lo + m])
+        sess.model()
+        _apply_pass(sess, reads, rg, second, batch_reads)
+
+
 def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None):
     """Recalibrate the reads of one FASTQ file with the errors found from their own k-mer counts (kbbq.kmer); FASTQ to
-    stdout as recalibrate_fastq prints it.  The whole file is one batch on the first of `devices`."""
+    stdout as recalibrate_fastq prints it, on the first of `devices`.  The file is one batch unless KBBQ_BATCH_READS
+    is set, the file is larger than STREAM_ABOVE_BYTES, or the batch and its k-mer table do not fit the GPU: then it
+    streams through in batches (_recalibrate_reads_streamed), with the same output."""
+    import os
     from . import fastx
     if not 1 <= k <= 31:
         raise ValueError("k must be in 1..31, got %d" % k)
     if min_count < 0:
         raise ValueError("min_count must be >= 0, got %d" % min_count)
+    batch_reads = int(os.environ.get("KBBQ_BATCH_READS", "0"))
+    if batch_reads <= 0 and _fastq_size(path) > STREAM_ABOVE_BYTES:
+        batch_reads = STREAM_BATCH_READS
+    device = _native.device_list(devices)[0]
     reads = fastx.NativeFastq(path)
     try:
         if reads.N == 0:
             return
+        if batch_reads > 0:
+            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device)
         seq, qual = reads.pack()   # ValueError for reads of unequal length, as on the -f path
         rg, second, keys = reads.infer(infer_rg)
         L, R = reads.L, max(1, len(keys))
-        out, _ = _native.recalibrate_kmer_host(seq, qual, rg, second, L, R, 6, k, min_count,
-                                               device=_native.device_list(devices)[0])
+        try:
+            out, _ = _native.recalibrate_kmer_host(seq, qual, rg, second, L, R, 6, k, min_count, device=device)
+        except _native.DoesNotFit:
+            del seq, qual
+            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, STREAM_BATCH_READS, device)
         fd = _stdout_fd()
         if fd is not None:
             reads.write(fd, out)
