@@ -57,7 +57,7 @@ extern "C" {
 #define KBBQ_FLAG_BAD_BASE 2   /* a base outside ACGTN: TypeError in Dinucleotide.vecget */
 #define KBBQ_FLAG_RG_RANGE 4   /* rg[i] >= R */
 #define KBBQ_FLAG_SEGMENTS 8   /* kbbq_*_segmented: malformed span table (not sorted / not 16-row aligned / past rows_bound) */
-#define KBBQ_FLAG_KMER_FULL 16 /* kbbq_kmer_count / _sieve / _flag: a probe walked the whole k-mer table */
+#define KBBQ_FLAG_KMER_FULL 16 /* kbbq_kmer_count / _sieve / _flag / _correct: a probe walked the whole k-mer table */
 
 int kbbq_abi_version(void);
 const char *kbbq_strerror(int code);
@@ -558,6 +558,41 @@ int kbbq_session_build_chunk_kmer(kbbq_session *s, const uint8_t *seq, const uin
                                   const uint8_t *second, int64_t n);
 /* sizes the session's k-mer buffers were given (0 before kmer_begin) */
 int kbbq_session_kmer_sizes(const kbbq_session *s, uint64_t *filter_words, uint64_t *capacity);
+
+/*
+ * The correcting walk (DESIGN.md §10): an opt-in rule that finds the errors by correcting each read against its
+ * trusted k-mers, as k-mer correctors such as Lighter do.  The boundary rule above flags only the two ends of each
+ * uncovered run, so it misses the inner errors of a cluster within k and the outer error of a run at a read end.
+ * Counts, keys, validity, t and solid as above; nw = L - k + 1, and L < k flags nothing.  Per read:
+ *   1. no solid window: nothing is flagged;
+ *   2. the anchor is the longest maximal run [a0, a1] of solid windows, the leftmost of equal ones;
+ *   3. right walk on a copy w of the read, j = a1 + 1 .. nw - 1: a solid window j of w goes on to j + 1; otherwise
+ *      e = j + k - 1, a w[e] that is not A/C/G/T stops the walk, and for each c in A, C, G, T with c != w[e],
+ *      score(c) = the consecutive solid windows j, j + 1, ... of w with w[e] = c, at most min(k, nw - j).  e is
+ *      flagged; when exactly one c reaches the best score and it is >= 1, w[e] = c and the walk goes on to j + 1,
+ *      else it stops;
+ *   4. left walk, the mirror image: j = a0 - 1 down to 0, e = j, at most min(k, j + 1) windows j, j - 1, ...
+ * Every flagged base is A/C/G/T.  The bits depend only on the counts.  On a sieved table with t >= 2 they equal the
+ * exact table's (an absent key has count <= 1 < t).
+ *
+ * kbbq_kmer_correct: the map by this rule, on an exact or a sieved table, same arguments and buffers as
+ * kbbq_kmer_flag.  min_count == 1 (every valid window solid) only zeroes the map.  A probe that walks the whole table
+ * raises KBBQ_FLAG_KMER_FULL.  kbbq_kmer_errors_rule_host / kbbq_recalibrate_kmer_rule_host: kbbq_kmer_errors_host /
+ * kbbq_recalibrate_kmer_host with the rule given (kbbq_kmer_errors_host and kbbq_recalibrate_kmer_host are rule
+ * KBBQ_KMER_BOUNDARIES).  kbbq_session_kmer_rule: the rule of a streaming session's build_chunk_kmer, allowed from
+ * kmer_begin until the first build_chunk_kmer.  An unknown rule or a call out of order returns KBBQ_E_ARG.
+ */
+#define KBBQ_KMER_BOUNDARIES 0
+#define KBBQ_KMER_CORRECT 1
+int kbbq_kmer_correct(const uint8_t *seq_dev, int64_t N, int L, int k, const void *table_dev, uint64_t capacity,
+                      int min_count, uint32_t *bits_dev, int *status_dev, void *stream);
+int kbbq_kmer_errors_rule_host(const uint8_t *seq, int64_t N, int L, int k, int min_count, int rule, uint32_t *bits_out,
+                               uint64_t *hist_out, int *min_count_used, int device);
+int kbbq_recalibrate_kmer_rule_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second,
+                                    int64_t N, int L, int R, int minscore, int k, int min_count, int rule,
+                                    uint8_t *out_qual, int64_t *tables_host, int64_t *deltas_host, int *min_count_used,
+                                    int *status_out, int device);
+int kbbq_session_kmer_rule(kbbq_session *s, int rule);
 
 /* Number of kernel launches this library has issued since load (bench.py's gpu_launches). */
 int64_t kbbq_launch_count(void);

@@ -21,7 +21,7 @@
 // `kbbq recalibrate -r` streams through the same session: kbbq_session_kmer_sieve x n and kbbq_session_kmer_count x n
 // fill a sieved k-mer table (kmer.cuh) in the same slots and streams, kbbq_session_kmer_threshold takes the exact
 // histogram, and kbbq_session_build_chunk_kmer is pass 1 with the map flagged on the device in place of the corrected
-// reads.
+// reads -- by the boundary rule, or by the correcting walk after kbbq_session_kmer_rule (`-r --correct`).
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -155,6 +155,9 @@ struct kbbq_session {
     void *kmer_filter = nullptr, *kmer_base = nullptr, *kmer_table = nullptr;
     uint64_t *kmer_windows = nullptr, *kmer_hist = nullptr;
     uint32_t *kmer_bits = nullptr;
+    // the rule build_chunk_kmer flags by (kbbq_session_kmer_rule), and whether it has flagged a chunk yet
+    int kmer_rule = KBBQ_KMER_BOUNDARIES;
+    bool kmer_built = false;
     std::mutex mu;
 
     ~kbbq_session() {
@@ -309,6 +312,8 @@ int kmer_release(kbbq_session *S) {
     S->filter_words = S->kmer_cap = 0;
     S->kmer_stage = KMER_NONE;
     S->kmer_chunks = 0;
+    S->kmer_rule = KBBQ_KMER_BOUNDARIES;
+    S->kmer_built = false;
     return KBBQ_OK;
 }
 
@@ -412,8 +417,12 @@ int build_chunk_finish(kbbq_session *S, int64_t k, const uint8_t *seq, const uin
     KBBQ_CUDA(cudaEventRecord(u.uploaded, S->s_up));
     KBBQ_CUDA(cudaStreamWaitEvent(S->s_comp, u.uploaded, 0));
     if (kmer) {
-        KBBQ_TRY(kbbq_kmer_flag_sieved(p.d_seq, n, L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_t, S->kmer_bits,
+        if (S->kmer_rule == KBBQ_KMER_CORRECT)
+            KBBQ_TRY(kbbq_kmer_correct(p.d_seq, n, L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_t, S->kmer_bits,
                                        S->d_status, S->s_comp));
+        else
+            KBBQ_TRY(kbbq_kmer_flag_sieved(p.d_seq, n, L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_t,
+                                           S->kmer_bits, S->d_status, S->s_comp));
         KBBQ_TRY(kbbq_expand_mismatch_bits(p.d_seq, S->kmer_bits, (int64_t)nb, u.corr, S->s_comp));
     } else if (S->pack == PACK_NIBBLES) KBBQ_TRY(kbbq_expand_nibbles((const uint8_t *)u.bits, (int64_t)nb, p.d_seq, u.corr, S->s_comp));
     else if (S->pack == PACK_BITS) KBBQ_TRY(kbbq_expand_mismatch_bits(p.d_seq, u.bits, (int64_t)nb, u.corr, S->s_comp));
@@ -549,11 +558,20 @@ int kmer_threshold(kbbq_session *S, int min_count, uint64_t *hist_out, int *t_us
     return KBBQ_OK;
 }
 
+// the rule may change from kmer_begin until a chunk has been flagged: every chunk of a run is flagged by one rule
+int kmer_rule(kbbq_session *S, int rule) {
+    if ((rule != KBBQ_KMER_BOUNDARIES && rule != KBBQ_KMER_CORRECT) || S->kmer_stage == KMER_NONE || S->kmer_built)
+        return KBBQ_E_ARG;
+    S->kmer_rule = rule;
+    return KBBQ_OK;
+}
+
 int build_chunk_kmer_async(kbbq_session *S, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg,
                            const uint8_t *second, int64_t n) {
     if (S->kmer_stage != KMER_READY || n < 0 || n > S->C) return KBBQ_E_ARG;
     if (n == 0) return KBBQ_OK;
     if (!seq || !qual) return KBBQ_E_ARG;
+    S->kmer_built = true;
     const int64_t k = S->built++;
     KBBQ_TRY(build_chunk_upload(S, k, seq, qual, rg, second, n, false, true));
     return build_chunk_finish(S, k, seq, nullptr, rg != nullptr, second != nullptr, n, false);
@@ -812,6 +830,12 @@ int kbbq_session_kmer_threshold(kbbq_session *s, int min_count, uint64_t *hist_o
     std::lock_guard<std::mutex> lock(s->mu);
     KBBQ_CUDA(cudaSetDevice(s->device));
     return kmer_threshold(s, min_count, hist_out, t_used);
+}
+
+int kbbq_session_kmer_rule(kbbq_session *s, int rule) {
+    if (!s) return KBBQ_E_ARG;
+    std::lock_guard<std::mutex> lock(s->mu);
+    return kmer_rule(s, rule);
 }
 
 int kbbq_session_build_chunk_kmer(kbbq_session *s, const uint8_t *seq, const uint8_t *qual, const uint16_t *rg,
@@ -1628,9 +1652,9 @@ int kbbq_marginals_host(const int64_t *pos_errs, const int64_t *pos_total, int L
 
 namespace {
 
-// clear + count + histogram, the threshold on the host, then the flags.  A full table stops before the flags:
-// *status = KBBQ_FLAG_KMER_FULL and KBBQ_E_DATA.
-int kmer_errors_dev(const uint8_t *seq, int64_t N, int L, int k, int min_count, void *table, uint64_t cap,
+// clear + count + histogram, the threshold on the host, then the flags by `rule`.  A full table stops before the
+// flags: *status = KBBQ_FLAG_KMER_FULL and KBBQ_E_DATA.
+int kmer_errors_dev(const uint8_t *seq, int64_t N, int L, int k, int min_count, int rule, void *table, uint64_t cap,
                     uint64_t *d_hist, uint32_t *bits, int *d_status, uint64_t *hist, int *t, int *status) {
     KBBQ_TRY(kbbq_kmer_clear(table, cap, nullptr));
     KBBQ_TRY(kbbq_kmer_count(seq, N, L, k, table, cap, d_status, nullptr));
@@ -1639,8 +1663,11 @@ int kmer_errors_dev(const uint8_t *seq, int64_t N, int L, int k, int min_count, 
     KBBQ_CUDA(cudaMemcpy(status, d_status, sizeof(int), cudaMemcpyDeviceToHost));
     if (*status) return KBBQ_E_DATA;
     *t = min_count > 0 ? min_count : kbbq_kmer_min_count(hist);
+    if (rule == KBBQ_KMER_CORRECT) return kbbq_kmer_correct(seq, N, L, k, table, cap, *t, bits, d_status, nullptr);
     return kbbq_kmer_flag(seq, N, L, k, table, cap, *t, bits, d_status, nullptr);
 }
+
+bool kmer_rule_ok(int rule) { return rule == KBBQ_KMER_BOUNDARIES || rule == KBBQ_KMER_CORRECT; }
 
 }  // namespace
 
@@ -1648,7 +1675,14 @@ extern "C" {
 
 int kbbq_kmer_errors_host(const uint8_t *seq, int64_t N, int L, int k, int min_count, uint32_t *bits_out,
                           uint64_t *hist_out, int *min_count_used, int device) {
-    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 0 || (N > 0 && (!seq || !bits_out))) return KBBQ_E_ARG;
+    return kbbq_kmer_errors_rule_host(seq, N, L, k, min_count, KBBQ_KMER_BOUNDARIES, bits_out, hist_out, min_count_used,
+                                      device);
+}
+
+int kbbq_kmer_errors_rule_host(const uint8_t *seq, int64_t N, int L, int k, int min_count, int rule, uint32_t *bits_out,
+                               uint64_t *hist_out, int *min_count_used, int device) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 0 || !kmer_rule_ok(rule) || (N > 0 && (!seq || !bits_out)))
+        return KBBQ_E_ARG;
     uint64_t cap = 0;
     size_t table_bytes = 0;
     KBBQ_TRY(kbbq_kmer_table_bytes(N, L, k, &cap, &table_bytes));
@@ -1664,8 +1698,8 @@ int kbbq_kmer_errors_host(const uint8_t *seq, int64_t N, int L, int k, int min_c
     KBBQ_TRY(c.begin());
     uint64_t hist[256];
     int t = 0, st = 0;
-    KBBQ_TRY(kmer_errors_dev(d_seq, N, L, k, min_count, table, cap, (uint64_t *)(void *)d_hist, d_bits, c.status, hist,
-                             &t, &st));
+    KBBQ_TRY(kmer_errors_dev(d_seq, N, L, k, min_count, rule, table, cap, (uint64_t *)(void *)d_hist, d_bits, c.status,
+                             hist, &t, &st));
     if (hist_out) memcpy(hist_out, hist, sizeof(hist));
     if (min_count_used) *min_count_used = t;
     return c.finish();
@@ -1675,7 +1709,16 @@ int kbbq_recalibrate_kmer_host(const uint8_t *seq, const uint8_t *qual, const ui
                                int64_t N, int L, int R, int minscore, int k, int min_count, uint8_t *out_qual,
                                int64_t *tables_host, int64_t *deltas_host, int *min_count_used, int *status_out,
                                int device) {
-    if (N < 0 || L < 1 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ || k < 1 || k > 31 || min_count < 0)
+    return kbbq_recalibrate_kmer_rule_host(seq, qual, rg, second, N, L, R, minscore, k, min_count, KBBQ_KMER_BOUNDARIES,
+                                           out_qual, tables_host, deltas_host, min_count_used, status_out, device);
+}
+
+int kbbq_recalibrate_kmer_rule_host(const uint8_t *seq, const uint8_t *qual, const uint16_t *rg, const uint8_t *second,
+                                    int64_t N, int L, int R, int minscore, int k, int min_count, int rule,
+                                    uint8_t *out_qual, int64_t *tables_host, int64_t *deltas_host, int *min_count_used,
+                                    int *status_out, int device) {
+    if (N < 0 || L < 1 || R < 1 || R > 65535 || minscore < 0 || minscore >= NQ || k < 1 || k > 31 || min_count < 0 ||
+        !kmer_rule_ok(rule))
         return KBBQ_E_ARG;
     if (N > 0 && (!seq || !qual || !out_qual)) return KBBQ_E_ARG;
     uint64_t cap = 0;
@@ -1703,7 +1746,7 @@ int kbbq_recalibrate_kmer_host(const uint8_t *seq, const uint8_t *qual, const ui
     KBBQ_TRY(c.begin());
     uint64_t hist[256];
     int t = 0, st = 0;
-    const int rc = kmer_errors_dev(d_seq, N, L, k, min_count, table, cap, (uint64_t *)(void *)d_hist,
+    const int rc = kmer_errors_dev(d_seq, N, L, k, min_count, rule, table, cap, (uint64_t *)(void *)d_hist,
                                    (uint32_t *)(void *)d_bits, c.status, hist, &t, &st);
     if (rc == KBBQ_E_DATA && status_out) *status_out = st;
     KBBQ_TRY(rc);

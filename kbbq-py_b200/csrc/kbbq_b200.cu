@@ -871,4 +871,32 @@ int kbbq_kmer_flag_sieved(const uint8_t *seq, int64_t N, int L, int k, const voi
     return KBBQ_OK;
 }
 
+// ---- the correcting walk (kmer.cuh, DESIGN.md §10 "The correcting walk") ----
+
+int kbbq_kmer_correct(const uint8_t *seq, int64_t N, int L, int k, const void *table, uint64_t capacity, int min_count,
+                      uint32_t *bits, int *status, void *stream) {
+    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 1 || !status || !kmer_table_ok(table, capacity))
+        return KBBQ_E_ARG;
+    if (N == 0) return KBBQ_OK;
+    if (!seq || !bits) return KBBQ_E_ARG;
+    if (min_count == 1) {   // every valid window is solid: nothing is flagged
+        KBBQ_CUDA(cudaMemsetAsync(bits, 0, ((size_t)N * L + 31) / 32 * 4, (cudaStream_t)stream));
+        return KBBQ_OK;
+    }
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    // a warp's map words and its reads' solid bits: 4 warps a block while that stays under 48 KB
+    const int words = kmer_correct_warp_words(L, k);
+    const int warps = std::max(1, std::min(4, 49152 / (4 * words)));
+    const size_t smem = (size_t)warps * words * 4;
+    if (smem > (size_t)max_smem) return KBBQ_E_ARG;
+    if (smem > 49152) KBBQ_CUDA(cudaFuncSetAttribute(kmer_correct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t blocks = (N + 32 * warps - 1) / (32 * warps);
+    kmer_correct_kernel<<<(unsigned)blocks, 32 * warps, smem, (cudaStream_t)stream>>>(
+        seq, N, L, k, (const ulonglong2 *)table, capacity - 1, (unsigned long long)min_count, bits, status);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
 }  // extern "C"

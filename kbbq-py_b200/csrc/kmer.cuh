@@ -22,6 +22,9 @@
 // windows W.  Then h[c] for c >= 2 is binned from the table and h[1] = W - sum of the counts >= 2
 // (kmer_hist_sieved_kernel + kmer_hist_tail_kernel): the exact histogram, so the exact threshold and, for t >= 2,
 // the exact flags from the unchanged kmer_flag_kernel (an absent key has count <= 1 < t); t = 1 needs no lookup.
+//
+// The correcting walk (kmer_correct_kernel, below; DESIGN.md §10): an opt-in second rule on the same table that finds
+// every error of a cluster and those at read ends by correcting each read against its trusted k-mers.
 #pragma once
 #include "common.cuh"
 
@@ -304,6 +307,192 @@ __global__ void kmer_hist_sieved_kernel(const ulonglong2 *table, unsigned long l
 
 __global__ void kmer_hist_tail_kernel(const unsigned long long *windows, unsigned long long *hist) {
     hist[1] = *windows - hist[1];
+}
+
+// ---- the correcting walk (kbbq_kmer_correct, DESIGN.md §10 "The correcting walk") ----
+//
+// The rule, per read (nw = L - k + 1 windows; L < k flags nothing); counts, keys, validity and solid (count >= t) as
+// above:
+//   1. solid[j] for every window of the read.  No solid window: nothing is flagged.
+//   2. Anchor: the longest maximal run [a0, a1] of solid windows, the leftmost of equal ones.
+//   3. Right walk over a copy w of the read, j = a1 + 1 .. nw - 1: a solid window j of w goes on to j + 1.  Otherwise
+//      e = j + k - 1 (the one base of window j not in the solid window j - 1); w[e] not A/C/G/T stops the walk.  For
+//      each c in A, C, G, T with c != w[e], score(c) = the number of consecutive solid windows j, j + 1, ... of w with
+//      w[e] = c, at most min(k, nw - j).  e is flagged; a best score >= 1 that exactly one c reaches sets w[e] = c and
+//      goes on to j + 1, anything else (a tie, no candidate) stops.
+//   4. Left walk, the mirror image: j = a0 - 1 down to 0, e = j, scores over windows j, j - 1, ..., at most
+//      min(k, j + 1).  The right walk changes bases >= a1 + k, the left walk bases < a0: the order does not matter.
+// Every flagged base is A/C/G/T.  The bits depend only on the counts, so any schedule gives the same bits; on a sieved
+// table with t >= 2 an absent key has count <= 1 < t, so it gives the exact table's bits.  With t = 1 every valid
+// window is solid and nothing is flagged (the host writes a zero map and launches nothing).
+//
+// The kernel: one thread per read, one warp per 32 reads and the map words in shared memory, as kmer_flag_kernel.
+// The first pass looks every window up once and keeps its solid bit in shared memory next to the warp's map words
+// (word i of a lane at [32 i + lane]: no bank conflict) while it tracks the anchor.  The walks need no copy of the
+// read: the right walk keeps the code of window j - 1 of w, a candidate's windows are that code rolled with c and then
+// with the read's own bases beyond e (everything right of e is unchanged), and the left walk prepends.  A window that
+// holds no corrected base reuses its first-pass bit.  After a correction the windows its score counted are known
+// solid, and when that score is below k the next one is known not to be: the walk moves past them without a lookup.
+
+// forward and reverse-complement 2-bit codes of one window, rolled at either end
+struct KmerCode {
+    unsigned long long fwd, rc;
+    __device__ __forceinline__ void append(int c, unsigned long long kmask, int shift) {
+        fwd = ((fwd << 2) | (unsigned)c) & kmask;
+        rc = (rc >> 2) | ((unsigned long long)(3 - c) << shift);
+    }
+    __device__ __forceinline__ void prepend(int c, unsigned long long kmask, int shift) {
+        fwd = (fwd >> 2) | ((unsigned long long)c << shift);
+        rc = ((rc << 2) | (unsigned)(3 - c)) & kmask;
+    }
+    __device__ __forceinline__ unsigned long long key() const { return fwd < rc ? fwd : rc; }
+};
+
+// shared-memory words a warp of kmer_correct_kernel uses: the L map words of its 32 reads, then ceil(nw / 32) words
+// of solid bits per read
+__host__ __device__ __forceinline__ int kmer_correct_warp_words(int L, int k) {
+    return L + (L >= k ? 32 * ((L - k + 1 + 31) >> 5) : 0);
+}
+
+__global__ void kmer_correct_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
+                                    unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
+    extern __shared__ uint32_t kmer_words[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long r0 = ((long long)blockIdx.x * (blockDim.x >> 5) + warp) * 32;
+    if (r0 >= N) return;
+    uint32_t *wb = kmer_words + (size_t)warp * kmer_correct_warp_words(L, k);
+    for (int w = lane; w < L; w += 32) wb[w] = 0;
+    __syncwarp();
+    const long long r = r0 + lane;
+    const int nw = L - k + 1;
+    if (r < N && nw > 0) {
+        const uint8_t *s = seq + r * L;
+        const int base_bit = lane * L;
+        uint32_t *sol = wb + L + lane;   // solid bit of window j: bit j & 31 of sol[32 * (j >> 5)]
+        const unsigned long long kmask = (1ull << (2 * k)) - 1;
+        const int shift = 2 * (k - 1);
+        bool full = false;
+        auto flag = [&](int i) { atomicOr(&wb[(base_bit + i) >> 5], 1u << ((base_bit + i) & 31)); };
+        auto solid = [&](const KmerCode &x) { return kmer_lookup(table, mask, x.key(), &full) >= t; };
+        auto was_solid = [&](int j) { return (sol[32 * (j >> 5)] >> (j & 31)) & 1u; };
+        auto code_at = [&](int p) {   // window p of the read, all A/C/G/T
+            KmerCode x{0, 0};
+            for (int i = 0; i < k; ++i) x.append(kmer_code(s[p + i]), kmask, shift);
+            return x;
+        };
+
+        // first pass: solid bits and the anchor
+        KmerRoll roll(k);
+        int a0 = 0, best = 0, run = 0;
+        uint32_t word = 0;
+        for (int e = 0; e < L; ++e) {
+            roll.push(s[e]);
+            if (e < k - 1) continue;
+            const int j = e - k + 1;
+            const bool ok = roll.valid() && kmer_lookup(table, mask, roll.key(), &full) >= t;
+            word |= (uint32_t)ok << (j & 31);
+            if ((j & 31) == 31 || j == nw - 1) {
+                sol[32 * (j >> 5)] = word;
+                word = 0;
+            }
+            run = ok ? run + 1 : 0;
+            if (run > best) {
+                best = run;
+                a0 = j - run + 1;
+            }
+        }
+
+        if (best > 0) {
+            // right walk: x is window j - 1 of w; known_bad: window j holds the last correction and is not solid
+            const int a1 = a0 + best - 1;
+            KmerCode x = code_at(a1);
+            bool known_bad = false;
+            for (int j = a1 + 1; j < nw;) {
+                const int e = j + k - 1;
+                const int b = kmer_code(s[e]);
+                if (!known_bad && b >= 0 && was_solid(j)) {
+                    x.append(b, kmask, shift);
+                    ++j;
+                    continue;
+                }
+                if (b < 0) break;
+                flag(e);
+                const int m = min(k, nw - j);
+                int best_c = -1, best_n = 0;
+                bool tie = false;
+                for (int c = 0; c < 4; ++c) {
+                    if (c == b) continue;
+                    KmerCode y = x;
+                    y.append(c, kmask, shift);
+                    int n = 0;
+                    while (solid(y) && ++n < m) {
+                        const int nb = kmer_code(s[e + n]);
+                        if (nb < 0) break;
+                        y.append(nb, kmask, shift);
+                    }
+                    if (n > best_n) {
+                        best_n = n;
+                        best_c = c;
+                        tie = false;
+                    } else if (n == best_n && n > 0) {
+                        tie = true;
+                    }
+                }
+                if (best_n == 0 || tie) break;
+                x.append(best_c, kmask, shift);
+                for (int i = 1; i < best_n; ++i) x.append(kmer_code(s[e + i]), kmask, shift);
+                j += best_n;
+                known_bad = best_n < k;
+            }
+
+            // left walk: x is window j + 1 of w
+            x = code_at(a0);
+            known_bad = false;
+            for (int j = a0 - 1; j >= 0;) {
+                const int e = j;
+                const int b = kmer_code(s[e]);
+                if (!known_bad && b >= 0 && was_solid(j)) {
+                    x.prepend(b, kmask, shift);
+                    --j;
+                    continue;
+                }
+                if (b < 0) break;
+                flag(e);
+                const int m = min(k, j + 1);
+                int best_c = -1, best_n = 0;
+                bool tie = false;
+                for (int c = 0; c < 4; ++c) {
+                    if (c == b) continue;
+                    KmerCode y = x;
+                    y.prepend(c, kmask, shift);
+                    int n = 0;
+                    while (solid(y) && ++n < m) {
+                        const int nb = kmer_code(s[e - n]);
+                        if (nb < 0) break;
+                        y.prepend(nb, kmask, shift);
+                    }
+                    if (n > best_n) {
+                        best_n = n;
+                        best_c = c;
+                        tie = false;
+                    } else if (n == best_n && n > 0) {
+                        tie = true;
+                    }
+                }
+                if (best_n == 0 || tie) break;
+                x.prepend(best_c, kmask, shift);
+                for (int i = 1; i < best_n; ++i) x.prepend(kmer_code(s[e - i]), kmask, shift);
+                j -= best_n;
+                known_bad = best_n < k;
+            }
+        }
+        if (full) atomicOr(status, KBBQ_FLAG_KMER_FULL);
+    }
+    __syncwarp();
+    const long long nreads = N - r0 < 32 ? N - r0 : 32;
+    const int nwords = (int)((nreads * L + 31) / 32);
+    uint32_t *out = bits + (r0 / 32) * L;
+    for (int w = lane; w < nwords; w += 32) out[w] = wb[w];
 }
 
 }  // namespace kbbq

@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(HERE, "libkbbq_b200.so")
 NQ = 43
 FLAG_QUAL_RANGE, FLAG_BAD_BASE, FLAG_RG_RANGE, FLAG_SEGMENTS = 1, 2, 4, 8
 FLAG_KMER_FULL = 16
+KMER_BOUNDARIES, KMER_CORRECT = 0, 1   # k-mer error rules (include/kbbq_b200.h)
 APPLY_BASES_CHECKED = 0x10   # kbbq_apply path flag: skip the base check (include/kbbq_b200.h)
 E_DATA = -4
 E_UNSUPPORTED = -12
@@ -119,6 +120,10 @@ SIGNATURES = {
     "kbbq_session_kmer_threshold": (_i, [_vp, _i, _vp, C.POINTER(_i)]),
     "kbbq_session_build_chunk_kmer": (_i, [_vp] * 5 + [_i64]),
     "kbbq_session_kmer_sizes": (_i, [_vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "kbbq_kmer_correct": (_i, [_vp, _i64, _i, _i, _vp, C.c_uint64, _i, _vp, _vp, _vp]),
+    "kbbq_kmer_errors_rule_host": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, _vp, C.POINTER(_i), _i]),
+    "kbbq_recalibrate_kmer_rule_host": (_i, [_vp] * 4 + [_i64, _i, _i, _i, _i, _i, _i] + [_vp] * 3 + [C.POINTER(_i), C.POINTER(_i), _i]),
+    "kbbq_session_kmer_rule": (_i, [_vp, _i]),
 }
 
 
@@ -410,8 +415,9 @@ def _kmer_check(rc, status, N, L, k, device):
     check(rc, status)
 
 
-def kmer_errors_host(seq, L, k=23, min_count=0, device=None):
-    """Errors from the batch's k-mer counts (kbbq_kmer_errors_host) -> (bits u32[ceil(N*L/32)], hist u64[256], t)."""
+def kmer_errors_host(seq, L, k=23, min_count=0, device=None, rule=KMER_BOUNDARIES):
+    """Errors from the batch's k-mer counts (kbbq_kmer_errors_rule_host) by `rule` (KMER_BOUNDARIES or KMER_CORRECT)
+    -> (bits u32[ceil(N*L/32)], hist u64[256], t)."""
     seq = u8(seq).ravel()
     N = seq.size // L
     assert seq.size == N * L
@@ -419,14 +425,16 @@ def kmer_errors_host(seq, L, k=23, min_count=0, device=None):
     hist = np.zeros(256, np.uint64)
     t = C.c_int(0)
     dev = _dev(device)
-    rc = lib().kbbq_kmer_errors_host(ptr(seq), N, L, k, min_count, ptr(bits), ptr(hist), C.byref(t), dev)
+    rc = lib().kbbq_kmer_errors_rule_host(ptr(seq), N, L, k, min_count, rule, ptr(bits), ptr(hist), C.byref(t), dev)
     _kmer_check(rc, FLAG_KMER_FULL, N, L, k, dev)   # a full table is the only data error of this entry point
     return bits, hist, t.value
 
 
-def recalibrate_kmer_host(seq, qual, rg, second, L, R, minscore=6, k=23, min_count=0, want_tables=False, device=None):
-    """The whole path with the errors found from the reads' k-mer counts (kbbq_recalibrate_kmer_host)
-    -> (out_qual [N, L] u8, t), or (out_qual, t, tables, deltas) as recalibrate_host's with want_tables."""
+def recalibrate_kmer_host(seq, qual, rg, second, L, R, minscore=6, k=23, min_count=0, want_tables=False, device=None,
+                          correct=False):
+    """The whole path with the errors found from the reads' k-mer counts (kbbq_recalibrate_kmer_rule_host; correct:
+    by the correcting walk instead of the boundary rule) -> (out_qual [N, L] u8, t), or (out_qual, t, tables, deltas)
+    as recalibrate_host's with want_tables."""
     seq, qual = u8(seq).ravel(), u8(qual).ravel()
     N = seq.size // L
     assert seq.size == qual.size == N * L
@@ -439,8 +447,10 @@ def recalibrate_kmer_host(seq, qual, rg, second, L, R, minscore=6, k=23, min_cou
         deltas = np.zeros(2 * R + R * NQ * (1 + 2 * L + 17), np.int64)
     t, st = C.c_int(0), C.c_int(0)
     dev = _dev(device)
-    rc = lib().kbbq_recalibrate_kmer_host(ptr(seq), ptr(qual), ptr(rg), ptr(second), N, L, R, minscore, k, min_count,
-                                          ptr(out), ptr(tables), ptr(deltas), C.byref(t), C.byref(st), dev)
+    rule = KMER_CORRECT if correct else KMER_BOUNDARIES
+    rc = lib().kbbq_recalibrate_kmer_rule_host(ptr(seq), ptr(qual), ptr(rg), ptr(second), N, L, R, minscore, k,
+                                               min_count, rule, ptr(out), ptr(tables), ptr(deltas), C.byref(t),
+                                               C.byref(st), dev)
     _kmer_check(rc, st.value, N, L, k, dev)
     if not want_tables:
         return out, t.value
@@ -611,6 +621,11 @@ class Session:
             self._kmer_full()
         check(rc)
         return t.value, hist
+
+    def kmer_rule(self, rule):
+        """The rule build_chunk_kmer flags by (KMER_BOUNDARIES or KMER_CORRECT), from kmer_begin until the first
+        build_chunk_kmer."""
+        check(lib().kbbq_session_kmer_rule(self.h, int(rule)))
 
     def build_chunk_kmer(self, seq, qual, rg=None, second=None):
         """Pass 1 of the build for a chunk, its errors flagged from the k-mer table."""

@@ -11,7 +11,7 @@ from kbbq import recalibrate as re
 def recalibrate(args):
     re.recalibrate(bam=args.bam, fastq=args.fastq, infer_rg=args.infer_rg,
                    use_oq=args.use_oq, set_oq=args.set_oq, gatkreport=args.gatkreport,
-                   reads=args.reads, kmer_size=args.kmer_size, min_count=args.min_count)
+                   reads=args.reads, kmer_size=args.kmer_size, min_count=args.min_count, kmer_correct=args.correct)
 
 
 def _int_in(lo, hi):
@@ -51,6 +51,8 @@ def main():
     recalibrate_parser.add_argument('--min-count', type=_int_in(0, 2 ** 31 - 1), default=0,
                                     help='Count from which a k-mer of --reads is trusted; 0 (default) takes the first '
                                          'valley of the count histogram.')
+    recalibrate_parser.add_argument('--correct', action='store_true',
+                                    help='with -r: find each error by correcting the read against its trusted k-mers')
     recalibrate_parser.add_argument('-u', '--use-oq', action='store_true', help=oq_help)
     recalibrate_parser.add_argument('-s', '--set-oq', action='store_true',
                                     help='Set the \'OQ\' flag prior to recalibration. Only works when producing BAM output.')
@@ -69,6 +71,8 @@ def main():
         sub.set_defaults(command=_out_of_scope(name))
 
     args = parser.parse_args()
+    if getattr(args, 'correct', False) and args.reads is None:
+        recalibrate_parser.error('--correct needs -r/--reads')
     args.command(args)
 
 

@@ -192,12 +192,13 @@ def recalibrate_fastq(fastq, infer_rg=False, devices=None):
     w.write(''.join(chunks))
 
 
-def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device):
+def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device, correct=False):
     """recalibrate_reads through a streaming session, for files of any size (DESIGN.md §10, "Streaming"): two passes
     over every batch fill a sieved k-mer table that only holds the k-mers seen at least twice (A: sieve, B: count),
     the threshold is taken from its histogram -- the exact one --, a third pass flags and builds, the model runs once
     and a fourth pass applies and prints, as _recalibrate_fastq_streamed does.  Host memory holds two batches (plus
-    the index of the file); the output is the single-batch path's, byte for byte."""
+    the index of the file); the output is the single-batch path's, byte for byte.  correct: the third pass flags by
+    the correcting walk."""
     if reads.L < 0:
         raise ValueError("%s: reads of unequal length are not supported on this path" % reads.path)
     rg, second, keys = reads.infer(infer_rg)
@@ -208,6 +209,8 @@ def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, devi
 
     with _native.Session(L, R, 6, chunk_reads=batch_reads, resident_reads=0, device=device) as sess:
         sess.kmer_begin(k, N * max(0, L - k + 1))
+        if correct:
+            sess.kmer_rule(_native.KMER_CORRECT)
         for seq in _packed_batches(N, batch_reads, seq_only):
             sess.kmer_sieve(seq)
         for seq in _packed_batches(N, batch_reads, seq_only):
@@ -219,11 +222,13 @@ def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, devi
         _apply_pass(sess, reads, rg, second, batch_reads)
 
 
-def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None):
+def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None, correct=False):
     """Recalibrate the reads of one FASTQ file with the errors found from their own k-mer counts (kbbq.kmer); FASTQ to
     stdout as recalibrate_fastq prints it, on the first of `devices`.  The file is one batch unless KBBQ_BATCH_READS
     is set, the file is larger than STREAM_ABOVE_BYTES, or the batch and its k-mer table do not fit the GPU: then it
-    streams through in batches (_recalibrate_reads_streamed), with the same output."""
+    streams through in batches (_recalibrate_reads_streamed), with the same output.  correct: find the errors by
+    correcting each read against its trusted k-mers (DESIGN.md §10, "The correcting walk") instead of by the
+    boundaries of the uncovered runs."""
     import os
     from . import fastx
     if not 1 <= k <= 31:
@@ -234,20 +239,22 @@ def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None):
     if batch_reads <= 0 and _fastq_size(path) > STREAM_ABOVE_BYTES:
         batch_reads = STREAM_BATCH_READS
     device = _native.device_list(devices)[0]
+    # the option is passed on only when set: without it both drivers are called exactly as before it existed
+    opts = {"correct": True} if correct else {}
     reads = fastx.NativeFastq(path)
     try:
         if reads.N == 0:
             return
         if batch_reads > 0:
-            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device)
+            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device, **opts)
         seq, qual = reads.pack()   # ValueError for reads of unequal length, as on the -f path
         rg, second, keys = reads.infer(infer_rg)
         L, R = reads.L, max(1, len(keys))
         try:
-            out, _ = _native.recalibrate_kmer_host(seq, qual, rg, second, L, R, 6, k, min_count, device=device)
+            out, _ = _native.recalibrate_kmer_host(seq, qual, rg, second, L, R, 6, k, min_count, device=device, **opts)
         except _native.DoesNotFit:
             del seq, qual
-            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, STREAM_BATCH_READS, device)
+            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, STREAM_BATCH_READS, device, **opts)
         fd = _stdout_fd()
         if fd is not None:
             reads.write(fd, out)
@@ -266,9 +273,10 @@ def recalibrate_bam(bam, use_oq=False, set_oq=False):
 
 
 def recalibrate(bam, fastq, infer_rg=False, use_oq=False, set_oq=False, gatkreport=None, devices=None, reads=None,
-                kmer_size=23, min_count=0):
+                kmer_size=23, min_count=0, kmer_correct=False):
     """reference: kbbq/recalibrate.py:166-174 (devices: see recalibrate_fastq).  reads: one FASTQ file whose errors
-    come from its own k-mer counts (recalibrate_reads) instead of a corrected twin."""
+    come from its own k-mer counts (recalibrate_reads) instead of a corrected twin; kmer_correct: found by the
+    correcting walk."""
     if gatkreport is not None:
         raise NotImplementedError('GATKreport reading / creation is not yet supported.')
     elif bam is not None:
@@ -276,6 +284,7 @@ def recalibrate(bam, fastq, infer_rg=False, use_oq=False, set_oq=False, gatkrepo
     elif fastq is not None:
         recalibrate_fastq(fastq, infer_rg=infer_rg, devices=devices)
     elif reads is not None:
-        recalibrate_reads(reads, infer_rg=infer_rg, k=kmer_size, min_count=min_count, devices=devices)
+        opts = {"correct": True} if kmer_correct else {}   # as in recalibrate_reads: passed on only when set
+        recalibrate_reads(reads, infer_rg=infer_rg, k=kmer_size, min_count=min_count, devices=devices, **opts)
     else:
         raise ValueError("A BAM or FASTQ file should be provided for recalibration.")

@@ -16,7 +16,8 @@ sum c h[c] = W), then the whole streamed session by wall clock.  The big leg's r
 of 1 M reads on all host cores (blocks_reads: genome_reads' sampling, one genome, block b drawn from the seed and b);
 the run holds seq, qual and the true error mask in host memory, 3 bytes per base (22 GB at 48 M x 150 bp).  The card's
 name, power limit and clock come from nvidia-smi in the same run; each leg's results are written to --out as soon as
-it ends.
+it ends.  --correct runs both legs with the correcting walk (kbbq_kmer_correct, DESIGN.md §10) in place of the
+boundary rule: the device pass, the single-batch call and the session.
 """
 import argparse
 import ctypes as C
@@ -86,7 +87,7 @@ def write(res, path):
     return line
 
 
-def session_run(seq, qual, second, L, k, batch):
+def session_run(seq, qual, second, L, k, batch, correct=False):
     """The streamed path from memory (kbbq_session_kmer_*) -> (out, t, hist, (filter_words, capacity), seconds)"""
     from kbbq import _native
     n = seq.shape[0]
@@ -96,6 +97,8 @@ def session_run(seq, qual, second, L, k, batch):
     t0 = time.perf_counter()
     with _native.Session(L, 1, 6, chunk_reads=batch, resident_reads=0) as s:
         s.kmer_begin(k, n * max(0, L - k + 1))
+        if correct:
+            s.kmer_rule(_native.KMER_CORRECT)
         sizes = s.kmer_sizes()
         s.flush()
         secs["begin"] = time.perf_counter() - t0
@@ -128,11 +131,11 @@ def session_run(seq, qual, second, L, k, batch):
 class Passes:
     """Sieve / count-present / histogram / flag on torch buffers, chunk by chunk, timed with CUDA events."""
 
-    def __init__(self, L, k, windows):
+    def __init__(self, L, k, windows, correct=False):
         import torch
         from kbbq import _native
         self.torch, self.native, self.lib = torch, _native, _native.lib()
-        self.L, self.k = L, k
+        self.L, self.k, self.correct = L, k, correct
         free, _ = torch.cuda.mem_get_info()
         self.F, self.cap = _native.kmer_stream_plan(windows, int(0.8 * free))
         self.filter = torch.zeros(self.F, dtype=torch.int64, device="cuda")
@@ -141,7 +144,8 @@ class Passes:
         self.windows = torch.zeros(1, dtype=torch.int64, device="cuda")
         self.hist = torch.zeros(256, dtype=torch.int64, device="cuda")
         self.stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        self.ms = {"clear": 0.0, "sieve": 0.0, "count_present": 0.0, "histogram": 0.0, "flag": 0.0}
+        self.ms = {"clear": 0.0, "sieve": 0.0, "count_present": 0.0, "histogram": 0.0,
+                   "correct" if correct else "flag": 0.0}
         self.timed("clear", lambda: self.lib.kbbq_kmer_clear(self.p(self.table), self.cap, self.stream))
 
     def p(self, t):
@@ -171,9 +175,10 @@ class Passes:
         return self.hist.cpu().numpy().astype(np.uint64)
 
     def flag(self, d_seq, n, t, bits):
-        self.timed("flag", lambda: self.lib.kbbq_kmer_flag_sieved(self.p(d_seq), n, self.L, self.k, self.p(self.table),
-                                                                  self.cap, t, self.p(bits), self.p(self.status),
-                                                                  self.stream))
+        fn = self.lib.kbbq_kmer_correct if self.correct else self.lib.kbbq_kmer_flag_sieved
+        self.timed("correct" if self.correct else "flag",
+                   lambda: fn(self.p(d_seq), n, self.L, self.k, self.p(self.table), self.cap, t, self.p(bits),
+                              self.p(self.status), self.stream))
 
     def table_stats(self):
         """-> (keys in the table, of which count 1), a slice of slots at a time"""
@@ -187,13 +192,13 @@ class Passes:
         return keys, ones
 
 
-def run_passes(seq, L, k, chunk, err=None):
+def run_passes(seq, L, k, chunk, err=None, correct=False):
     """The four passes over seq in chunks of `chunk` reads -> dict of results (and flags checked against err)."""
     import torch
     from kbbq.kmer import bits_to_mask
     n = seq.shape[0]
     W = n * max(0, L - k + 1)
-    ps = Passes(L, k, W)
+    ps = Passes(L, k, W, correct)
     spans = [(lo, min(chunk, n - lo)) for lo in range(0, n, chunk)]
     for step in (ps.sieve, ps.count):
         for lo, m in spans:
@@ -258,6 +263,7 @@ def main():
     ap.add_argument("--k", type=int, default=23)
     ap.add_argument("--batch", type=int, default=8_000_000)
     ap.add_argument("--seed", type=int, default=1)
+    ap.add_argument("--correct", action="store_true", help="the correcting walk in place of the boundary rule")
     ap.add_argument("--out", help="also write the JSON line to this file")
     args = ap.parse_args()
     import torch
@@ -266,18 +272,20 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("needs a CUDA device")
     L, k = args.L, args.k
-    res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), L=L, k=k, batch=args.batch)
+    res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), L=L, k=k, batch=args.batch,
+               rule="correct" if args.correct else "boundaries")
+    opt = {"correct": True} if args.correct else {}
 
     t0 = time.perf_counter()
     seq, qual, err, second = synth.genome_reads(args.seed, args.genome, args.reads, L, 0.01)
     leg = dict(reads=args.reads, genome=args.genome, generate_s=round(time.perf_counter() - t0, 1))
     leg["exact_capacity"], leg["exact_keys"] = exact_keys(seq, L, k)
-    leg.update(run_passes(seq, L, k, args.reads, err))
+    leg.update(run_passes(seq, L, k, args.reads, err, args.correct))
     t0 = time.perf_counter()
-    out_single, t_single = _native.recalibrate_kmer_host(seq, qual, None, second, L, 1, 6, k)
+    out_single, t_single = _native.recalibrate_kmer_host(seq, qual, None, second, L, 1, 6, k, **opt)
     leg["single_batch_s"] = round(time.perf_counter() - t0, 3)
     _native.lib().kbbq_host_release(_native.DEVICE)
-    out_stream, t_stream, _, sizes, secs = session_run(seq, qual, second, L, k, args.batch)
+    out_stream, t_stream, _, sizes, secs = session_run(seq, qual, second, L, k, args.batch, args.correct)
     leg.update(streamed_s=secs, streamed_sizes=sizes, same_threshold=t_single == t_stream,
                same_qualities=bool(np.array_equal(out_single, out_stream)))
     res["leg_10m"] = leg
@@ -290,12 +298,12 @@ def main():
         leg = dict(reads=args.big_reads, genome=args.big_genome, generate_s=round(time.perf_counter() - t0, 1),
                    exact_rule_bytes=_native.kmer_table_bytes(args.big_reads, L, k)[1])
         try:
-            _native.recalibrate_kmer_host(seq, qual, None, second, L, 1, 6, k)
+            _native.recalibrate_kmer_host(seq, qual, None, second, L, 1, 6, k, **opt)
             leg["single_batch"] = "ran"
         except _native.DoesNotFit as e:
             leg["single_batch"] = "refused: %s" % e
-        leg.update(run_passes(seq, L, k, args.batch, err))
-        out, t, hist, sizes, secs = session_run(seq, qual, second, L, k, args.batch)
+        leg.update(run_passes(seq, L, k, args.batch, err, args.correct))
+        out, t, hist, sizes, secs = session_run(seq, qual, second, L, k, args.batch, args.correct)
         leg.update(streamed_s=secs, streamed_sizes=sizes, streamed_min_count=t,
                    streamed_sum_c_hist=int(sum(c * int(hist[c]) for c in range(1, 256))),
                    streamed_hist_255=int(hist[255]), windows=args.big_reads * max(0, L - k + 1), changed_qualities=int((out != qual).sum()))
