@@ -594,6 +594,46 @@ int kbbq_recalibrate_kmer_rule_host(const uint8_t *seq, const uint8_t *qual, con
                                     int *status_out, int device);
 int kbbq_session_kmer_rule(kbbq_session *s, int rule);
 
+/*
+ * Several GPUs (DESIGN.md §10, "Several GPUs"): the sieved table split by key into n_parts partitions of `capacity`
+ * slots each, partition p on any device.  With h = splitmix64(key), the key belongs to partition
+ * owner = ((h >> 32) * n_parts) >> 32 and its home slot there is h & (capacity - 1), as in a single table.  Each
+ * partition runs passes A and B over EVERY chunk and takes only the windows it owns, W included; each sieved
+ * histogram (kbbq_kmer_histogram_sieved of the partition) is then that of its keys, and their sum is the exact
+ * histogram of the input.  So the threshold, the flags and everything built from them equal the single table's for
+ * any number of partitions and any placement.
+ *   kbbq_kmer_sieve_part / kbbq_kmer_count_present_part  pass A / B of partition `part`: kbbq_kmer_sieve /
+ *                            _count_present restricted to the windows that partition owns
+ *   kbbq_kmer_flag_parts / kbbq_kmer_correct_parts  the map of kbbq_kmer_flag_sieved / kbbq_kmer_correct with every
+ *                            lookup in its owner's table (tables[p], read from the device of `stream` -- peer
+ *                            memory, NVLink, for the tables of other devices).  min_count == 1 makes no lookup.
+ * n_parts == 1 (part 0) is the single-table call.  KBBQ_E_ARG for n_parts outside 1..16, part outside 0..n_parts - 1,
+ * a NULL table, or n_parts > 1 with capacity > 2^32.  Device pointers, asynchronous on `stream`, no allocation.
+ *
+ * kbbq_session_kmer_begin_parts: kbbq_session_kmer_begin with partition p of the table on devices[p] (devices[0] the
+ * session's device, KBBQ_E_ARG otherwise; a device may be listed more than once); kbbq_session_kmer_begin is its
+ * n_parts = 1 case.  Each chunk of kmer_sieve / kmer_count goes up into the session's device once and is copied
+ * (cudaMemcpyPeerAsync) to each other partition; kmer_threshold sums the partitions' histograms; build_chunk_kmer
+ * flags on the session's device, reading the other partitions' tables as peer memory.  filter_words / capacity 0:
+ * every partition gets the same sizes, kbbq_kmer_stream_plan of ceil(windows / n_parts) windows within the smallest
+ * partition budget -- 90 % of its device's free memory shared by the partitions on that device, less two chunks for
+ * the copies of partitions p >= 1 -- and at most 2^32 slots (kbbq_session_kmer_sizes reports them).  KBBQ_E_PEER,
+ * having allocated nothing, when the session's device cannot read another partition's device (or with
+ * KBBQ_MULTI_NO_P2P=1 and n_parts > 1).  A table that fills in any partition is reported as for one table.
+ */
+int kbbq_kmer_sieve_part(const uint8_t *seq_dev, int64_t N, int L, int k, int part, int n_parts, void *filter_dev,
+                         uint64_t filter_words, void *table_dev, uint64_t capacity, int *status_dev, void *stream);
+int kbbq_kmer_count_present_part(const uint8_t *seq_dev, int64_t N, int L, int k, int part, int n_parts,
+                                 void *table_dev, uint64_t capacity, uint64_t *windows_dev, int *status_dev,
+                                 void *stream);
+int kbbq_kmer_flag_parts(const uint8_t *seq_dev, int64_t N, int L, int k, const void *const *tables_dev, int n_parts,
+                         uint64_t capacity, int min_count, uint32_t *bits_dev, int *status_dev, void *stream);
+int kbbq_kmer_correct_parts(const uint8_t *seq_dev, int64_t N, int L, int k, const void *const *tables_dev,
+                            int n_parts, uint64_t capacity, int min_count, uint32_t *bits_dev, int *status_dev,
+                            void *stream);
+int kbbq_session_kmer_begin_parts(kbbq_session *s, int k, int64_t windows, uint64_t filter_words, uint64_t capacity,
+                                  const int *devices, int n_parts);
+
 /* Number of kernel launches this library has issued since load (bench.py's gpu_launches). */
 int64_t kbbq_launch_count(void);
 

@@ -21,7 +21,9 @@
 // `kbbq recalibrate -r` streams through the same session: kbbq_session_kmer_sieve x n and kbbq_session_kmer_count x n
 // fill a sieved k-mer table (kmer.cuh) in the same slots and streams, kbbq_session_kmer_threshold takes the exact
 // histogram, and kbbq_session_build_chunk_kmer is pass 1 with the map flagged on the device in place of the corrected
-// reads -- by the boundary rule, or by the correcting walk after kbbq_session_kmer_rule (`-r --correct`).
+// reads -- by the boundary rule, or by the correcting walk after kbbq_session_kmer_rule (`-r --correct`).  After
+// kbbq_session_kmer_begin_parts the table is split by key across devices: every chunk is copied from the session's
+// device to each other partition for its passes, and the map reads the other partitions' tables as peer memory.
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -121,6 +123,29 @@ struct OutSlot {
     cudaEvent_t applied = nullptr, drained = nullptr;
 };
 
+// Partition p >= 1 of a k-mer table split by key across devices (kbbq_session_kmer_begin_parts): on `device`, its
+// copies of the two staging slots, filter, table, window count, histogram and status word.  Partition 0 is the
+// session's own k-mer buffers.
+struct KmerPartition {
+    int device = 0;
+    cudaStream_t up = nullptr, comp = nullptr;       // the peer copy of a chunk; the passes over it
+    cudaEvent_t copied[2] = {}, consumed[2] = {};    // per chunk buffer
+    uint8_t *chunk[2] = {};
+    void *filter = nullptr, *base = nullptr;
+    ulonglong2 *table = nullptr;
+    uint64_t *windows = nullptr, *hist = nullptr;
+    int *status = nullptr;
+
+    void release() {   // waits for its streams; leaves `device` current
+        cudaSetDevice(device);
+        for (auto s : {up, comp}) if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
+        for (auto e : {copied[0], copied[1], consumed[0], consumed[1]}) if (e) cudaEventDestroy(e);
+        if (filter) cudaFree(filter);
+        if (base) cudaFree(base);
+        *this = KmerPartition();
+    }
+};
+
 }  // namespace
 
 struct kbbq_session {
@@ -158,9 +183,12 @@ struct kbbq_session {
     // the rule build_chunk_kmer flags by (kbbq_session_kmer_rule), and whether it has flagged a chunk yet
     int kmer_rule = KBBQ_KMER_BOUNDARIES;
     bool kmer_built = false;
+    // partitions 1.. of a table split across devices (kbbq_session_kmer_begin_parts); empty: one table
+    std::vector<KmerPartition> kparts;
     std::mutex mu;
 
     ~kbbq_session() {
+        for (auto &q : kparts) q.release();
         cudaSetDevice(device);
         for (auto s : {s_up, s_comp, s_down}) if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
         for (auto &u : up) { if (u.uploaded) cudaEventDestroy(u.uploaded); if (u.consumed) cudaEventDestroy(u.consumed); }
@@ -303,6 +331,9 @@ int session_create(int device, int L, int R, int minscore, int64_t C, int64_t M,
 
 // Free the k-mer buffers once the compute stream is done with them.
 int kmer_release(kbbq_session *S) {
+    for (auto &q : S->kparts) q.release();
+    S->kparts.clear();
+    KBBQ_CUDA(cudaSetDevice(S->device));
     if (S->kmer_filter || S->kmer_base) KBBQ_CUDA(cudaStreamSynchronize(S->s_comp));
     if (S->kmer_filter) KBBQ_CUDA(cudaFree(S->kmer_filter));
     if (S->kmer_base) KBBQ_CUDA(cudaFree(S->kmer_base));
@@ -416,13 +447,17 @@ int build_chunk_finish(kbbq_session *S, int64_t k, const uint8_t *seq, const uin
     }
     KBBQ_CUDA(cudaEventRecord(u.uploaded, S->s_up));
     KBBQ_CUDA(cudaStreamWaitEvent(S->s_comp, u.uploaded, 0));
-    if (kmer) {
+    if (kmer) {   // every lookup in its owner's table; the tables of other devices are peer memory (NVLink)
+        const void *tables[MAX_DEVICES];
+        const int n_parts = 1 + (int)S->kparts.size();
+        tables[0] = S->kmer_table;
+        for (int q = 1; q < n_parts; ++q) tables[q] = S->kparts[(size_t)q - 1].table;
         if (S->kmer_rule == KBBQ_KMER_CORRECT)
-            KBBQ_TRY(kbbq_kmer_correct(p.d_seq, n, L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_t, S->kmer_bits,
-                                       S->d_status, S->s_comp));
+            KBBQ_TRY(kbbq_kmer_correct_parts(p.d_seq, n, L, S->kmer_k, tables, n_parts, S->kmer_cap, S->kmer_t,
+                                             S->kmer_bits, S->d_status, S->s_comp));
         else
-            KBBQ_TRY(kbbq_kmer_flag_sieved(p.d_seq, n, L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_t,
-                                           S->kmer_bits, S->d_status, S->s_comp));
+            KBBQ_TRY(kbbq_kmer_flag_parts(p.d_seq, n, L, S->kmer_k, tables, n_parts, S->kmer_cap, S->kmer_t,
+                                          S->kmer_bits, S->d_status, S->s_comp));
         KBBQ_TRY(kbbq_expand_mismatch_bits(p.d_seq, S->kmer_bits, (int64_t)nb, u.corr, S->s_comp));
     } else if (S->pack == PACK_NIBBLES) KBBQ_TRY(kbbq_expand_nibbles((const uint8_t *)u.bits, (int64_t)nb, p.d_seq, u.corr, S->s_comp));
     else if (S->pack == PACK_BITS) KBBQ_TRY(kbbq_expand_mismatch_bits(p.d_seq, u.bits, (int64_t)nb, u.corr, S->s_comp));
@@ -464,14 +499,48 @@ int build_chunk_async(kbbq_session *S, const uint8_t *seq, const uint8_t *qual, 
 
 // ---- kbbq recalibrate -r through a streaming session (kbbq_session_kmer_*, DESIGN.md §10 "Streaming") ----
 
-int kmer_begin(kbbq_session *S, int k, int64_t windows, uint64_t F, uint64_t cap) {
+// Partition p of the table on devices[p] (devices[0] = the session's device; n = 1: one table, as before there were
+// several).  Nothing is allocated unless every check passes.
+int kmer_begin(kbbq_session *S, int k, int64_t windows, uint64_t F, uint64_t cap, const int *devices, int n) {
     auto pow2 = [](uint64_t x) { return x >= 1 && (x & (x - 1)) == 0; };
     if (k < 1 || k > 31 || windows < 0 || S->kmer_stage != KMER_NONE || S->M > 0) return KBBQ_E_ARG;   // streaming only
     if ((F == 0) != (cap == 0) || (F && (!pow2(F) || !pow2(cap)))) return KBBQ_E_ARG;
+    if (!devices || n < 1 || n > MAX_DEVICES || devices[0] != S->device || (n > 1 && cap > (1ull << 32)))
+        return KBBQ_E_ARG;
+    int ndev = 0;
+    KBBQ_CUDA(cudaGetDeviceCount(&ndev));
+    for (int p = 0; p < n; ++p)
+        if (devices[p] < 0 || devices[p] >= ndev) return KBBQ_E_ARG;
+    // the session's device reads every partition's table when it flags (the same device listed twice trivially can)
+    if (n > 1 && !env_flag_off("KBBQ_MULTI_NO_P2P")) return KBBQ_E_PEER;   // test hook: as if no peer were reachable
+    for (int p = 1; p < n; ++p) {
+        if (devices[p] == S->device) continue;
+        int ok = 0;
+        if (cudaDeviceCanAccessPeer(&ok, S->device, devices[p]) != cudaSuccess || !ok) return KBBQ_E_PEER;
+    }
+    for (int p = 1; p < n; ++p) {
+        if (devices[p] == S->device) continue;
+        const cudaError_t e = cudaDeviceEnablePeerAccess(devices[p], 0);
+        if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+        else if (e != cudaSuccess) { cudaGetLastError(); return KBBQ_E_PEER; }
+    }
+    const size_t chunk_bytes = (size_t)S->C * S->L + 16;
     if (!F) {
-        size_t free_b = 0, total_b = 0;
-        KBBQ_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        KBBQ_TRY(kbbq_kmer_stream_plan((uint64_t)windows, (uint64_t)(0.9 * (double)free_b), &F, &cap));
+        // each partition's budget: 90 % of its device's free memory shared by the partitions there, less the two chunk
+        // copies of a partition p >= 1; every partition gets the sizes of the smallest budget
+        double budget = 0;
+        for (int p = 0; p < n; ++p) {
+            size_t free_b = 0, total_b = 0;
+            KBBQ_CUDA(cudaSetDevice(devices[p]));
+            KBBQ_CUDA(cudaMemGetInfo(&free_b, &total_b));
+            const int hosts = (int)std::count(devices, devices + n, devices[p]);
+            const double b = 0.9 * (double)free_b / hosts - (p ? 2.0 * (double)chunk_bytes : 0.0);
+            budget = p ? std::min(budget, b) : b;
+        }
+        KBBQ_CUDA(cudaSetDevice(S->device));
+        if (budget < 0) return KBBQ_E_UNSUPPORTED;
+        KBBQ_TRY(kbbq_kmer_stream_plan(((uint64_t)windows + n - 1) / n, (uint64_t)budget, &F, &cap));
+        if (n > 1) cap = std::min<uint64_t>(cap, 1ull << 32);
     }
     const size_t bits_words = ((size_t)S->C * S->L + 31) / 32 + 4;
     Carver c(nullptr);
@@ -502,55 +571,147 @@ int kmer_begin(kbbq_session *S, int k, int64_t windows, uint64_t F, uint64_t cap
     KBBQ_CUDA(cudaMemsetAsync(S->kmer_filter, 0, F * 8, S->s_comp));
     KBBQ_CUDA(cudaMemsetAsync(S->kmer_windows, 0, 8, S->s_comp));
     KBBQ_TRY(kbbq_kmer_clear(S->kmer_table, cap, S->s_comp));
-    S->kmer_stage = KMER_SIEVE;
+    S->kmer_stage = KMER_SIEVE;   // from here on kmer_release (reset) frees whatever has been allocated
+    for (int p = 1; p < n; ++p) {
+        S->kparts.emplace_back();
+        KmerPartition &q = S->kparts.back();
+        q.device = devices[p];
+        KBBQ_CUDA(cudaSetDevice(q.device));
+        KBBQ_CUDA(cudaStreamCreateWithFlags(&q.up, cudaStreamNonBlocking));
+        KBBQ_CUDA(cudaStreamCreateWithFlags(&q.comp, cudaStreamNonBlocking));
+        for (auto e : {&q.copied[0], &q.copied[1], &q.consumed[0], &q.consumed[1]})
+            KBBQ_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+        Carver m(nullptr);
+        m.take<uint8_t>(chunk_bytes);
+        m.take<uint8_t>(chunk_bytes);
+        m.take<ulonglong2>(cap);
+        m.take<uint64_t>(1);
+        m.take<uint64_t>(256);
+        m.take<int>(64);
+        KBBQ_TRY(alloc(&q.filter, F * 8));
+        KBBQ_TRY(alloc(&q.base, m.off));
+        Carver e(q.base);
+        q.chunk[0] = e.take<uint8_t>(chunk_bytes);
+        q.chunk[1] = e.take<uint8_t>(chunk_bytes);
+        q.table = e.take<ulonglong2>(cap);
+        q.windows = e.take<uint64_t>(1);
+        q.hist = e.take<uint64_t>(256);
+        q.status = e.take<int>(64);
+        KBBQ_CUDA(cudaMemsetAsync(q.filter, 0, F * 8, q.comp));
+        KBBQ_CUDA(cudaMemsetAsync(q.windows, 0, 8, q.comp));
+        KBBQ_CUDA(cudaMemsetAsync(q.status, 0, sizeof(int), q.comp));
+        KBBQ_TRY(kbbq_kmer_clear(q.table, cap, q.comp));
+    }
+    KBBQ_CUDA(cudaSetDevice(S->device));
+    return KBBQ_OK;
+}
+
+// Whether partition p >= 1 found its table full (its status word; waits for its passes), and the host-side flag that
+// makes kbbq_session_sync report it as the session's own status word reports partition 0.
+int kmer_parts_full(kbbq_session *S, bool *full) {
+    *full = false;
+    for (auto &q : S->kparts) {
+        int st = 0;
+        KBBQ_CUDA(cudaSetDevice(q.device));
+        KBBQ_CUDA(cudaMemcpyAsync(&st, q.status, sizeof(int), cudaMemcpyDeviceToHost, q.comp));
+        KBBQ_CUDA(cudaStreamSynchronize(q.comp));
+        if (st & KBBQ_FLAG_KMER_FULL) *full = true;
+    }
+    KBBQ_CUDA(cudaSetDevice(S->device));
+    if (*full) S->host_status |= KBBQ_FLAG_KMER_FULL;
     return KBBQ_OK;
 }
 
 // Pass A (count = false) or B of one chunk: its bytes go up into a staging slot while the previous chunk's kernel runs.
+// Partition 0 runs on the slot in place; every other partition copies the slot into its own chunk buffer first, and
+// the slot is free again (consumed) once every copy is done.
 int kmer_chunk(kbbq_session *S, const uint8_t *seq, int64_t n, bool count, UpSlot **slot) {
     *slot = nullptr;
     const bool in_order = S->kmer_stage == KMER_SIEVE || (count && S->kmer_stage == KMER_COUNT);
     if (!in_order) return KBBQ_E_ARG;
     if (n < 0 || n > S->C || (n > 0 && !seq)) return KBBQ_E_ARG;
-    if (count && S->kmer_stage == KMER_SIEVE) {   // pass A is over: its filter is not needed any more
+    if (count && S->kmer_stage == KMER_SIEVE) {   // pass A is over: its filters are not needed any more
         int st = 0;
+        bool parts_full = false;
         KBBQ_CUDA(cudaMemcpyAsync(&st, S->d_status, sizeof(int), cudaMemcpyDeviceToHost, S->s_comp));
         KBBQ_CUDA(cudaStreamSynchronize(S->s_comp));
+        KBBQ_TRY(kmer_parts_full(S, &parts_full));
         KBBQ_CUDA(cudaFree(S->kmer_filter));
         S->kmer_filter = nullptr;
+        for (auto &q : S->kparts) {
+            KBBQ_CUDA(cudaSetDevice(q.device));
+            KBBQ_CUDA(cudaFree(q.filter));
+            q.filter = nullptr;
+        }
+        KBBQ_CUDA(cudaSetDevice(S->device));
         S->kmer_stage = KMER_COUNT;
         // a table that filled in pass A is reported here, before pass B; one that fills in pass B stops its kernels
         // (kmer.cuh) and is reported by kbbq_session_kmer_threshold
-        if (st & KBBQ_FLAG_KMER_FULL) return KBBQ_E_DATA;
+        if ((st & KBBQ_FLAG_KMER_FULL) || parts_full) return KBBQ_E_DATA;
     }
     if (n == 0) return KBBQ_OK;
-    UpSlot &u = S->up[S->kmer_chunks++ & 1];
+    const int b = (int)(S->kmer_chunks++ & 1);
+    UpSlot &u = S->up[b];
     const size_t nb = (size_t)n * S->L;
+    const int L = S->L, k = S->kmer_k, n_parts = 1 + (int)S->kparts.size();
     KBBQ_CUDA(cudaStreamWaitEvent(S->s_up, u.consumed, 0));
     KBBQ_CUDA(cudaMemcpyAsync(u.seq, seq, nb, cudaMemcpyHostToDevice, S->s_up));
     S->h2d_bytes += (int64_t)nb;
     KBBQ_CUDA(cudaEventRecord(u.uploaded, S->s_up));
     KBBQ_CUDA(cudaStreamWaitEvent(S->s_comp, u.uploaded, 0));
     if (count)
-        KBBQ_TRY(kbbq_kmer_count_present(u.seq, n, S->L, S->kmer_k, S->kmer_table, S->kmer_cap, S->kmer_windows,
-                                         S->d_status, S->s_comp));
+        KBBQ_TRY(kbbq_kmer_count_present_part(u.seq, n, L, k, 0, n_parts, S->kmer_table, S->kmer_cap, S->kmer_windows,
+                                              S->d_status, S->s_comp));
     else
-        KBBQ_TRY(kbbq_kmer_sieve(u.seq, n, S->L, S->kmer_k, S->kmer_filter, S->filter_words, S->kmer_table, S->kmer_cap,
-                                 S->d_status, S->s_comp));
+        KBBQ_TRY(kbbq_kmer_sieve_part(u.seq, n, L, k, 0, n_parts, S->kmer_filter, S->filter_words, S->kmer_table,
+                                      S->kmer_cap, S->d_status, S->s_comp));
+    for (int p = 1; p < n_parts; ++p) {   // a copy even on the session's own device: one GPU runs this path too
+        KmerPartition &q = S->kparts[(size_t)p - 1];
+        KBBQ_CUDA(cudaSetDevice(q.device));
+        KBBQ_CUDA(cudaStreamWaitEvent(q.up, u.uploaded, 0));
+        KBBQ_CUDA(cudaStreamWaitEvent(q.up, q.consumed[b], 0));   // the partition's pass over its previous copy
+        KBBQ_CUDA(cudaMemcpyPeerAsync(q.chunk[b], q.device, u.seq, S->device, nb, q.up));
+        KBBQ_CUDA(cudaEventRecord(q.copied[b], q.up));
+        KBBQ_CUDA(cudaStreamWaitEvent(q.comp, q.copied[b], 0));
+        if (count)
+            KBBQ_TRY(kbbq_kmer_count_present_part(q.chunk[b], n, L, k, p, n_parts, q.table, S->kmer_cap, q.windows,
+                                                  q.status, q.comp));
+        else
+            KBBQ_TRY(kbbq_kmer_sieve_part(q.chunk[b], n, L, k, p, n_parts, q.filter, S->filter_words, q.table,
+                                          S->kmer_cap, q.status, q.comp));
+        KBBQ_CUDA(cudaEventRecord(q.consumed[b], q.comp));
+        KBBQ_CUDA(cudaSetDevice(S->device));
+        KBBQ_CUDA(cudaStreamWaitEvent(S->s_comp, q.copied[b], 0));
+    }
     KBBQ_CUDA(cudaEventRecord(u.consumed, S->s_comp));
     *slot = &u;
     return KBBQ_OK;
 }
 
+// One sieved histogram per partition, summed on the host: the exact histogram of the input.
 int kmer_threshold(kbbq_session *S, int min_count, uint64_t *hist_out, int *t_used) {
     if (S->kmer_stage != KMER_COUNT || min_count < 0) return KBBQ_E_ARG;
-    uint64_t hist[256];
+    std::vector<uint64_t> h(256 * (1 + S->kparts.size()));
     int st = 0;
+    for (size_t p = 1; p <= S->kparts.size(); ++p) {
+        KmerPartition &q = S->kparts[p - 1];
+        KBBQ_CUDA(cudaSetDevice(q.device));
+        KBBQ_TRY(kbbq_kmer_histogram_sieved(q.table, S->kmer_cap, q.windows, q.hist, q.comp));
+        KBBQ_CUDA(cudaMemcpyAsync(&h[256 * p], q.hist, 256 * sizeof(uint64_t), cudaMemcpyDeviceToHost, q.comp));
+    }
+    KBBQ_CUDA(cudaSetDevice(S->device));
     KBBQ_TRY(kbbq_kmer_histogram_sieved(S->kmer_table, S->kmer_cap, S->kmer_windows, S->kmer_hist, S->s_comp));
-    KBBQ_CUDA(cudaMemcpyAsync(hist, S->kmer_hist, sizeof(hist), cudaMemcpyDeviceToHost, S->s_comp));
+    KBBQ_CUDA(cudaMemcpyAsync(h.data(), S->kmer_hist, 256 * sizeof(uint64_t), cudaMemcpyDeviceToHost, S->s_comp));
     KBBQ_CUDA(cudaMemcpyAsync(&st, S->d_status, sizeof(int), cudaMemcpyDeviceToHost, S->s_comp));
     KBBQ_CUDA(cudaStreamSynchronize(S->s_comp));
-    if (st & KBBQ_FLAG_KMER_FULL) return KBBQ_E_DATA;
+    bool parts_full = false;
+    KBBQ_TRY(kmer_parts_full(S, &parts_full));
+    if ((st & KBBQ_FLAG_KMER_FULL) || parts_full) return KBBQ_E_DATA;
+    uint64_t hist[256];
+    for (int c = 0; c < 256; ++c) {
+        hist[c] = 0;
+        for (size_t p = 0; p < h.size() / 256; ++p) hist[c] += h[256 * p + c];
+    }
     S->kmer_t = min_count > 0 ? min_count : kbbq_kmer_min_count(hist);
     S->kmer_stage = KMER_READY;
     if (hist_out) memcpy(hist_out, hist, sizeof(hist));
@@ -806,9 +967,15 @@ int kbbq_session_build_range(kbbq_session *s, const uint8_t *seq, const uint8_t 
 
 int kbbq_session_kmer_begin(kbbq_session *s, int k, int64_t windows, uint64_t filter_words, uint64_t capacity) {
     if (!s) return KBBQ_E_ARG;
+    return kbbq_session_kmer_begin_parts(s, k, windows, filter_words, capacity, &s->device, 1);
+}
+
+int kbbq_session_kmer_begin_parts(kbbq_session *s, int k, int64_t windows, uint64_t filter_words, uint64_t capacity,
+                                  const int *devices, int n_parts) {
+    if (!s) return KBBQ_E_ARG;
     std::lock_guard<std::mutex> lock(s->mu);
     KBBQ_CUDA(cudaSetDevice(s->device));
-    return kmer_begin(s, k, windows, filter_words, capacity);
+    return kmer_begin(s, k, windows, filter_words, capacity, devices, n_parts);
 }
 
 static int session_kmer_chunk(kbbq_session *s, const uint8_t *seq, int64_t n, bool count) {

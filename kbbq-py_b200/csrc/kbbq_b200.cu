@@ -900,3 +900,104 @@ int kbbq_kmer_correct(const uint8_t *seq, int64_t N, int L, int k, const void *t
 }
 
 }  // extern "C"
+
+// ---- a table split by key across partitions (kmer.cuh, DESIGN.md §10 "Several GPUs") ----
+
+// n partitions of `capacity` slots each: for n > 1 the owner bits (the top 32 of the hash) and the slot bits must not
+// overlap
+static bool kmer_parts_ok(int part, int n_parts, uint64_t capacity) {
+    return n_parts >= 1 && n_parts <= KMER_MAX_PARTS && part >= 0 && part < n_parts &&
+           (n_parts == 1 || capacity <= (1ull << 32));
+}
+
+// the peer-readable table set of a lookup; every table as kmer_table_ok wants it
+static bool kmer_parts_set(const void *const *tables, int n_parts, uint64_t capacity, KmerParts *set) {
+    if (!tables || !kmer_parts_ok(0, n_parts, capacity)) return false;
+    *set = KmerParts{};
+    for (int p = 0; p < n_parts; ++p) {
+        if (!kmer_table_ok(tables[p], capacity)) return false;
+        set->t[p] = (const ulonglong2 *)tables[p];
+    }
+    set->mask = capacity - 1;
+    set->n = (unsigned)n_parts;
+    return true;
+}
+
+// a map kernel of one warp per 32 reads, `words` shared-memory words per warp: 4 warps a block while that stays
+// under 48 KB (as kbbq_kmer_flag and kbbq_kmer_correct launch theirs)
+template <class Kernel, class... Args>
+static int kmer_map_launch(Kernel kernel, int64_t N, int words, void *stream, Args... args) {
+    int device, sms, max_smem;
+    int rc = current_device_info(&device, &sms, &max_smem);
+    if (rc) return rc;
+    const int warps = std::max(1, std::min(4, 49152 / (4 * words)));
+    const size_t smem = (size_t)warps * words * 4;
+    if (smem > (size_t)max_smem) return KBBQ_E_ARG;
+    if (smem > 49152) KBBQ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t blocks = (N + 32 * warps - 1) / (32 * warps);
+    kernel<<<(unsigned)blocks, 32 * warps, smem, (cudaStream_t)stream>>>(args...);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+extern "C" {
+
+int kbbq_kmer_sieve_part(const uint8_t *seq, int64_t N, int L, int k, int part, int n_parts, void *filter,
+                         uint64_t filter_words, void *table, uint64_t capacity, int *status, void *stream) {
+    if (!kmer_parts_ok(part, n_parts, capacity)) return KBBQ_E_ARG;
+    if (n_parts == 1) return kbbq_kmer_sieve(seq, N, L, k, filter, filter_words, table, capacity, status, stream);
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !status || !kmer_table_ok(table, capacity) || !filter ||
+        misaligned(filter, 8) || !pow2(filter_words))
+        return KBBQ_E_ARG;
+    if (N == 0 || L < k) return KBBQ_OK;
+    if (!seq) return KBBQ_E_ARG;
+    kmer_sieve_part_kernel<<<(unsigned)((N + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        seq, N, L, k, (unsigned long long *)filter, filter_words - 1, (unsigned long long *)table, capacity - 1, status,
+        (unsigned)part, (unsigned)n_parts);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_count_present_part(const uint8_t *seq, int64_t N, int L, int k, int part, int n_parts, void *table,
+                                 uint64_t capacity, uint64_t *windows, int *status, void *stream) {
+    if (!kmer_parts_ok(part, n_parts, capacity)) return KBBQ_E_ARG;
+    if (n_parts == 1) return kbbq_kmer_count_present(seq, N, L, k, table, capacity, windows, status, stream);
+    if (N < 0 || L < 1 || k < 1 || k > 31 || !status || !windows || misaligned(windows, 8) ||
+        !kmer_table_ok(table, capacity))
+        return KBBQ_E_ARG;
+    if (N == 0 || L < k) return KBBQ_OK;
+    if (!seq) return KBBQ_E_ARG;
+    kmer_count_present_part_kernel<<<(unsigned)((N + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        seq, N, L, k, (unsigned long long *)table, capacity - 1, (unsigned long long *)windows, status, (unsigned)part,
+        (unsigned)n_parts);
+    KBBQ_LAUNCHED();
+    return KBBQ_OK;
+}
+
+int kbbq_kmer_flag_parts(const uint8_t *seq, int64_t N, int L, int k, const void *const *tables, int n_parts,
+                         uint64_t capacity, int min_count, uint32_t *bits, int *status, void *stream) {
+    KmerParts set;
+    if (!kmer_parts_set(tables, n_parts, capacity, &set)) return KBBQ_E_ARG;
+    if (n_parts == 1 || min_count == 1)   // one table, or no lookup at all
+        return kbbq_kmer_flag_sieved(seq, N, L, k, tables[0], capacity, min_count, bits, status, stream);
+    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 1 || !status) return KBBQ_E_ARG;
+    if (N == 0) return KBBQ_OK;
+    if (!seq || !bits) return KBBQ_E_ARG;
+    return kmer_map_launch(kmer_flag_parts_kernel, N, L, stream, seq, (long long)N, L, k, set,
+                           (unsigned long long)min_count, bits, status);
+}
+
+int kbbq_kmer_correct_parts(const uint8_t *seq, int64_t N, int L, int k, const void *const *tables, int n_parts,
+                            uint64_t capacity, int min_count, uint32_t *bits, int *status, void *stream) {
+    KmerParts set;
+    if (!kmer_parts_set(tables, n_parts, capacity, &set)) return KBBQ_E_ARG;
+    if (n_parts == 1 || min_count == 1)   // one table, or nothing to flag
+        return kbbq_kmer_correct(seq, N, L, k, tables[0], capacity, min_count, bits, status, stream);
+    if (N < 0 || L < 1 || k < 1 || k > 31 || min_count < 1 || !status) return KBBQ_E_ARG;
+    if (N == 0) return KBBQ_OK;
+    if (!seq || !bits) return KBBQ_E_ARG;
+    return kmer_map_launch(kmer_correct_parts_kernel, N, kmer_correct_warp_words(L, k), stream, seq, (long long)N, L, k,
+                           set, (unsigned long long)min_count, bits, status);
+}
+
+}  // extern "C"

@@ -25,6 +25,9 @@
 //
 // The correcting walk (kmer_correct_kernel, below; DESIGN.md §10): an opt-in second rule on the same table that finds
 // every error of a cluster and those at read ends by correcting each read against its trusted k-mers.
+//
+// Several GPUs (the _part / _parts kernels; DESIGN.md §10, "Several GPUs"): the sieved table split by key into
+// partitions, each filled by the same two passes restricted to the keys it owns, and looked up in the owner's table.
 #pragma once
 #include "common.cuh"
 
@@ -117,9 +120,9 @@ __global__ void kmer_hist_kernel(const ulonglong2 *table, unsigned long long cap
         if (h[i]) atomicAdd(hist + i, (unsigned long long)h[i]);
 }
 
-__device__ __forceinline__ unsigned long long kmer_lookup(const ulonglong2 *table, unsigned long long mask,
-                                                          unsigned long long key, bool *full) {
-    unsigned long long slot = kmer_mix(key) & mask;
+// count of `key` in a table whose probe for it starts at `slot` (0 when absent)
+__device__ __forceinline__ unsigned long long kmer_probe(const ulonglong2 *table, unsigned long long mask,
+                                                         unsigned long long slot, unsigned long long key, bool *full) {
     for (unsigned long long p = 0; p <= mask; ++p) {
         const ulonglong2 v = __ldg(table + slot);
         if (v.x == key) return v.y;
@@ -130,15 +133,62 @@ __device__ __forceinline__ unsigned long long kmer_lookup(const ulonglong2 *tabl
     return 0;
 }
 
+__device__ __forceinline__ unsigned long long kmer_lookup(const ulonglong2 *table, unsigned long long mask,
+                                                          unsigned long long key, bool *full) {
+    return kmer_probe(table, mask, kmer_mix(key) & mask, key, full);
+}
+
+// ---- a table split by key across partitions (DESIGN.md §10, "Several GPUs") ----
+//
+// With h = kmer_mix(key) and n partitions, partition owner(key) = ((h >> 32) * n) >> 32 holds the key, at the home
+// slot h & (capacity - 1) of its own table.  For n > 1 a partition has at most 2^32 slots, so the owner and the home
+// slot come from disjoint bits of h; n = 1 puts every key in partition 0 and is the single table.  Passes A and B of
+// partition p see every window and skip the ones it does not own before touching memory, so all occurrences of a key
+// meet in its owner's filter word and table: each partition's table, counts and W_p are those of a single table fed
+// only its keys, and the sum of the partitions' sieved histograms is the exact one.  A lookup reads the owner's table.
+constexpr int KMER_MAX_PARTS = 16;
+
+__device__ __forceinline__ unsigned kmer_owner(unsigned long long h, unsigned n) {   // h = kmer_mix(key)
+    return (unsigned)(((h >> 32) * n) >> 32);
+}
+
+// the windows a counting pass takes: all of them (one table), or those partition `part` of `n` owns
+struct KmerAllKeys {
+    __device__ __forceinline__ bool owns(unsigned long long) const { return true; }
+};
+struct KmerOwnedKeys {
+    unsigned part, n;
+    __device__ __forceinline__ bool owns(unsigned long long key) const { return kmer_owner(kmer_mix(key), n) == part; }
+};
+
+// the tables a lookup reads: one table, or the partitions' tables (those of other devices are peer memory, read
+// over NVLink) -- the owner and the home slot from one kmer_mix
+struct KmerTable {
+    const ulonglong2 *table;
+    unsigned long long mask;
+    __device__ __forceinline__ unsigned long long lookup(unsigned long long key, bool *full) const {
+        return kmer_lookup(table, mask, key, full);
+    }
+};
+struct KmerParts {
+    const ulonglong2 *t[KMER_MAX_PARTS];
+    unsigned long long mask;
+    unsigned n;
+    __device__ __forceinline__ unsigned long long lookup(unsigned long long key, bool *full) const {
+        const unsigned long long h = kmer_mix(key);
+        return kmer_probe(t[kmer_owner(h, n)], mask, h & mask, key, full);
+    }
+};
+
 // One thread per read, one warp per 32 consecutive reads.  Each window's count is looked up once; base i is covered
 // when the last solid window that starts at or before i starts at i - k + 1 or later (the running form of "one of the
 // k windows over i is solid").  A base's coverage is final once the window that starts at it has been looked up, so
 // the run rule runs one window behind the lookups.  The 32 reads of a warp are 32 L bits = L whole words of the
 // map, starting at word (first read / 32) * L: the warp assembles them in shared memory and stores whole words.
 // ALL_SOLID: every valid window is solid (t = 1 on a sieved table, where a key seen once may be absent); no lookups.
-template <bool ALL_SOLID>
-__global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
-                                 unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
+template <bool ALL_SOLID, class Tables>
+__device__ __forceinline__ void kmer_flag_reads(const uint8_t *seq, long long N, int L, int k, Tables tables,
+                                                unsigned long long t, uint32_t *bits, int *status) {
     extern __shared__ uint32_t kmer_words[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const long long r0 = ((long long)blockIdx.x * (blockDim.x >> 5) + warp) * 32;
@@ -170,7 +220,7 @@ __global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, 
             roll.push(s[e]);
             if (e < k - 1) continue;
             const int j = e - k + 1;
-            if (roll.valid() && (ALL_SOLID || kmer_lookup(table, mask, roll.key(), &full) >= t)) last = j;
+            if (roll.valid() && (ALL_SOLID || tables.lookup(roll.key(), &full) >= t)) last = j;
             settle(j);
         }
         for (int i = L - k + 1; i < L; ++i) settle(i);
@@ -182,6 +232,20 @@ __global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, 
     const int nwords = (int)((nreads * L + 31) / 32);
     uint32_t *out = bits + (r0 / 32) * L;
     for (int w = lane; w < nwords; w += 32) out[w] = wb[w];
+}
+
+template <bool ALL_SOLID>
+__global__ void kmer_flag_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
+                                 unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
+    kmer_flag_reads<ALL_SOLID>(seq, N, L, k, KmerTable{table, mask}, t, bits, status);
+}
+
+// the boundary rule on a table split across partitions (t >= 2; t = 1 is kmer_flag_kernel<true>).  The set goes to
+// the body by reference, so that it stays in parameter space (the owner's pointer is one LDC; a copy would be a local
+// array); the single table goes by value, as the two parameters it was.
+__global__ void kmer_flag_parts_kernel(const uint8_t *seq, long long N, int L, int k, const KmerParts tables,
+                                       unsigned long long t, uint32_t *bits, int *status) {
+    kmer_flag_reads<false, const KmerParts &>(seq, N, L, k, tables, t, bits, status);
 }
 
 // Filter word and bit pattern of a key for the sieve: splitmix64 of the key plus a constant, so independent of the
@@ -202,10 +266,12 @@ __device__ __forceinline__ bool kmer_table_full(const int *status) {
 
 // Pass A.  One thread per read as kmer_count_kernel; per valid window one 64-bit atomicOr on one filter word, and
 // when the old word held the whole pattern, the key is claimed (count 0) or found in the table.  A thread stops once
-// the table is full.
-__global__ void kmer_sieve_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *filter,
-                                  unsigned long long fmask, unsigned long long *table, unsigned long long mask,
-                                  int *status) {
+// the table is full.  Keys: the windows it takes (KmerAllKeys, or those one partition owns).
+template <class Keys>
+__device__ __forceinline__ void kmer_sieve_reads(const uint8_t *seq, long long N, int L, int k,
+                                                 unsigned long long *filter, unsigned long long fmask,
+                                                 unsigned long long *table, unsigned long long mask, int *status,
+                                                 Keys keys) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= N) return;
     const uint8_t *s = seq + r * L;
@@ -214,6 +280,7 @@ __global__ void kmer_sieve_kernel(const uint8_t *seq, long long N, int L, int k,
         roll.push(s[e]);
         if (!roll.valid()) continue;
         const unsigned long long key = roll.key();
+        if (!keys.owns(key)) continue;
         unsigned long long w, pattern;
         kmer_sieve_hash(key, fmask, &w, &pattern);
         if ((atomicOr(filter + w, pattern) & pattern) != pattern) continue;   // first sight (or so it seems)
@@ -240,12 +307,28 @@ __global__ void kmer_sieve_kernel(const uint8_t *seq, long long N, int L, int k,
     }
 }
 
+__global__ void kmer_sieve_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *filter,
+                                  unsigned long long fmask, unsigned long long *table, unsigned long long mask,
+                                  int *status) {
+    kmer_sieve_reads(seq, N, L, k, filter, fmask, table, mask, status, KmerAllKeys{});
+}
+
+// pass A of partition `part` of `n`: only the windows it owns
+__global__ void kmer_sieve_part_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *filter,
+                                       unsigned long long fmask, unsigned long long *table, unsigned long long mask,
+                                       int *status, unsigned part, unsigned n) {
+    kmer_sieve_reads(seq, N, L, k, filter, fmask, table, mask, status, KmerOwnedKeys{part, n});
+}
+
 // Pass B.  One thread per read: a key present in the table gets 1 added, an absent one nothing (its count is <= 1).
 // The valid windows of the batch are added to *windows: a warp sum, one atomic per warp.  A probe that walks the
 // whole table (no empty slot: every absent key would cost `capacity` loads) raises KBBQ_FLAG_KMER_FULL, and a thread
-// stops once the flag is up; W is then incomplete, but the table is reported full anyway.
-__global__ void kmer_count_present_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *table,
-                                          unsigned long long mask, unsigned long long *windows, int *status) {
+// stops once the flag is up; W is then incomplete, but the table is reported full anyway.  Keys: as in pass A; a
+// partition counts only the windows it owns, in W too.
+template <class Keys>
+__device__ __forceinline__ void kmer_count_present_reads(const uint8_t *seq, long long N, int L, int k,
+                                                         unsigned long long *table, unsigned long long mask,
+                                                         unsigned long long *windows, int *status, Keys keys) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     unsigned int valid = 0;
     if (r < N) {
@@ -254,6 +337,7 @@ __global__ void kmer_count_present_kernel(const uint8_t *seq, long long N, int L
         for (int e = 0; e < L; ++e) {
             roll.push(s[e]);
             if (!roll.valid()) continue;
+            if (!keys.owns(roll.key())) continue;
             if (kmer_table_full(status)) break;   // not return: the whole warp takes part in the sum below
             ++valid;
             const unsigned long long key = roll.key();
@@ -277,6 +361,18 @@ __global__ void kmer_count_present_kernel(const uint8_t *seq, long long N, int L
     }
     valid = __reduce_add_sync(0xffffffffu, valid);
     if ((threadIdx.x & 31) == 0 && valid) atomicAdd(windows, (unsigned long long)valid);
+}
+
+__global__ void kmer_count_present_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *table,
+                                          unsigned long long mask, unsigned long long *windows, int *status) {
+    kmer_count_present_reads(seq, N, L, k, table, mask, windows, status, KmerAllKeys{});
+}
+
+// pass B of partition `part` of `n`
+__global__ void kmer_count_present_part_kernel(const uint8_t *seq, long long N, int L, int k, unsigned long long *table,
+                                               unsigned long long mask, unsigned long long *windows, int *status,
+                                               unsigned part, unsigned n) {
+    kmer_count_present_reads(seq, N, L, k, table, mask, windows, status, KmerOwnedKeys{part, n});
 }
 
 // h[c] for c >= 2 from the slots of a sieved table (count >= 255 in bin 255, as kmer_hist_kernel bins), and the sum of
@@ -354,8 +450,9 @@ __host__ __device__ __forceinline__ int kmer_correct_warp_words(int L, int k) {
     return L + (L >= k ? 32 * ((L - k + 1 + 31) >> 5) : 0);
 }
 
-__global__ void kmer_correct_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
-                                    unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
+template <class Tables>
+__device__ __forceinline__ void kmer_correct_reads(const uint8_t *seq, long long N, int L, int k, Tables tables,
+                                                   unsigned long long t, uint32_t *bits, int *status) {
     extern __shared__ uint32_t kmer_words[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const long long r0 = ((long long)blockIdx.x * (blockDim.x >> 5) + warp) * 32;
@@ -373,7 +470,7 @@ __global__ void kmer_correct_kernel(const uint8_t *seq, long long N, int L, int 
         const int shift = 2 * (k - 1);
         bool full = false;
         auto flag = [&](int i) { atomicOr(&wb[(base_bit + i) >> 5], 1u << ((base_bit + i) & 31)); };
-        auto solid = [&](const KmerCode &x) { return kmer_lookup(table, mask, x.key(), &full) >= t; };
+        auto solid = [&](const KmerCode &x) { return tables.lookup(x.key(), &full) >= t; };
         auto was_solid = [&](int j) { return (sol[32 * (j >> 5)] >> (j & 31)) & 1u; };
         auto code_at = [&](int p) {   // window p of the read, all A/C/G/T
             KmerCode x{0, 0};
@@ -389,7 +486,7 @@ __global__ void kmer_correct_kernel(const uint8_t *seq, long long N, int L, int 
             roll.push(s[e]);
             if (e < k - 1) continue;
             const int j = e - k + 1;
-            const bool ok = roll.valid() && kmer_lookup(table, mask, roll.key(), &full) >= t;
+            const bool ok = roll.valid() && tables.lookup(roll.key(), &full) >= t;
             word |= (uint32_t)ok << (j & 31);
             if ((j & 31) == 31 || j == nw - 1) {
                 sol[32 * (j >> 5)] = word;
@@ -493,6 +590,17 @@ __global__ void kmer_correct_kernel(const uint8_t *seq, long long N, int L, int 
     const int nwords = (int)((nreads * L + 31) / 32);
     uint32_t *out = bits + (r0 / 32) * L;
     for (int w = lane; w < nwords; w += 32) out[w] = wb[w];
+}
+
+__global__ void kmer_correct_kernel(const uint8_t *seq, long long N, int L, int k, const ulonglong2 *table,
+                                    unsigned long long mask, unsigned long long t, uint32_t *bits, int *status) {
+    kmer_correct_reads(seq, N, L, k, KmerTable{table, mask}, t, bits, status);
+}
+
+// the correcting walk on a table split across partitions
+__global__ void kmer_correct_parts_kernel(const uint8_t *seq, long long N, int L, int k, const KmerParts tables,
+                                          unsigned long long t, uint32_t *bits, int *status) {
+    kmer_correct_reads<const KmerParts &>(seq, N, L, k, tables, t, bits, status);
 }
 
 }  // namespace kbbq

@@ -18,6 +18,7 @@ FLAG_KMER_FULL = 16
 KMER_BOUNDARIES, KMER_CORRECT = 0, 1   # k-mer error rules (include/kbbq_b200.h)
 APPLY_BASES_CHECKED = 0x10   # kbbq_apply path flag: skip the base check (include/kbbq_b200.h)
 E_DATA = -4
+E_PEER = -11
 E_UNSUPPORTED = -12
 
 _lib = None
@@ -124,11 +125,21 @@ SIGNATURES = {
     "kbbq_kmer_errors_rule_host": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, _vp, C.POINTER(_i), _i]),
     "kbbq_recalibrate_kmer_rule_host": (_i, [_vp] * 4 + [_i64, _i, _i, _i, _i, _i, _i] + [_vp] * 3 + [C.POINTER(_i), C.POINTER(_i), _i]),
     "kbbq_session_kmer_rule": (_i, [_vp, _i]),
+    "kbbq_kmer_sieve_part": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, C.c_uint64, _vp, C.c_uint64, _vp, _vp]),
+    "kbbq_kmer_count_present_part": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, C.c_uint64, _vp, _vp, _vp]),
+    "kbbq_kmer_flag_parts": (_i, [_vp, _i64, _i, _i, _vp, _i, C.c_uint64, _i, _vp, _vp, _vp]),
+    "kbbq_kmer_correct_parts": (_i, [_vp, _i64, _i, _i, _vp, _i, C.c_uint64, _i, _vp, _vp, _vp]),
+    "kbbq_session_kmer_begin_parts": (_i, [_vp, _i, _i64, C.c_uint64, C.c_uint64, _vp, _i]),
 }
 
 
 class KbbqNativeError(RuntimeError):
     """The CUDA library is missing, or a CUDA / argument error came back from it."""
+
+
+class PeerUnreachable(KbbqNativeError):
+    """A k-mer table split across several GPUs: the session's GPU cannot read another partition's GPU (KBBQ_E_PEER).
+    Nothing was allocated; one partition on the session's GPU gives the same result."""
 
 
 class DoesNotFit(ValueError):
@@ -575,14 +586,28 @@ class Session:
 
     # ---- `kbbq recalibrate -r` in chunks: a sieved k-mer table (include/kbbq_b200.h, kbbq_session_kmer_*) ----
 
-    def kmer_begin(self, k, windows, filter_words=0, capacity=0):
+    def kmer_begin(self, k, windows, filter_words=0, capacity=0, devices=None):
         """Allocate and clear the filter and the table for k-mers of length k; 0 sizes them by kbbq_kmer_stream_plan
-        of `windows` (the input's windows) from the free memory.  ValueError when that does not fit."""
+        of `windows` (the input's windows) from the free memory.  ValueError when that does not fit.  devices: a list
+        of GPUs, the first the session's, one partition of the table on each (kbbq_session_kmer_begin_parts; a GPU may
+        be listed more than once); PeerUnreachable when the session's GPU cannot read another one's memory."""
         self.k = int(k)
-        rc = lib().kbbq_session_kmer_begin(self.h, self.k, int(windows), filter_words, capacity)
+        if devices is None:
+            self.kmer_parts = 1
+            rc = lib().kbbq_session_kmer_begin(self.h, self.k, int(windows), filter_words, capacity)
+        else:
+            devs = (C.c_int * len(devices))(*[int(d) for d in devices])
+            self.kmer_parts = len(devices)
+            rc = lib().kbbq_session_kmer_begin_parts(self.h, self.k, int(windows), filter_words, capacity, devs,
+                                                     len(devices))
+            if rc == E_PEER:
+                raise PeerUnreachable("k-mer table over GPUs %s: GPU %d cannot read the memory of the others"
+                                      % (list(devices), self.device))
         if rc == E_UNSUPPORTED:
             what = ("%d filter words and %d slots (%.2f GB)" % (filter_words, capacity, (8 * filter_words + 16 * capacity) / 1e9)
                     if filter_words else "the smallest sieved table for %d windows" % windows)
+            if self.kmer_parts > 1:
+                what += " in each of %d partitions" % self.kmer_parts
             raise ValueError("k-mer table (k = %d): %s do not fit the free memory of GPU %d" % (self.k, what, self.device))
         check(rc)
 
@@ -608,6 +633,10 @@ class Session:
 
     def _kmer_full(self):
         f, cap = self.kmer_sizes()
+        if self.kmer_parts > 1:
+            raise MemoryError("the sieved k-mer table (k = %d) of %d partitions of %d slots (%.2f GB each) is full: "
+                              "more distinct repeated k-mers than a partition holds" % (self.k, self.kmer_parts, cap,
+                                                                                         16 * cap / 1e9))
         raise MemoryError("the sieved k-mer table (k = %d) of %d slots (%.2f GB) is full: more distinct repeated "
                           "k-mers than it holds" % (self.k, cap, 16 * cap / 1e9))
 

@@ -192,13 +192,15 @@ def recalibrate_fastq(fastq, infer_rg=False, devices=None):
     w.write(''.join(chunks))
 
 
-def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device, correct=False):
+def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device, correct=False, devices=None):
     """recalibrate_reads through a streaming session, for files of any size (DESIGN.md §10, "Streaming"): two passes
     over every batch fill a sieved k-mer table that only holds the k-mers seen at least twice (A: sieve, B: count),
     the threshold is taken from its histogram -- the exact one --, a third pass flags and builds, the model runs once
     and a fourth pass applies and prints, as _recalibrate_fastq_streamed does.  Host memory holds two batches (plus
     the index of the file); the output is the single-batch path's, byte for byte.  correct: the third pass flags by
-    the correcting walk."""
+    the correcting walk.  devices: several GPUs, the first `device`, each holding one partition of the table split by
+    key (DESIGN.md §10, "Several GPUs"): the same output with room for n times the k-mers.  When `device` cannot read
+    the others' memory the table stays whole on `device`."""
     if reads.L < 0:
         raise ValueError("%s: reads of unequal length are not supported on this path" % reads.path)
     rg, second, keys = reads.infer(infer_rg)
@@ -208,7 +210,11 @@ def _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, devi
         return reads.pack(lo, m)[0]
 
     with _native.Session(L, R, 6, chunk_reads=batch_reads, resident_reads=0, device=device) as sess:
-        sess.kmer_begin(k, N * max(0, L - k + 1))
+        windows = N * max(0, L - k + 1)
+        try:
+            sess.kmer_begin(k, windows, devices=devices)
+        except _native.PeerUnreachable:
+            sess.kmer_begin(k, windows)
         if correct:
             sess.kmer_rule(_native.KMER_CORRECT)
         for seq in _packed_batches(N, batch_reads, seq_only):
@@ -226,9 +232,9 @@ def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None, cor
     """Recalibrate the reads of one FASTQ file with the errors found from their own k-mer counts (kbbq.kmer); FASTQ to
     stdout as recalibrate_fastq prints it, on the first of `devices`.  The file is one batch unless KBBQ_BATCH_READS
     is set, the file is larger than STREAM_ABOVE_BYTES, or the batch and its k-mer table do not fit the GPU: then it
-    streams through in batches (_recalibrate_reads_streamed), with the same output.  correct: find the errors by
-    correcting each read against its trusted k-mers (DESIGN.md §10, "The correcting walk") instead of by the
-    boundaries of the uncovered runs."""
+    streams through in batches (_recalibrate_reads_streamed), with the same output, and with its k-mer table split
+    across every GPU of `devices`.  correct: find the errors by correcting each read against its trusted k-mers
+    (DESIGN.md §10, "The correcting walk") instead of by the boundaries of the uncovered runs."""
     import os
     from . import fastx
     if not 1 <= k <= 31:
@@ -238,15 +244,17 @@ def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None, cor
     batch_reads = int(os.environ.get("KBBQ_BATCH_READS", "0"))
     if batch_reads <= 0 and _fastq_size(path) > STREAM_ABOVE_BYTES:
         batch_reads = STREAM_BATCH_READS
-    device = _native.device_list(devices)[0]
+    devs = _native.device_list(devices)
+    device = devs[0]
     # the option is passed on only when set: without it both drivers are called exactly as before it existed
     opts = {"correct": True} if correct else {}
+    stream_opts = dict(opts, devices=devs) if len(devs) > 1 else opts
     reads = fastx.NativeFastq(path)
     try:
         if reads.N == 0:
             return
         if batch_reads > 0:
-            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device, **opts)
+            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, batch_reads, device, **stream_opts)
         seq, qual = reads.pack()   # ValueError for reads of unequal length, as on the -f path
         rg, second, keys = reads.infer(infer_rg)
         L, R = reads.L, max(1, len(keys))
@@ -254,7 +262,7 @@ def recalibrate_reads(path, infer_rg=False, k=23, min_count=0, devices=None, cor
             out, _ = _native.recalibrate_kmer_host(seq, qual, rg, second, L, R, 6, k, min_count, device=device, **opts)
         except _native.DoesNotFit:
             del seq, qual
-            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, STREAM_BATCH_READS, device, **opts)
+            return _recalibrate_reads_streamed(reads, infer_rg, k, min_count, STREAM_BATCH_READS, device, **stream_opts)
         fd = _stdout_fd()
         if fd is not None:
             reads.write(fd, out)

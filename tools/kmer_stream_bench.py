@@ -18,6 +18,12 @@ the run holds seq, qual and the true error mask in host memory, 3 bytes per base
 name, power limit and clock come from nvidia-smi in the same run; each leg's results are written to --out as soon as
 it ends.  --correct runs both legs with the correcting walk (kbbq_kmer_correct, DESIGN.md §10) in place of the
 boundary rule: the device pass, the single-batch call and the session.
+
+--devices 0,1,2,3 (lists separated by ';' run in turn, e.g. "0;0,1;0,1,2,3") runs the big leg with the table split
+by key across those GPUs (DESIGN.md §10, "Several GPUs"): per pass, the kernel time on each device (CUDA events on its
+stream) and the wall time; the load of each partition; the bytes copied between devices; the map on the first device
+reading every partition (the correcting walk with --correct); then the streamed session over the same devices, and
+whether its qualities equal the first list's.
 """
 import argparse
 import ctypes as C
@@ -87,16 +93,17 @@ def write(res, path):
     return line
 
 
-def session_run(seq, qual, second, L, k, batch, correct=False):
-    """The streamed path from memory (kbbq_session_kmer_*) -> (out, t, hist, (filter_words, capacity), seconds)"""
+def session_run(seq, qual, second, L, k, batch, correct=False, devices=None):
+    """The streamed path from memory (kbbq_session_kmer_*; devices: the table split across them) -> (out, t, hist,
+    (filter_words, capacity), seconds)"""
     from kbbq import _native
     n = seq.shape[0]
     rg = np.zeros(n, np.uint16)
     spans = [(lo, min(batch, n - lo)) for lo in range(0, n, batch)]
     secs = {}
     t0 = time.perf_counter()
-    with _native.Session(L, 1, 6, chunk_reads=batch, resident_reads=0) as s:
-        s.kmer_begin(k, n * max(0, L - k + 1))
+    with _native.Session(L, 1, 6, chunk_reads=batch, resident_reads=0, device=devices[0] if devices else None) as s:
+        s.kmer_begin(k, n * max(0, L - k + 1), devices=devices)
         if correct:
             s.kmer_rule(_native.KMER_CORRECT)
         sizes = s.kmer_sizes()
@@ -233,6 +240,166 @@ def run_passes(seq, L, k, chunk, err=None, correct=False):
     return res
 
 
+class PartPasses:
+    """Passes A and B of a table split across `devices` (kbbq_kmer_sieve_part / _count_present_part), the sieved
+    histogram of each partition and the map (kbbq_kmer_flag_parts / _correct_parts) on devices[0], on torch buffers.
+    Each partition has its own stream on its device; every chunk goes up to devices[0] and is copied to each other
+    partition, as the session does.  Kernel time per device from CUDA events on its stream; wall time per pass from
+    the host clock around the pass, which ends when every stream is done."""
+
+    def __init__(self, L, k, windows, devices, correct=False):
+        import torch
+        from kbbq import _native
+        self.torch, self.native, self.lib = torch, _native, _native.lib()
+        self.L, self.k, self.correct, self.devices = L, k, correct, devices
+        n = len(devices)
+        budget = None
+        for d in devices:   # as kbbq_session_kmer_begin_parts sizes them
+            free, _ = torch.cuda.mem_get_info(d)
+            b = 0.8 * free / devices.count(d)
+            budget = b if budget is None else min(budget, b)
+        self.F, self.cap = _native.kmer_stream_plan(-(-windows // n), int(budget))
+        self.cap = min(self.cap, 1 << 32) if n > 1 else self.cap
+        self.parts = []
+        for d in devices:
+            with torch.cuda.device(d):
+                self.parts.append(dict(
+                    device=d, stream=torch.cuda.Stream(d),
+                    filter=torch.zeros(self.F, dtype=torch.int64, device=d),
+                    table=torch.empty(2 * self.cap, dtype=torch.int64, device=d),
+                    status=torch.zeros(1, dtype=torch.int32, device=d),
+                    windows=torch.zeros(1, dtype=torch.int64, device=d),
+                    hist=torch.zeros(256, dtype=torch.int64, device=d)))
+        self.kernel_ms = {}   # pass -> per-partition milliseconds
+        self.wall_ms = {}
+        self.peer_bytes = 0
+        self.timed_pass("clear", lambda q, p, d_seq, n_: self.lib.kbbq_kmer_clear(self.p(p["table"]), self.cap,
+                                                                                   self.st(p)), [None])
+
+    def p(self, t):
+        return C.c_void_p(t.data_ptr())
+
+    def st(self, part):
+        return C.c_void_p(part["stream"].cuda_stream)
+
+    def timed_pass(self, name, call, chunks):
+        """call(q, part, d_seq, n) for every chunk (a device tensor of n reads on devices[0], or None) and partition"""
+        torch = self.torch
+        ms = self.kernel_ms.setdefault(name, [0.0] * len(self.parts))
+        t0 = time.perf_counter()
+        for chunk in chunks:
+            d0, n = chunk if chunk is not None else (None, 0)
+            ready = torch.cuda.Event()
+            if d0 is not None:
+                with torch.cuda.device(self.devices[0]):
+                    ready.record(torch.cuda.current_stream(self.devices[0]))
+            for q, part in enumerate(self.parts):
+                with torch.cuda.device(part["device"]), torch.cuda.stream(part["stream"]):
+                    part["stream"].wait_event(ready)
+                    d = d0
+                    if d0 is not None and q > 0:   # a copy even on the same device, as the session makes
+                        d = torch.empty_like(d0, device=part["device"])
+                        d.copy_(d0, non_blocking=True)
+                        self.peer_bytes += d0.numel()
+                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                    e0.record(part["stream"])
+                    self.native.check(call(q, part, d, n))
+                    e1.record(part["stream"])
+                    part.setdefault("events", []).append((e0, e1))
+                    if d is not None:
+                        d.record_stream(part["stream"])
+        for q, part in enumerate(self.parts):
+            part["stream"].synchronize()
+            ms[q] += sum(a.elapsed_time(b) for a, b in part.pop("events", []))
+        self.wall_ms[name] = self.wall_ms.get(name, 0.0) + 1000 * (time.perf_counter() - t0)
+
+    def sieve(self, chunks):
+        n_parts = len(self.parts)
+        self.timed_pass("sieve", lambda q, p, d, n: self.lib.kbbq_kmer_sieve_part(
+            self.p(d), n, self.L, self.k, q, n_parts, self.p(p["filter"]), self.F, self.p(p["table"]), self.cap,
+            self.p(p["status"]), self.st(p)), chunks)
+
+    def count(self, chunks):
+        n_parts = len(self.parts)
+        self.timed_pass("count_present", lambda q, p, d, n: self.lib.kbbq_kmer_count_present_part(
+            self.p(d), n, self.L, self.k, q, n_parts, self.p(p["table"]), self.cap, self.p(p["windows"]),
+            self.p(p["status"]), self.st(p)), chunks)
+
+    def histogram(self):
+        self.timed_pass("histogram", lambda q, p, d, n: self.lib.kbbq_kmer_histogram_sieved(
+            self.p(p["table"]), self.cap, self.p(p["windows"]), self.p(p["hist"]), self.st(p)), [None])
+        return sum(p["hist"].cpu().numpy().astype(np.uint64) for p in self.parts)
+
+    def flag(self, d_seq, n, t, bits):
+        """the map on devices[0] only: one timed call"""
+        torch = self.torch
+        fn = self.lib.kbbq_kmer_correct_parts if self.correct else self.lib.kbbq_kmer_flag_parts
+        tables = (C.c_void_p * len(self.parts))(*[p["table"].data_ptr() for p in self.parts])
+        p0 = self.parts[0]
+        name = "correct" if self.correct else "flag"
+        with torch.cuda.device(p0["device"]):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            t0 = time.perf_counter()
+            e0.record(p0["stream"])
+            self.native.check(fn(self.p(d_seq), n, self.L, self.k, tables, len(self.parts), self.cap, t, self.p(bits),
+                                 self.p(p0["status"]), self.st(p0)))
+            e1.record(p0["stream"])
+            e1.synchronize()
+        self.kernel_ms.setdefault(name, [0.0])[0] += e0.elapsed_time(e1)
+        self.wall_ms[name] = self.wall_ms.get(name, 0.0) + 1000 * (time.perf_counter() - t0)
+
+    def loads(self):
+        """share of occupied slots of each partition, a slice of slots at a time"""
+        out = []
+        for p in self.parts:
+            keys = p["table"].view(-1, 2)[:, 0]
+            out.append(round(sum(int((keys[lo:lo + (1 << 28)] != -1).sum()) for lo in range(0, self.cap, 1 << 28))
+                             / self.cap, 4))
+        return out
+
+
+def run_parts(seq, L, k, chunk, devices, err=None, correct=False):
+    """The passes of a table split across `devices` over seq in chunks of `chunk` reads -> dict of results."""
+    import torch
+    from kbbq.kmer import bits_to_mask
+    n = seq.shape[0]
+    ps = PartPasses(L, k, n * max(0, L - k + 1), devices, correct)
+    spans = [(lo, min(chunk, n - lo)) for lo in range(0, n, chunk)]
+    for step in (ps.sieve, ps.count):
+        for lo, m in spans:   # one chunk on the device at a time, as the session holds it
+            with torch.cuda.device(devices[0]):
+                d = torch.from_numpy(seq[lo:lo + m].ravel()).to(devices[0])
+            step([(d, m)])
+            del d
+    hist = ps.histogram()
+    t = ps.native.kmer_min_count(hist)
+    res = dict(devices=devices, filter_words=ps.F, capacity=ps.cap, table_bytes_each=16 * ps.cap, min_count_used=t,
+               partition_load=ps.loads(), windows_valid=int(sum(int(p["windows"].cpu()[0]) for p in ps.parts)),
+               sum_c_hist=int(sum(c * int(hist[c]) for c in range(1, 256))))
+    tp = flagged = errors = 0
+    with torch.cuda.device(devices[0]):
+        bits = torch.empty((chunk * L + 31) // 32 + 1, dtype=torch.int32, device=devices[0])
+        for lo, m in spans:
+            d = torch.from_numpy(seq[lo:lo + m].ravel()).to(devices[0])
+            ps.flag(d, m, t, bits)
+            if err is not None:
+                got = bits_to_mask(bits.cpu().numpy().view(np.uint32), m, L)
+                e = err[lo:lo + m]
+                tp += int((got & e).sum())
+                flagged += int(got.sum())
+                errors += int(e.sum())
+            del d
+    res["status"] = [int(p["status"].cpu()[0]) for p in ps.parts]
+    res["kernel_ms"] = {name: [round(v, 2) for v in ms] for name, ms in ps.kernel_ms.items()}
+    res["wall_ms"] = {name: round(v, 2) for name, v in ps.wall_ms.items()}
+    res["bytes_between_devices"] = ps.peer_bytes
+    if err is not None:
+        res.update(flagged=flagged, precision=round(tp / max(1, flagged), 5), recall=round(tp / max(1, errors), 4))
+    del ps, bits
+    torch.cuda.empty_cache()
+    return res
+
+
 def exact_keys(seq, L, k):
     """Distinct keys of the exact table (kbbq_kmer_count) of the whole batch."""
     import torch
@@ -264,6 +431,8 @@ def main():
     ap.add_argument("--batch", type=int, default=8_000_000)
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--correct", action="store_true", help="the correcting walk in place of the boundary rule")
+    ap.add_argument("--devices", help="the table split across these GPUs, e.g. 0,1,2,3; lists separated by ';' run in "
+                                      "turn; only the --big-reads leg runs")
     ap.add_argument("--out", help="also write the JSON line to this file")
     args = ap.parse_args()
     import torch
@@ -275,6 +444,8 @@ def main():
     res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), L=L, k=k, batch=args.batch,
                rule="correct" if args.correct else "boundaries")
     opt = {"correct": True} if args.correct else {}
+    if args.devices:
+        return devices_leg(args, res)
 
     t0 = time.perf_counter()
     seq, qual, err, second = synth.genome_reads(args.seed, args.genome, args.reads, L, 0.01)
@@ -308,6 +479,27 @@ def main():
                    streamed_sum_c_hist=int(sum(c * int(hist[c]) for c in range(1, 256))),
                    streamed_hist_255=int(hist[255]), windows=args.big_reads * max(0, L - k + 1), changed_qualities=int((out != qual).sum()))
         res["leg_48m"] = leg
+    print(write(res, args.out))
+
+
+def devices_leg(args, res):
+    """The --big-reads leg with the table split across each device list of --devices: the passes on the device entry
+    points (run_parts), then the streamed session; its qualities against those of the first list's session."""
+    L, k = args.L, args.k
+    t0 = time.perf_counter()
+    seq, qual, err, second = blocks_reads(args.seed + 1, args.big_genome, args.big_reads, L, 0.01)
+    res.update(reads=args.big_reads, genome=args.big_genome, generate_s=round(time.perf_counter() - t0, 1), legs=[])
+    first = None
+    for spec in args.devices.split(";"):
+        devices = [int(x) for x in spec.split(",")]
+        leg = run_parts(seq, L, k, args.batch, devices, err, args.correct)
+        out, t, hist, sizes, secs = session_run(seq, qual, second, L, k, args.batch, args.correct, devices)
+        first = out if first is None else first
+        leg.update(streamed_s=secs, streamed_sizes=sizes, streamed_min_count=t,
+                   same_qualities_as_first=bool(np.array_equal(out, first)))
+        del out
+        res["legs"].append(leg)
+        write(res, args.out)
     print(write(res, args.out))
 
 
