@@ -87,13 +87,17 @@ int kbbq_build(const uint8_t *seq_dev, const uint8_t *qual_dev, const uint8_t *c
  * Marginals + meanq.  rg_* / q_* are the sums of pos_* over cycle (and q), which is what the
  * reference's separate np.add.at calls produce (kbbq/recalibrate.py:112-115); meanq is
  * p_to_q(expected_errs / rg_total) (:111,:120; kbbq/compare_reads.py:262-271).
- * Outputs: q_* int64[R][43], rg_* int64[R], meanq int64[R].
+ * Outputs: q_* int64[R][43], rg_* int64[R], meanq int64[R].  For counts below 2^53, meanq is the exact
+ * floor of -10 log10(expected / total) unless expected / total lies within 2^-96 (relative) of a bucket
+ * boundary 10^(-m/10) (DESIGN.md §4 K3).  KBBQ_E_ARG for R > 65535.
  */
 int kbbq_marginals(const int64_t *pos_errs_dev, const int64_t *pos_total_dev, int L, int R,
                    int64_t *q_errs_dev, int64_t *q_total_dev, int64_t *rg_errs_dev,
                    int64_t *rg_total_dev, int64_t *meanq_dev, void *stream);
 
-/* gatk_delta_q on n independent cells (kbbq/compare_reads.py:235-260). */
+/* gatk_delta_q on n independent cells (kbbq/compare_reads.py:235-260).  An inconsistent cell with
+ * errs >= tot + 2 gets delta = -prior, as in the reference (its log-likelihood is -inf at every
+ * candidate, outside the binomial's support, and np.argmax then gives candidate 0). */
 int kbbq_delta_q(const int64_t *prior_q_dev, const int64_t *numerrs_dev,
                  const int64_t *numtotal_dev, int64_t n, int64_t *delta_dev, void *stream);
 

@@ -1797,7 +1797,7 @@ int kbbq_calibration_counts_host(const uint8_t *qual, const uint8_t *err, const 
 
 int kbbq_marginals_host(const int64_t *pos_errs, const int64_t *pos_total, int L, int R, int64_t *q_errs,
                         int64_t *q_total, int64_t *rg_errs, int64_t *rg_total, int64_t *meanq, int device) {
-    if (L < 1 || R < 1) return KBBQ_E_ARG;
+    if (L < 1 || R < 1 || R > 65535) return KBBQ_E_ARG;
     if (!pos_errs || !pos_total || !q_errs || !q_total || !rg_errs || !rg_total || !meanq) return KBBQ_E_ARG;
     const size_t npos = (size_t)R * NQ * 2 * L * 8, n_q = (size_t)R * NQ * 8, nr = (size_t)R * 8;
     HostCall c(device, false);

@@ -321,7 +321,9 @@ int kbbq_build_segmented(const uint8_t *seq, const uint8_t *qual, const uint8_t 
 
 int kbbq_marginals(const int64_t *pos_errs, const int64_t *pos_total, int L, int R, int64_t *q_errs,
                    int64_t *q_total, int64_t *rg_errs, int64_t *rg_total, int64_t *meanq, void *stream) {
-    if (L < 1 || R < 1 || !pos_errs || !pos_total || !q_errs || !q_total || !rg_errs || !rg_total || !meanq)
+    // R > 65535 would exceed the grid's y limit of marginals_q_kernel
+    if (L < 1 || R < 1 || R > 65535 || !pos_errs || !pos_total || !q_errs || !q_total || !rg_errs || !rg_total ||
+        !meanq)
         return KBBQ_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
     int rc = upload_constants();

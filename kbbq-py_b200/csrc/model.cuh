@@ -125,7 +125,8 @@ __device__ __forceinline__ dd round_to_x87(dd s) {
 // posterior[c] = prior_dist[|c - prior|] + ((errs+1) ln p_c + (tot+1-errs) log1p(-p_c)); the
 // reference adds the fp64 log-likelihood to an x87 long-double prior (kbbq/compare_reads.py:257-258), i.e.
 // the sum is rounded to a 64-bit significand: the exact sum (two_sum) is rounded the same way and the
-// candidates compared on that value.  First maximum wins (np.argmax).
+// candidates compared on that value.  First maximum wins (np.argmax); a +inf log-likelihood (errs >= tot + 2)
+// gives candidate 0.
 // `prior` is an integer quality, or (PRIOR = double: the read-group row of a recalibration report,
 // kbbq/gatk/bqsr.py:293-297) a real one: the reference truncates candidate - prior towards zero
 // before taking the absolute value (kbbq/compare_reads.py:245).  Returns the MAP candidate.
@@ -143,7 +144,12 @@ __device__ __forceinline__ int posterior_q_cell(PRIOR prior, long long errs, lon
         const double b = (mm == 0.0) ? 0.0 : __dmul_rn(mm, c_ln1mp[c]);
         const double ll = __dadd_rn(a, b);
         double h, l;
-        if (isinf(pr) || isinf(ll)) { h = -KBBQ_INF; l = 0.0; }
+        if (isinf(pr) || isinf(ll)) {
+            // ll = +inf only at c = 0 of an inconsistent cell (errs >= tot + 2: (negative) * log1p(-1)).  The
+            // reference's binom.logpmf is -inf at every candidate there (k > n), so np.argmax gives candidate 0.
+            if (ll > 0.0) return c;
+            h = -KBBQ_INF; l = 0.0;
+        }
         else { dd s = round_to_x87(two_sum(pr, ll)); h = s.hi; l = s.lo; }
         if (!have || h > bh || (h == bh && l > bl)) { best = c; bh = h; bl = l; have = true; }
     }

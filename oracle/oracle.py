@@ -136,6 +136,44 @@ def near_tie_cells(n, seed, log10_lo=3.0, log10_hi=11.0):
     return pq, k - 1, m + k - 2
 
 
+def posterior_q_real(prior_q, numerrs, numtotal, gap=False):
+    """gatk_delta_q(prior, ...) + prior for real priors (the read-group table of a recalibration report); with gap, also
+    the relative gap between the two best posteriors of every cell."""
+    prior_q = np.ascontiguousarray(prior_q, dtype=np.float64)
+    numerrs, numtotal = _i64(numerrs), _i64(numtotal)
+    assert prior_q.shape == numerrs.shape == numtotal.shape
+    out = np.zeros(prior_q.shape, np.int64)
+    rel = np.zeros(prior_q.shape, np.float64) if gap else None
+    lib().oracle_posterior_q_real(_p(prior_q), _p(numerrs), _p(numtotal), C.c_int64(prior_q.size), _p(out), _p(rel))
+    return (out, rel) if gap else out
+
+
+def near_tie_counts(priors, seed, log10_lo=3.0, log10_hi=11.0):
+    """near_tie_cells for the given priors (integer or real, in [0, 42]): for every prior, a random adjacent candidate
+    pair (c, c + 1) within 18 of it and a random failure count m, the error count that balances the two posteriors by
+    the same formula.  The candidate distance is |trunc(c - prior)|, as the real-prior posterior takes it.
+    -> (errs, total), int64, shaped like priors."""
+    _, lnp, ln1mp, prior = constants()
+    rng = np.random.default_rng(seed)
+    pq = np.asarray(priors, dtype=np.float64).ravel()
+    errs, tot = np.zeros(pq.size, np.int64), np.zeros(pq.size, np.int64)
+    todo = np.arange(pq.size)
+    while todo.size:
+        p = pq[todo]
+        c = np.clip(np.floor(p).astype(np.int64) + rng.integers(-17, 18, todo.size), 1, 41)
+        m = (10 ** rng.uniform(log10_lo, log10_hi, todo.size)).astype(np.int64)
+        d1, d2 = np.abs(np.trunc(c - p)).astype(np.int64), np.abs(np.trunc(c + 1 - p)).astype(np.int64)
+        ok = (d1 < 19) & (d2 < 19)   # both priors finite
+        k = np.zeros(todo.size, np.int64)
+        k[ok] = np.rint(-((prior[d1[ok]] - prior[d2[ok]]) + m[ok] * (ln1mp[c[ok]] - ln1mp[c[ok] + 1]))
+                        / (lnp[c[ok]] - lnp[c[ok] + 1])).astype(np.int64)
+        ok &= k >= 1
+        errs[todo[ok]], tot[todo[ok]] = k[ok] - 1, m[ok] + k[ok] - 2
+        todo = todo[~ok]
+    shape = np.shape(priors)
+    return errs.reshape(shape), tot.reshape(shape)
+
+
 def get_delta_qs(meanq, rg_errs, rg_total, q_errs, q_total, pos_errs, pos_total, din_errs, din_total):
     R, _, L2 = pos_total.shape
     rgdq = np.zeros(R, np.int64)
