@@ -276,7 +276,9 @@ int kbbq_recalibrate_host_multi(const uint8_t *seq, const uint8_t *qual, const u
  * through a session in chunks: a chunk is tokenised into pinned memory while the previous one crosses PCIe and is
  * added to the tables; after the model step a chunk is applied and copied back while the previous one is formatted
  * straight into the (mapped) output file.  out_fd: where the text goes (stdout's descriptor; a pipe works, a regular
- * file is mapped).  Returns KBBQ_E_UNSUPPORTED, having written nothing, when the files hold different numbers of
+ * file is mapped).  The text lands at out_fd's offset, which then stands right behind it; the bytes before and behind
+ * it stay, and an error leaves the file's bytes, size and offset as they were.  Returns KBBQ_E_UNSUPPORTED, having
+ * written nothing, when the files hold different numbers of
  * reads (the reference's zip() semantics) or do not fit the device at once: the chunked driver of
  * kbbq-py_b200/kbbq/recalibrate.py handles those.  *n_reads / *n_rg / *status_out as the other entry points.
  */

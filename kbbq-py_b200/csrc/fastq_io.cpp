@@ -381,21 +381,20 @@ int kbbq_fastq_open(const char *path, int threads, kbbq_fastq **out) {
     if (!path || !out) return KBBQ_E_ARG;
     kbbq_fastq *f = new kbbq_fastq;
     // gzip by its magic bytes (pysam's FastxFile does not look at the suffix either); a pipe cannot be sniffed
-    // without consuming it, so there the suffix decides
+    // without consuming it, so there the suffix decides.  The path is opened once: a named pipe opened a second time
+    // waits for a writer that may have given up when the first reader closed it.
     bool gz = ends_with(path, ".gz");
-    {
-        const int fd = open(path, O_RDONLY);
-        if (fd < 0) { delete f; return KBBQ_E_IO; }
-        struct stat st;
-        if (fstat(fd, &st) == 0 && S_ISREG(st.st_mode)) {
-            unsigned char magic[2] = {0, 0};
-            gz = pread(fd, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
-        }
-        close(fd);
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) { delete f; return KBBQ_E_IO; }
+    struct stat st;
+    if (fstat(fd, &st) != 0) { close(fd); delete f; return KBBQ_E_IO; }
+    if (S_ISREG(st.st_mode)) {
+        unsigned char magic[2] = {0, 0};
+        gz = pread(fd, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
     }
     if (gz) {
-        gzFile g = gzopen(path, "rb");
-        if (!g) { delete f; return KBBQ_E_IO; }
+        gzFile g = gzdopen(fd, "rb");   // closes fd
+        if (!g) { close(fd); delete f; return KBBQ_E_IO; }
         gzbuffer(g, 1 << 20);
         std::vector<char> &buf = f->owned;
         size_t used = 0;
@@ -411,10 +410,6 @@ int kbbq_fastq_open(const char *path, int threads, kbbq_fastq **out) {
         f->data = buf.data();
         f->len = used;
     } else {
-        const int fd = open(path, O_RDONLY);
-        if (fd < 0) { delete f; return KBBQ_E_IO; }
-        struct stat st;
-        if (fstat(fd, &st) != 0) { close(fd); delete f; return KBBQ_E_IO; }
         void *m = MAP_FAILED;
         if (S_ISREG(st.st_mode) && st.st_size > 0) m = mmap(nullptr, (size_t)st.st_size, PROT_READ, MAP_PRIVATE, fd, 0);
         if (m != MAP_FAILED) {
@@ -697,8 +692,10 @@ int kbbq_fastq_write(int fd, const kbbq_fastq *f, int64_t first, int64_t n, cons
             const long page = sysconf(_SC_PAGESIZE);
             const off_t base = pos0 / page * page;
             const size_t span = (size_t)(pos0 - base) + (size_t)total;
+            // the file only grows: bytes already behind the records stay, as write() leaves them
             void *m = MAP_FAILED;
-            if (ftruncate(rw, pos0 + (off_t)total) == 0) m = mmap(nullptr, span, PROT_READ | PROT_WRITE, MAP_SHARED, rw, base);
+            const off_t end = pos0 + (off_t)total;
+            if (end <= st.st_size || ftruncate(rw, end) == 0) m = mmap(nullptr, span, PROT_READ | PROT_WRITE, MAP_SHARED, rw, base);
             close(rw);
             if (m != MAP_FAILED) {
                 rc = kbbq_fastq_format(f, first, n, out_qual, (char *)m + (pos0 - base), total, threads);

@@ -1180,10 +1180,11 @@ struct OutputMap {   // the output file mapped read-write (fastq_io.cpp: kbbq_fa
                 size0 = st.st_size;
                 base = pos0 / page * page;
                 span = (size_t)(pos0 - base) + (size_t)bytes;
+                // the file only grows: bytes already behind the text stay, as write() leaves them
                 void *m = MAP_FAILED;
-                if (ftruncate(rw, pos0 + (off_t)bytes) == 0) m = mmap(nullptr, span, PROT_READ | PROT_WRITE, MAP_SHARED, rw, base);
+                if (!grew() || ftruncate(rw, pos0 + (off_t)bytes) == 0) m = mmap(nullptr, span, PROT_READ | PROT_WRITE, MAP_SHARED, rw, base);
                 if (m != MAP_FAILED) map = (char *)m;
-                else { if (ftruncate(rw, size0)) {} close(rw); rw = -1; }
+                else { if (grew() && ftruncate(rw, size0)) {} close(rw); rw = -1; }
             }
         }
         // A new file's pages are instantiated one fault at a time, and adding a page to the file is serialised per
@@ -1202,6 +1203,7 @@ struct OutputMap {   // the output file mapped read-write (fastq_io.cpp: kbbq_fa
         }
         return KBBQ_OK;
     }
+    bool grew() const { return pos0 + (off_t)total > size0; }   // the text reaches past the file's old end
     char *at(int64_t off, int64_t bytes) {   // where `bytes` of output starting at `off` are formatted
         if (map) return map + (pos0 - base) + off;
         buf.resize((size_t)bytes);
@@ -1242,8 +1244,9 @@ struct OutputMap {   // the output file mapped read-write (fastq_io.cpp: kbbq_fa
         join_ahead();
         if (map) munmap(map, span);
         // an error before the end: nothing has been printed as far as the caller is concerned (the reference raises
-        // in its first pass, before any output), so the file gets its size back
-        if (rw >= 0 && !finished && ftruncate(rw, size0)) {}
+        // in its first pass, before any output), so the file gets its size back: what the call added goes, the bytes
+        // that were there stay
+        if (rw >= 0 && !finished && grew() && ftruncate(rw, size0)) {}
         if (rw >= 0) close(rw);
     }
 };

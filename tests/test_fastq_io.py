@@ -231,6 +231,25 @@ def test_writer_mapped_equals_plain(tmp_path, monkeypatch, flags):
     buf = np.empty(nbytes.value, np.uint8)
     assert _native.lib().kbbq_fastq_format(f._h, 0, f.N, _native.ptr(out), _native.ptr(buf), nbytes.value, 4) == 0
     assert buf.tobytes() == texts[0][len(b"# header line\n"):]
+    # a descriptor opened without O_TRUNC over a longer file (`1<>file`): the records overwrite their share of it and
+    # the bytes behind them stay, mapped as written
+    body = texts[0][len(b"# header line\n"):]
+    old = b"# header line\n" + bytes(range(1, 251)) * (len(body) // 250 + 40)
+    longer = []
+    for no_mmap in ("", "1"):
+        monkeypatch.delenv("KBBQ_FASTQ_NO_MMAP", raising=False)
+        if no_mmap:
+            monkeypatch.setenv("KBBQ_FASTQ_NO_MMAP", "1")
+        p = tmp_path / ("longer%s.fq" % no_mmap)
+        p.write_bytes(old)
+        fd = os.open(p, flags)
+        os.lseek(fd, len(b"# header line\n"), os.SEEK_SET)
+        f.write(fd, out[:5000], 0, 5000)
+        f.write(fd, out[5000:], 5000, f.N - 5000)
+        assert os.lseek(fd, 0, os.SEEK_CUR) == len(b"# header line\n") + len(body)
+        os.close(fd)
+        longer.append(p.read_bytes())
+    assert longer[0] == longer[1] == b"# header line\n" + body + old[len(b"# header line\n") + len(body):]
     f.close()
 
 
